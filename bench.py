@@ -5,7 +5,13 @@ Headline workload (BASELINE.json configs[1], "C2"): a 4096-patch drum sweep per 
 tom, every FFI-reachable parameter drawn U[0,1), one trigger at frame 0), 2 s each at 44.1 kHz = 88 200 samples per voice,
 per-voice envelopes + filters, per-voice f32 output kept.  One "step" = one full render of the sweep.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|c2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|c2] [--dump-outputs DIR]
+
+* --dump-outputs DIR (ours, rank 0): after the timed loops, writes what the last timed step of each C2 loop computed as
+  DIR/c2_device.npy (device-resident render), DIR/c2_host.npy (host-buffer render) and DIR/c2_pcm16.npy (16-bit PCM render,
+  the integer samples as float32): every voice of the rank's shard at DUMP_FRAMES, 4096 x 1024 float32 each, 48 MiB in all.
+  The inputs are seeded, so two builds of the library can be compared array for array.  The batch keeps its voices'
+  state from render to render, so the arrays also depend on --warmup and --steps: compare runs with the same arguments.
 
 * ours: `value` = voice-samples/s with patches and output resident in HBM (device time, CUDA events on the library's
   launching streams, max over ranks); `e2e` = the same through the C ABI with HOST buffers (event tables H2D + kernels +
@@ -43,6 +49,8 @@ import numpy as np
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+# The benchmark runs from the tree build() left and writes nothing into it (the tree may be read-only).
+sys.dont_write_bytecode = True
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -57,6 +65,9 @@ C4_ENGINES, C4_SECONDS = 1600, 10.0
 C5_ENGINES_PER_GPU, C5_BARS = 8192, 2
 # Algorithmic bytes per engine-sample of the C5 chain (SURVEY.md §8d): 4 stored + delay 24 + spring 96 (+ plate 268)
 C5_BYTES_PER_ENGINE_SAMPLE = 4 + 24 + 96
+# Frames of every voice that --dump-outputs keeps: the attack densely (where the voices differ most), then a seeded
+# sample of the decay.
+DUMP_FRAMES = np.concatenate([np.arange(512), np.sort(np.random.default_rng(SEED).choice(np.arange(512, FRAMES), 512, replace=False))])
 
 
 def workload_config(world):
@@ -401,7 +412,7 @@ def loops_block():
     """Sample-playback sources at batch size (tools/loops_bench.py), in a SUBPROCESS: these kernels were finished with the round's last
     GPU seconds, so whatever they do stays outside this process and the headline line; a failure is recorded, not raised."""
     try:
-        p = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "loops_bench.py"), "1024", "2"], capture_output=True, text=True, timeout=150)
+        p = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "tools", "loops_bench.py"), "1024", "2"], capture_output=True, text=True, timeout=150)
         lines = [ln for ln in p.stdout.splitlines() if ln.startswith("{")]
         if p.returncode != 0 or not lines:
             return {"error": ((p.stderr or "") + (p.stdout or ""))[-400:]}
@@ -492,6 +503,9 @@ def run_ours(args, rank, world, local_rank):
     launches = L.gooey_b200_launch_count() - launches_before
     clocks = sampler.stop()
     kstats = kernel_stats(L)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    if dump is not None:
+        dump["c2_device"] = out_dev[:, torch.from_numpy(DUMP_FRAMES).to(out_dev.device)].cpu().numpy()
 
     # end-to-end through the C ABI with host buffers
     for _ in range(max(args.warmup, 3 if world == 1 else 10)):   # the host-buffer path has its own first-call costs (staging allocations, page touch)
@@ -507,6 +521,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     wall_e2e = time.perf_counter() - t0
     checksum = float(np.abs(out_np[:, ::97]).sum())
+    if dump is not None:
+        dump["c2_host"] = out_np[:, DUMP_FRAMES]          # a copy: the PCM pass below reuses this memory
     # the same end to end with the bounce_to_wav product: 16-bit PCM quantised on the device, half the bytes drained
     for _ in range(2):
         batch.trigger_all(0, vel); batch.render_pcm16(FRAMES, pcm_np)
@@ -516,6 +532,11 @@ def run_ours(args, rank, world, local_rank):
         batch.trigger_all(0, vel); batch.render_pcm16(FRAMES, pcm_np)
     barrier()
     wall_pcm = time.perf_counter() - t0
+    if dump is not None:
+        dump["c2_pcm16"] = pcm_np[:, DUMP_FRAMES].astype(np.float32)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.ascontiguousarray(a, np.float32))
     dev_ms, wall_e2e, wall_pcm = max_over_ranks([dev_ms, wall_e2e, wall_pcm])
     numa_node = host_buf.numa_node
     batch.close()
@@ -604,6 +625,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--configs", default="all", choices=["all", "c2", "c5"], help="c2: headline only (profiling runs); c5: headline + the C5 block only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of what the last timed C2 step of each loop computed as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
