@@ -49,12 +49,12 @@ __device__ __forceinline__ Env env_after(const Env& e, const EnvBlk& b, int n) {
 
 template <int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) bass_wave_kernel(const VoiceLaunch L) {
-  __shared__ w32::GeoTables T;
+  __shared__ wave::GeoTables T;
   __shared__ BassState states[WARPS];
   __shared__ float stashes[WARPS][6][32];
   __shared__ double phase_stash[WARPS][3][32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  w32::geo_tables_init(T, L.rc, threadIdx.x, WARPS * 32);
+  wave::geo_tables_init(T, L.rc, threadIdx.x, WARPS * 32);
   __syncthreads();
   const int v = blockIdx.x * WARPS + warp;
   if (v >= L.n) return;
@@ -159,7 +159,7 @@ __global__ void __launch_bounds__(WARPS * 32) bass_wave_kernel(const VoiceLaunch
         Oversamp os = s.ws.os;
         if (shaping) {
           const float wmix = s.ws.mix, d_ = drive, c_ = comp;
-          const float shaped = w32::os_scan(os, mix, [d_, c_](float x) { return w32::w_tanh(x * d_) * c_; }, T, lane, last);
+          const float shaped = wave::os_scan(os, mix, [d_, c_](float x) { return wave::w_tanh(x * d_) * c_; }, T, lane, last);
           sat = mix * (1.0f - wmix) + shaped * wmix;
         }
         // envelopes: lane-local copies as the frames before mine leave them

@@ -21,26 +21,18 @@
 // at deactivation) each round; a voice without work just attends the barriers.
 //
 // Exactness: the S phases execute the reference's operations in the reference's order (same as the replays they
-// replace); the P phases are the scans / memoryless stages of wave.cuh unchanged.  tests/test_voices_gpu.py compares this
-// back end with the per-sample-order back end (GOOEY_B200_BACKEND=serial) and with the oracle.
+// replace); the P phases are the scans / memoryless stages of wave.cuh unchanged.  tests/test_backend_choice_gpu.py
+// renders enough toms for this back end to be chosen and compares it with the per-sample-order back end
+// (GOOEY_B200_BACKEND=serial) and with the oracle.
 #pragma once
 #include <climits>
 #include <type_traits>
 #include "wave.cuh"
 
 namespace gd { namespace coop {
-using namespace gd::w32;      // scan helpers for full-warp groups: scan1 / ap_sec / hb_run / os_scan / lin2_scan / biquad_scan / tpt_scan ...
+using namespace gd::wave;     // warp-wide scan helpers: scan1 / ap_sec / hb_run / os_scan / lin2_scan / biquad_scan / tpt_scan ...
 
 constexpr unsigned FULL = 0xffffffffu;
-// -DGOOEY_COOP_PROFILE: thread 0 of CTA 0 accumulates the cycles between the phase barriers of a round and prints them at
-// the end of the launch (diagnostic build only; selected with GOOEY_B200_LIB).
-#ifdef GOOEY_COOP_PROFILE
-#define COOP_T(i) do { if (threadIdx.x == 0 && blockIdx.x == 0) { const long long t_ = clock64(); g_coop_prof[i] += t_ - g_coop_last; g_coop_last = t_; } } while (0)
-__device__ long long g_coop_prof[16];
-__device__ long long g_coop_last;
-#else
-#define COOP_T(i) do {} while (0)
-#endif
 constexpr int SP = 33;        // stash row pitch (floats)
 enum { M_IDLE = 0, M_NORMAL = 1, M_TAIL = 2, M_GENERIC = 3, M_SERIAL = 4 };
 enum { F_NORMAL = 1u << M_NORMAL, F_TAIL = 1u << M_TAIL, F_GENERIC = 1u << M_GENERIC, F_SERIAL = 1u << M_SERIAL, F_MEMBRANE = 1u << 8 };
@@ -90,7 +82,7 @@ struct TomC {
   static constexpr int NST = 12;
   enum { ST_INC = 0, ST_FFWD = 0, ST_RND = 1, ST_A1 = 1, ST_FF = 2, ST_A2 = 2, ST_TP = 3, ST_FILT = 3, ST_FSP = 4, ST_RIN = 4, ST_RV = 5, ST_Y0 = 5,
          ST_ENV = 10, ST_NOISE = 11, ST_RLEV = 11 };
-  static __host__ __device__ constexpr int min_ctas(int nv) { return nv <= 4 ? 6 : (nv <= 8 ? 3 : 2); }
+  static constexpr int MIN_CTAS = 2;     // resident 16-voice CTAs per SM the register allocation must allow
   static __device__ __forceinline__ int active_end(const TomV::Run&) { return 0x7fffffff; }
   template <class SM> static __device__ __forceinline__ void span_setup(SM&, int, int, const RateCtx&) {}
 
@@ -158,7 +150,6 @@ struct TomC {
     }
     if (lane == 0) S.wflags[rnd_idx & 1u][warp] = mode == M_IDLE ? 0u : ((1u << mode) | ((d.membrane > 0.0f && mode != M_GENERIC) ? F_MEMBRANE : 0u));
     __syncthreads();                                                                                   // b1
-    COOP_T(1);
     const unsigned fl = __reduce_or_sync(FULL, lane < NV ? S.wflags[rnd_idx & 1u][lane] : 0u);
     // ------------------------------------------------------------------------------------------------ phase S1
     if (fl & (F_NORMAL | F_GENERIC)) {
@@ -225,7 +216,6 @@ struct TomC {
         }
       }
       __syncthreads();                                                                                 // b2
-    COOP_T(2);
     }
     // ------------------------------------------------------------------------------------------------ phases B, S2
     float filtered = 0.0f;
@@ -266,7 +256,6 @@ struct TomC {
         if (lane == nv - 1) { Biquad& o = a.bp; o.b0 = b0; o.b1 = b1; o.b2 = b2; o.a1 = a1; o.a2 = a2; o.x1 = x; o.x2 = xm1; }
       }
       __syncthreads();                                                                                 // b3
-    COOP_T(3);
       if (warp == 0) {   // S2
         const int vv = lane < NV ? lane : 0;
         const bool on = lane < NV && S.ri[vv].mode == M_NORMAL;
@@ -294,7 +283,6 @@ struct TomC {
         if (on) { S.aud[vv].bp.y1 = y1; S.aud[vv].bp.y2 = y2; }
       }
       __syncthreads();                                                                                 // b4
-    COOP_T(4);
       if (mode == M_NORMAL) filtered = st[ST_FILT][warp][lane];
     }
     // ------------------------------------------------------------------------------------------------ phases C, S3, D, S4
@@ -319,7 +307,6 @@ struct TomC {
         }
       }
       __syncthreads();                                                                                 // b5
-    COOP_T(5);
       {   // S3: q = (filter, voice) pairs on lanes
         const int q = warp * 32 + lane;
         const int f = q / NV, vv = q - f * NV;
@@ -351,7 +338,6 @@ struct TomC {
         }
       }
       __syncthreads();                                                                                 // b6
-    COOP_T(6);
       if ((mode == M_NORMAL || mode == M_TAIL) && d.membrane > 0.0f) {   // D
         float acc = 0.0f;
 #pragma unroll
@@ -360,7 +346,6 @@ struct TomC {
         st[ST_RIN][warp][lane] = fabsf(mem_out) * 0.001f;
       }
       __syncthreads();                                                                                 // b7
-    COOP_T(7);
       if (warp == NV - 1) {   // S4
         const int vv = lane < NV ? lane : 0;
         const int m = S.ri[vv].mode;
@@ -399,7 +384,6 @@ struct TomC {
         if (on) S.aud[vv].ring_level = ring;
       }
       __syncthreads();                                                                                 // b8
-    COOP_T(8);
       if (mode == M_TAIL) rlev = st[ST_RLEV][warp][lane];
     }
     // ------------------------------------------------------------------------------------------------ output
@@ -422,7 +406,7 @@ struct TomC {
 
 // ---- the kernel --------------------------------------------------------------------------------------------------------
 template <class C, int NV>
-__global__ void __launch_bounds__(NV * 32, C::min_ctas(NV)) coop_kernel(const VoiceLaunch L) {
+__global__ void __launch_bounds__(NV * 32, C::MIN_CTAS) coop_kernel(const VoiceLaunch L) {
   using V = typename C::V; using Span = typename V::Span; using Aud = typename V::Aud;
   constexpr int WC = sizeof(typename V::Ctl) / 4;
   constexpr int WA = sizeof(Aud) / 4;
@@ -463,9 +447,6 @@ __global__ void __launch_bounds__(NV * 32, C::min_ctas(NV)) coop_kernel(const Vo
   int pj = -1;
 #pragma unroll
   for (int q = 0; q < V::NPL; q++) pn[q] = 0.0f;
-#ifdef GOOEY_COOP_PROFILE
-  if (threadIdx.x == 0 && blockIdx.x == 0) g_coop_last = clock64();
-#endif
   for (unsigned rnd_idx = 0;; rnd_idx++) {
     const bool more = alive && j < c1;
     bool work = false;
@@ -511,7 +492,6 @@ __global__ void __launch_bounds__(NV * 32, C::min_ctas(NV)) coop_kernel(const Vo
     __syncwarp();                                  // the previous round's readers of ri[warp] are done
     if (lane == 0) S.ri[warp] = RoundInfo{j, nl, nl, work ? M_NORMAL : M_IDLE};
     if (!__syncthreads_or(more ? 1 : 0)) break;                                                         // b0
-    COOP_T(0);
     float y = 0.0f;
     int nout = nl;
     C::template round<NV>(S, warp, lane, work, p, j, nout, y, L.rc, rnd_idx);
@@ -519,16 +499,8 @@ __global__ void __launch_bounds__(NV * 32, C::min_ctas(NV)) coop_kernel(const Vo
       if (lane < nout) out[j + lane] = y;
       j += nout;
     }
-    COOP_T(9);
   }
   __syncthreads();
-#ifdef GOOEY_COOP_PROFILE
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    printf("coop profile chunk0=%d:", L.chunk0);
-    for (int i = 0; i < 10; i++) { printf(" t%d=%lld", i, g_coop_prof[i]); g_coop_prof[i] = 0; }
-    printf("\n");
-  }
-#endif
   if (alive) {
     const uint32_t* aw = reinterpret_cast<const uint32_t*>(&a);
     for (int w = lane; w < WA; w += 32) L.state[(size_t)(WC + w) * L.n_pad + sv] = aw[w];

@@ -130,7 +130,7 @@ struct VoiceBank {
   // call after the launching stream has been synchronised
   void collect_stats() { kicks.collect_stats(); snares.collect_stats(); hats.collect_stats(); toms.collect_stats(); }
   // frames per output chunk of the last launch (identical for every bucket) and the per-chunk completion fence
-  int chunk_frames(int frames) const { return TypeRunner<gd::KickV>::chunk_of(frames, kicks.chunk_frames); }
+  int chunk_frames(int frames) const { return TypeRunner<gd::KickV>::chunk_of(frames); }
   void wait_chunk(cudaStream_t s, int i) { kicks.wait_chunk(s, i); snares.wait_chunk(s, i); hats.wait_chunk(s, i); toms.wait_chunk(s, i); basses.wait_chunk(s, i); polys.wait_chunk(s, i); grans.wait_chunk(s, i); }
 };
 

@@ -8,7 +8,7 @@
 // steal at <= 80 per second, parameter glides, cloud end) are run by lane 0 on the shared-memory copy of the state with
 // the very functions the per-sample path uses (voices2.cuh), so their arithmetic and order are the reference's.
 // The only re-association is the overlap-add itself: 80 f32 terms summed as a fixed shuffle tree instead of slot order
-// (<= 1e-7 of full scale; the per-sample path stays available as the A/B reference, GOOEY_B200_GRAN=serial).
+// (<= 1e-7 of full scale).
 #pragma once
 #include "kernels.cuh"
 
@@ -111,26 +111,14 @@ __global__ void __launch_bounds__(WARPS * 32) gran_wave_kernel(const VoiceLaunch
           Grain& g = s.grains[i];
           if (!g.active) continue;
           if (g.age >= g.duration) { g.active = 0; continue; }
-#ifdef GOOEY_GRAN_EXACT_WINDOW
-          const float phase = clampf(g.age / g.duration, 0.0f, 1.0f);
-#else
           const float phase = clampf(__fdividef(g.age, g.duration), 0.0f, 1.0f);     // 2-ulp quotient: the argument of a memoryless window (below)
-#endif
           // window = max(sin(pi phase), 0) ^ shape (granulator.rs:686-689).  A memoryless gain in [0, 1] applied to one grain of up to 80:
           // the ~1-ulp sine of the front ends (relative accuracy kept near its zeros: the reduction is exact) and exp2(shape log2 s) with
           // `lg2.approx` / CUDA's exp2f — relative error <= 3e-5 where the window is below 1e-4, <= 1e-6 elsewhere — replace ~180 instructions of the bit-exact ports per
-          // grain-sample (GOOEY_GRAN_EXACT_WINDOW restores them; the per-sample path, GOOEY_B200_GRAN=serial, always uses them)
-#ifdef GOOEY_GRAN_EXACT_WINDOW
-          const float window = gm::g_powf(fmaxf(gm::g_sinf(PI_F * clampf(phase, 0.0f, 1.0f)), 0.0f), g.window_shape);
-#else
+          // grain-sample.
           const float sw = fmaxf(gm::g_sinf_fast(PI_F * clampf(phase, 0.0f, 1.0f)), 0.0f);
           const float window = sw > 0.0f ? exp2f(g.window_shape * __log2f(sw)) : gm::g_powf(sw, g.window_shape);   // lg2.approx: 2^-22 absolute on [0.5, 2], relative elsewhere
-#endif
-#ifdef GOOEY_GRAN_EXACT_WINDOW
-          const float rg = g.release_total > 0.0f ? clampf(g.release_samples / g.release_total, 0.0f, 1.0f) : 1.0f;
-#else
           const float rg = g.release_total > 0.0f ? clampf(__fdividef(g.release_samples, g.release_total), 0.0f, 1.0f) : 1.0f;   // release fade: a gain, 2-ulp quotient
-#endif
           const float smp = gran_sample(buf, blen, g.source_pos);
           part += smp * window * rg * g.velocity * gc;
           g.source_pos += g.speed * g.direction;

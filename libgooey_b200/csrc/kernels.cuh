@@ -51,11 +51,7 @@ struct KickV {
   static __device__ __forceinline__ void front(const Span& sp, double now, uint32_t, float sr, float* o) {
     // ~1-ulp sine in the additive oscillators unless the feedback waveshaper's drive would amplify that ulp past the
     // parity margin (its tanh has slope `drive` at the origin, up to 100)
-#ifdef GOOEY_FRONT_EXACT_SIN
-    KickFront f = kick_front<false>(sp.c, sp.d, now, sr);
-#else
     KickFront f = sp.d.drive <= 8.0f ? kick_front<true>(sp.c, sp.d, now, sr) : kick_front<false>(sp.c, sp.d, now, sr);
-#endif
     o[0] = f.p1; o[1] = f.raw_click; o[2] = f.ne; o[3] = f.amp;
   }
   static __device__ __forceinline__ void span_begin(Aud& a, const Span& sp, Run& r, float) { kick_span_begin(a, sp.c, sp.resets); r.d = sp.d; r.j_act = sp.j_act; }
@@ -81,11 +77,7 @@ struct SnareV {
   static __device__ __forceinline__ void plan(Ctl& c, uint32_t r, const double* tt, int ja, int jb, Span& sp) { snare_plan(c, r, tt, ja, jb, sp); }
   static __device__ __forceinline__ int front_end(const Span& sp) { return sp.j_act; }
   static __device__ __forceinline__ void front(const Span& sp, double now, uint32_t, float sr, float* o) {
-#ifdef GOOEY_FRONT_EXACT_SIN
-    SnareFront f = snare_front<false>(sp.c, sp.d, now, sr);
-#else
     SnareFront f = snare_front<true>(sp.c, sp.d, now, sr);      // the snare's waveshaper drive is at most 10
-#endif
     o[0] = f.tonal_out; o[1] = f.raw_noise; o[2] = f.cne; o[3] = f.crack_out; o[4] = f.amp;
   }
   static __device__ __forceinline__ void span_begin(Aud& a, const Span& sp, Run& r, float) { snare_span_begin(a, sp.c, sp.resets); r.d = sp.d; r.j_act = sp.j_act; }

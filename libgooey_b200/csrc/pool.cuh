@@ -6,7 +6,8 @@
 // gm:: math) are uploaded lazily in bulk.
 // TypeRunner<V>: the per-render list of (slot, output row, events) for one type bucket and the
 // A -> (B | C pipelined over time chunks) + S launch sequence of kernels.cuh.  Type bucketing keeps
-// warps type-homogeneous (no cross-instrument divergence).
+// warps type-homogeneous (no cross-instrument divergence).  choose_back() fixes which kernel plays C for the drums;
+// the bass, the granulator and the poly synth have one path each (their warp kernels, or kernel S).
 #pragma once
 #include <algorithm>
 #include <atomic>
@@ -19,15 +20,6 @@
 #include "coop.cuh"
 #include "gran_wave.cuh"
 #include "bass_wave.cuh"
-#ifndef GOOEY_WAVE_CTA_WARPS_DEFAULT
-#define GOOEY_WAVE_CTA_WARPS_DEFAULT 1
-#endif
-#ifndef GOOEY_WAVE_G_KICK
-#define GOOEY_WAVE_G_KICK 32
-#define GOOEY_WAVE_G_SNARE 32
-#define GOOEY_WAVE_G_HAT 32
-#define GOOEY_WAVE_G_TOM 32
-#endif
 #include "../../include/gooey_batch.h"
 
 namespace gh {
@@ -149,44 +141,39 @@ struct ClockWindow {
 };
 ClockTable& clock_table(float sr);
 
-// Which voice types have a scan back-end (wave.cuh); the others use back_kernel (one voice per lane).  ID indexes the
-// per-type group width table below.
-template <class V> struct WaveOf { static constexpr bool has = false; static constexpr int ID = -1; static constexpr const char* name = "back_kernel"; };
-template <> struct WaveOf<gd::KickV> { static constexpr bool has = true; static constexpr int ID = 0; using w32 = gd::w32::KickW; static constexpr const char* name = "wave_kernel<KickW>";
-#ifdef GOOEY_WAVE_ALL_WIDTHS
-  using w16 = gd::w16::KickW; using w8 = gd::w8::KickW;
-#endif
-};
-template <> struct WaveOf<gd::SnareV> { static constexpr bool has = true; static constexpr int ID = 1; using w32 = gd::w32::SnareW; static constexpr const char* name = "wave_kernel<SnareW>";
-#ifdef GOOEY_WAVE_ALL_WIDTHS
-  using w16 = gd::w16::SnareW; using w8 = gd::w8::SnareW;
-#endif
-};
-template <> struct WaveOf<gd::HatV> { static constexpr bool has = true; static constexpr int ID = 2; using w32 = gd::w32::HatW; static constexpr const char* name = "wave_kernel<HatW>";
-#ifdef GOOEY_WAVE_ALL_WIDTHS
-  using w16 = gd::w16::HatW; using w8 = gd::w8::HatW;
-#endif
-};
-template <> struct WaveOf<gd::TomV> { static constexpr bool has = true; static constexpr int ID = 3; using w32 = gd::w32::TomW; static constexpr const char* name = "wave_kernel<TomW>";
-#ifdef GOOEY_WAVE_ALL_WIDTHS
-  using w16 = gd::w16::TomW; using w8 = gd::w8::TomW;
-#endif
-};
-// Which voice types have a CTA-cooperative back end (coop.cuh).
-template <class V> struct CoopOf { static constexpr bool has = false; };
-template <> struct CoopOf<gd::TomV> { static constexpr bool has = true; using C = gd::coop::TomC; static constexpr const char* name = "coop_kernel<TomC>"; };
-// GOOEY_B200_BACKEND: "serial" = per-sample-order kernel C everywhere (the A/B reference of the parity tests), "wave" = the
-// warp-per-voice scan back end of round 1, anything else / unset = the CTA-cooperative back end where a type has one.
-inline bool wave_backend() { const char* e = getenv("GOOEY_B200_BACKEND"); return e && strcmp(e, "wave") == 0; }
-// Voices per CTA of the cooperative back end (4, 8 or 16; GOOEY_B200_COOP_NV overrides the default).
-inline int coop_nv() { const char* e = getenv("GOOEY_B200_COOP_NV"); if (e) { int v = atoi(e); if (v == 4 || v == 8 || v == 16) return v; } return 16; }
+// ---- the drum back ends (kernel C of the A -> (B | C) + S sequence) ----
+// Which kernel renders a drum bucket depends on the voice type and on how many voices of the type one launch holds:
+//   tom, >= COOP_FROM voices                      coop_kernel<TomC, COOP_NV>   (coop.cuh)
+//   kick / snare / hi-hat / tom, fewer voices     wave_kernel<...W>           (wave.cuh)
+//   kick / snare / hi-hat, >= SERIAL_FROM voices  back_kernel<V, 32>          (kernels.cuh)
+// GOOEY_B200_BACKEND=serial puts every drum on back_kernel: the per-sample-order reference of the parity tests.
+enum class Back { Wave, Coop, Serial };
 // The cooperative back end issues ~3x fewer instructions per voice-frame but walks a block through barrier-separated phases,
 // so a voice's timeline is slower than in the warp-per-voice back end while voices are too few to fill the device with CTAs:
-// it takes over above this many voices of one type (measured crossover; GOOEY_B200_COOP_ABOVE overrides).
-inline int coop_above() { if (const char* e = getenv("GOOEY_B200_COOP_ABOVE")) { int v = atoi(e); if (v >= 0) return v; } return 4096; }
-template <class C, int NV> inline void coop_launch(int cnt, cudaStream_t s, const gd::VoiceLaunch& L) {
-  using SM = gd::coop::Smem<C, NV>;
-  auto kernel = gd::coop::coop_kernel<C, NV>;
+// it takes over from this many voices of one type (measured crossover).
+constexpr int COOP_FROM = 4096;
+constexpr int COOP_NV = 16;          // voices per cooperative CTA
+// From this many voices of one type the per-sample-order back end with one voice per THREAD wins: the warp-per-voice
+// back end spends 32 lanes on the replayed recurrences of one voice, which pays only while voices are too few to fill the
+// device with threads (measured, 32768 voices x 2 s: tom 234 vs 526 ms, hi-hat 117 vs 193 ms; at 16384: 176 vs 263 and
+// 104 vs 97 ms).
+constexpr int SERIAL_FROM = 12288;
+inline bool serial_backend() { const char* e = getenv("GOOEY_B200_BACKEND"); return e && strcmp(e, "serial") == 0; }
+template <class V> inline Back choose_back(int cnt) {
+  if (serial_backend()) return Back::Serial;
+  if (std::is_same<V, gd::TomV>::value) return cnt >= COOP_FROM ? Back::Coop : Back::Wave;
+  return cnt >= SERIAL_FROM ? Back::Serial : Back::Wave;
+}
+// The scan back end of each drum type and its kernel-statistics key.
+template <class V> struct WaveOf;
+template <> struct WaveOf<gd::KickV> { using W = gd::wave::KickW; static constexpr const char* name = "wave_kernel<KickW>"; };
+template <> struct WaveOf<gd::SnareV> { using W = gd::wave::SnareW; static constexpr const char* name = "wave_kernel<SnareW>"; };
+template <> struct WaveOf<gd::HatV> { using W = gd::wave::HatW; static constexpr const char* name = "wave_kernel<HatW>"; };
+template <> struct WaveOf<gd::TomV> { using W = gd::wave::TomW; static constexpr const char* name = "wave_kernel<TomW>"; };
+
+inline void coop_launch(int cnt, cudaStream_t s, const gd::VoiceLaunch& L) {
+  using SM = gd::coop::Smem<gd::coop::TomC, COOP_NV>;
+  auto kernel = gd::coop::coop_kernel<gd::coop::TomC, COOP_NV>;
   static std::mutex mu;
   static std::set<int> done;
   int dev = 0;
@@ -198,47 +185,7 @@ template <class C, int NV> inline void coop_launch(int cnt, cudaStream_t s, cons
       GH_CUDA(cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     }
   }
-  kernel<<<(cnt + NV - 1) / NV, NV * 32, sizeof(SM), s>>>(L);
-}
-
-// Lanes per voice for kick / snare / hat / tom (see wave.cuh "Group width").  GOOEY_B200_WAVE_G="32,32,8,8" overrides
-// (tuning only; every width renders the same audio up to the scans' re-association noise).
-inline int wave_group_width(int id) {
-  static int table[4] = {0, 0, 0, 0};
-  static std::once_flag once;
-  std::call_once(once, [] {
-    const int def[4] = {GOOEY_WAVE_G_KICK, GOOEY_WAVE_G_SNARE, GOOEY_WAVE_G_HAT, GOOEY_WAVE_G_TOM};
-    for (int i = 0; i < 4; i++) table[i] = def[i];
-    if (const char* e = getenv("GOOEY_B200_WAVE_G")) {
-      int v[4];
-      if (sscanf(e, "%d,%d,%d,%d", &v[0], &v[1], &v[2], &v[3]) == 4)
-        for (int i = 0; i < 4; i++) if (v[i] == 8 || v[i] == 16 || v[i] == 32) table[i] = v[i];
-    }
-#ifndef GOOEY_WAVE_ALL_WIDTHS
-    for (int i = 0; i < 4; i++) table[i] = 32;
-#endif
-  });
-  return table[id];
-}
-// GOOEY_B200_BACKEND=serial forces the per-sample-order back-end (kernel C) everywhere: the A/B switch used by the
-// parity tests to compare the two back-ends.
-inline bool serial_backend() { const char* e = getenv("GOOEY_B200_BACKEND"); return e && strcmp(e, "serial") == 0; }
-// Above this many voices of one type the per-sample-order back end with one voice per THREAD wins: the warp-per-voice
-// back end spends 32 lanes on the replayed recurrences of one voice, which pays only while voices are too few to fill the
-// device with threads (measured, 32768 voices x 2 s: tom 234 vs 526 ms, hi-hat 117 vs 193 ms; at 16384: 176 vs 263 and
-// 104 vs 97 ms).  GOOEY_B200_SERIAL_ABOVE overrides.
-// Warps (= voices) per CTA of the scan back end: 8 keeps an SM's warps in step (one CTA barrier per block) so they share
-// instruction fetches, 1 lets every voice run free.  Measured on C2: no gain from the lock-step (isolated buckets equal,
-// the mix 54.7 vs 50.1 ms), so 1 is the default; build with -DGOOEY_WAVE_LOCKSTEP and set GOOEY_B200_WAVE_WARPS=8 to try it.
-inline int wave_cta_warps() {
-  const char* e = getenv("GOOEY_B200_WAVE_WARPS");
-  if (e && atoi(e) == 1) return 1;
-  if (e && atoi(e) == 8) return 8;
-  return GOOEY_WAVE_CTA_WARPS_DEFAULT;
-}
-inline int serial_above() {
-  if (const char* e = getenv("GOOEY_B200_SERIAL_ABOVE")) { int v = atoi(e); if (v > 0) return v; }
-  return 12288;
+  kernel<<<(cnt + COOP_NV - 1) / COOP_NV, COOP_NV * 32, sizeof(SM), s>>>(L);
 }
 
 // Kernels whose shared-memory carve-out differs cannot share an SM: the L1 / shared split is an SM-wide setting, so a
@@ -255,19 +202,8 @@ template <class K> inline void same_carveout(K kernel) {
 }
 #define GH_LAUNCH(kernel, grid, block, stream, ...) do { same_carveout(kernel); kernel<<<grid, block, 0, stream>>>(__VA_ARGS__); } while (0)
 
-// Rank of a voice type by the length of its per-chunk dependency chain (tools/type_scaling.py: tom 31 ms, snare 22 ms,
-// kick 11 ms, hi-hat 10 ms per 1024 voices x 2 s); used for stream priorities.
-template <class V> struct PrioOf { static constexpr int rank = 4; };
-template <> struct PrioOf<gd::TomV> { static constexpr int rank = 0; };
-template <> struct PrioOf<gd::SnareV> { static constexpr int rank = 1; };
-template <> struct PrioOf<gd::KickV> { static constexpr int rank = 2; };
-template <> struct PrioOf<gd::HatV> { static constexpr int rank = 3; };
-
-// Frames per front/back pipeline stage.  GOOEY_B200_CHUNK overrides (tuning).
-inline int default_chunk_frames() {
-  if (const char* e = getenv("GOOEY_B200_CHUNK")) { int v = atoi(e); if (v >= 1024 && v <= (1 << 20)) return (v + 31) & ~31; }
-  return 8192;
-}
+// Frames per front/back pipeline stage.
+constexpr int CHUNK_FRAMES = 8192;
 // One type bucket of one render call.
 template <class V> struct TypeRunner {
   using State = typename V::State;
@@ -286,10 +222,9 @@ template <class V> struct TypeRunner {
   std::vector<cudaEvent_t> evT0, evT1;   // timing brackets of the back-end launch of chunk i (on sC)
   std::vector<double> timed_units;       // voice-frames of that launch
   std::vector<cudaEvent_t> evChunk;      // evChunk[i]: frames of chunk i are final in the output (fast-path voices)
-  int chunk_frames = default_chunk_frames();
   int launched_chunks = 0;               // chunks of the most recent launch (0 = one undivided launch)
   const char* backend_name = "back_kernel";   // the back-end kernel of the most recent launch (kernel statistics key)
-  static int chunk_of(int frames, int chunk_frames) { return std::min(chunk_frames, (frames + 31) & ~31); }
+  static int chunk_of(int frames) { return std::min(CHUNK_FRAMES, (frames + 31) & ~31); }
   // Makes `s` wait until every voice of this bucket has written frames [i * chunk, (i + 1) * chunk) of the last launch.
   void wait_chunk(cudaStream_t s, int i) {
     if (n() == 0) return;
@@ -314,18 +249,10 @@ template <class V> struct TypeRunner {
   }
   void ensure_streams() {
     if (sC) return;
-    // Stream priorities.  The buckets overlap on the device and the step ends when the slowest bucket's chunk chain
-    // does (tom on C2), so the bucket with the longest chain should win the block scheduler's slots whenever one frees up
-    // and the cheaper buckets fill the gaps: PrioOf<V> ranks the types by per-voice cost, 0 = longest chain.
-    // Measured on C2: 54.4 ms ranked vs 55.1 ms equal (noise) — the tom chain is slowed by sharing issue slots, not by
-    // waiting for slots — so equal priorities stay the default; GOOEY_B200_PRIO=1 enables the ranking (tuning knob).
-    int prio_lo = 0, prio_hi = 0;
-    GH_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));   // numerically lower = higher priority
-    const char* pe = getenv("GOOEY_B200_PRIO");
-    int prio = prio_lo;
-    if (pe && pe[0] == '1') prio = std::min(prio_lo, prio_hi + PrioOf<V>::rank);
-    GH_CUDA(cudaStreamCreateWithPriority(&sB, cudaStreamNonBlocking, prio));
-    GH_CUDA(cudaStreamCreateWithPriority(&sC, cudaStreamNonBlocking, prio));
+    // Equal stream priorities: ranking the buckets by the length of their chunk chains measured as noise on C2 (the tom
+    // chain is slowed by sharing issue slots, not by waiting for them).
+    GH_CUDA(cudaStreamCreateWithFlags(&sB, cudaStreamNonBlocking));
+    GH_CUDA(cudaStreamCreateWithFlags(&sC, cudaStreamNonBlocking));
     GH_CUDA(cudaStreamCreateWithFlags(&sS, cudaStreamNonBlocking));
     cudaEvent_t* evs[] = {&evA, &evB[0], &evB[1], &evC[0], &evC[1], &evDoneC, &evDoneS};
     for (auto e : evs) GH_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
@@ -382,7 +309,7 @@ template <class V> struct TypeRunner {
       d_span_off.upload(span_off.data(), span_off.size(), sC);
       d_n_spans.alloc(cnt); d_span_cursor.alloc(cnt); d_mode.alloc(cnt);
       d_spans.alloc((size_t)span_off.back() * sizeof(Span));
-      const int chunk = chunk_of(frames, chunk_frames);
+      const int chunk = chunk_of(frames);
       const int rows_pad = pad32(cnt);
       const size_t plane_floats = (size_t)rows_pad * chunk;
       d_planes[0].alloc(plane_floats * V::NPL); d_planes[1].alloc(plane_floats * V::NPL);
@@ -399,6 +326,7 @@ template <class V> struct TypeRunner {
       g_launches.fetch_add(1, std::memory_order_relaxed);
       GH_CUDA(cudaGetLastError());
       GH_CUDA(cudaEventRecord(evDoneS, sS));
+      const Back back = choose_back<V>(cnt);
       int i = 0;
       for (int c0 = 0; c0 < frames; c0 += chunk, i++) {
         const int b = i & 1;
@@ -413,35 +341,20 @@ template <class V> struct TypeRunner {
         if ((int)evT0.size() <= i) { cudaEvent_t e0, e1; GH_CUDA(cudaEventCreate(&e0)); GH_CUDA(cudaEventCreate(&e1)); evT0.push_back(e0); evT1.push_back(e1); timed_units.push_back(0.0); }
         timed_units[i] = (double)cnt * L.chunk_frames;
         GH_CUDA(cudaEventRecord(evT0[i], sC));
-        bool launched = false;
-        backend_name = WaveOf<V>::has ? WaveOf<V>::name : "back_kernel";
-        if constexpr (CoopOf<V>::has) {
-          if (!serial_backend() && !wave_backend() && cnt >= coop_above()) {
-            const int nv = coop_nv();
-            if (nv == 4) coop_launch<typename CoopOf<V>::C, 4>(cnt, sC, L);
-            else if (nv == 8) coop_launch<typename CoopOf<V>::C, 8>(cnt, sC, L);
-            else coop_launch<typename CoopOf<V>::C, 16>(cnt, sC, L);
-            backend_name = CoopOf<V>::name;
-            launched = true;
-          }
+        switch (back) {
+          case Back::Coop:
+            if constexpr (std::is_same<V, gd::TomV>::value) coop_launch(cnt, sC, L);
+            backend_name = "coop_kernel<TomC>";
+            break;
+          case Back::Wave:
+            GH_LAUNCH((gd::wave::wave_kernel<typename WaveOf<V>::W>), cnt, 32, sC, L);   // one voice per one-warp CTA
+            backend_name = WaveOf<V>::name;
+            break;
+          case Back::Serial:
+            GH_LAUNCH((gd::back_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);             // one voice per lane, one warp per CTA
+            backend_name = "back_kernel";
+            break;
         }
-        if (launched) {}
-        else if constexpr (WaveOf<V>::has) {
-          if (!serial_backend() && cnt < serial_above()) {
-            const int g = wave_group_width(WaveOf<V>::ID);          // voices per warp = 32 / g, one warp per CTA
-            const int warps = (cnt * g + 31) / 32;
-#ifdef GOOEY_WAVE_ALL_WIDTHS
-            if (g == 16) GH_LAUNCH((gd::w16::wave_kernel<typename WaveOf<V>::w16, 1>), warps, 32, sC, L);
-            else if (g == 8) GH_LAUNCH((gd::w8::wave_kernel<typename WaveOf<V>::w8, 1>), warps, 32, sC, L);
-            else
-#endif
-#ifdef GOOEY_WAVE_LOCKSTEP          // compiled on request only (it doubles the build time of the back ends)
-            if (wave_cta_warps() == 8) GH_LAUNCH((gd::w32::wave_kernel<typename WaveOf<V>::w32, 8>), (warps + 7) / 8, 256, sC, L);
-            else
-#endif
-            GH_LAUNCH((gd::w32::wave_kernel<typename WaveOf<V>::w32, 1>), warps, 32, sC, L);
-          } else GH_LAUNCH((gd::back_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);
-        } else GH_LAUNCH((gd::back_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);   // one voice per lane, one warp per CTA
         GH_CUDA(cudaGetLastError());
         GH_CUDA(cudaEventRecord(evT1[i], sC));
         GH_CUDA(cudaEventRecord(evC[b], sC));
@@ -471,37 +384,19 @@ template <class V> struct TypeRunner {
       }
     } else {
       if constexpr (std::is_same<V, gd::GranV>::value) {
-        const char* ge = getenv("GOOEY_B200_GRAN");
-        if (!(ge && strcmp(ge, "serial") == 0)) {       // one warp per granulator, grains on lanes (gran_wave.cuh)
-          GH_LAUNCH((gd::gran_wave_kernel<4>), (cnt + 3) / 4, 128, sC, L);
-          g_launches.fetch_add(1, std::memory_order_relaxed);
-          GH_CUDA(cudaGetLastError());
-          GH_CUDA(cudaEventRecord(evDoneC, sC));
-          GH_CUDA(cudaStreamWaitEvent(parent, evDoneC, 0));
-          return;
+        GH_LAUNCH((gd::gran_wave_kernel<4>), (cnt + 3) / 4, 128, sC, L);       // one warp per granulator, grains on lanes (gran_wave.cuh)
+      } else if (std::is_same<V, gd::BassV>::value && !modulated) {           // one warp per bass voice, lane = frame (bass_wave.cuh)
+        const bool ttrace = getenv("GOOEY_B200_TRACE_TYPES") != nullptr;
+        cudaEvent_t t0 = nullptr, t1 = nullptr;
+        if (ttrace) { cudaEventCreate(&t0); cudaEventCreate(&t1); cudaEventRecord(t0, sC); }
+        GH_LAUNCH((gd::bass_wave_kernel<2>), (cnt + 1) / 2, 64, sC, L);
+        if (ttrace) {
+          cudaEventRecord(t1, sC); GH_CUDA(cudaStreamSynchronize(sC));
+          float ms = 0.0f; cudaEventElapsedTime(&ms, t0, t1);
+          fprintf(stderr, "[gooey trace]   bass_wave_kernel: %d voices x %d frames, %.1f ms\n", cnt, frames, ms);
+          cudaEventDestroy(t0); cudaEventDestroy(t1);
         }
-      }
-      if constexpr (std::is_same<V, gd::BassV>::value) {
-        const char* be = getenv("GOOEY_B200_BASS");
-        if (!(be && strcmp(be, "serial") == 0) && !modulated) {      // LFO-routed basses take the per-sample kernel       // one warp per bass voice, lane = frame (bass_wave.cuh)
-          const bool ttrace = getenv("GOOEY_B200_TRACE_TYPES") != nullptr;
-          cudaEvent_t t0 = nullptr, t1 = nullptr;
-          if (ttrace) { cudaEventCreate(&t0); cudaEventCreate(&t1); cudaEventRecord(t0, sC); }
-          GH_LAUNCH((gd::bass_wave_kernel<2>), (cnt + 1) / 2, 64, sC, L);
-          if (ttrace) {
-            cudaEventRecord(t1, sC); GH_CUDA(cudaStreamSynchronize(sC));
-            float ms = 0.0f; cudaEventElapsedTime(&ms, t0, t1);
-            fprintf(stderr, "[gooey trace]   bass_wave_kernel: %d voices x %d frames, %.1f ms\n", cnt, frames, ms);
-            cudaEventDestroy(t0); cudaEventDestroy(t1);
-          }
-          g_launches.fetch_add(1, std::memory_order_relaxed);
-          GH_CUDA(cudaGetLastError());
-          GH_CUDA(cudaEventRecord(evDoneC, sC));
-          GH_CUDA(cudaStreamWaitEvent(parent, evDoneC, 0));
-          return;
-        }
-      }
-      if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);
+      } else if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);   // LFO-routed basses, poly synths
       else GH_LAUNCH((gd::slow_kernel<V, 128>), (cnt + 127) / 128, 128, sC, L);
       g_launches.fetch_add(1, std::memory_order_relaxed);
       GH_CUDA(cudaGetLastError());

@@ -276,7 +276,7 @@ G_D float kick_tick(KickState& s, const double* tt, const RateCtx& rc) {
   // the per-sample path carries gliding (FFI-edited) and LFO-routed voices; on the device its additive oscillators use the same
   // ~1-ulp sine under the same drive rule as the time-parallel front end (kernels.cuh KickV::front) — 89 harmonics x ~100
   // instructions of the bit-exact port were two thirds of a gliding kick's tick.  Host builds (tests/emu) keep the exact port.
-#if defined(__CUDA_ARCH__) && !defined(GOOEY_FRONT_EXACT_SIN)
+#ifdef __CUDA_ARCH__
   const KickFront f = d.drive <= 8.0f ? kick_front<true>(c, d, now, rc.sr) : kick_front<false>(c, d, now, rc.sr);
 #else
   const KickFront f = kick_front(c, d, now, rc.sr);
@@ -510,7 +510,7 @@ G_D float snare_tick(SnareState& s, const double* tt, const RateCtx& rc) {
   }
   snare_live(c);
   const SnareDer d = snare_derive(c);
-#if defined(__CUDA_ARCH__) && !defined(GOOEY_FRONT_EXACT_SIN)
+#ifdef __CUDA_ARCH__
   const SnareFront f = snare_front<true>(c, d, now, rc.sr);      // as SnareV::front (the snare's waveshaper drive is at most 10)
 #else
   const SnareFront f = snare_front(c, d, now, rc.sr);
