@@ -153,22 +153,33 @@ G_HD int env_advance(Env& e, const double* tt, uint32_t kbase, int ja, int jb) {
 }
 
 // ---- max_curve.rs ----------------------------------------------------------------------
-G_HD float max_curve_pos(float progress, float curve) {  // curve > 0 branch of :21-48
+// The factors of the curve > 0 branch of :21-48 that depend only on |curve|: fp and expm1f(fp).  A span stores them per
+// envelope segment, so that the front end evaluates one expm1f per frame instead of powf + 2 expm1f.
+struct CurveK { float fp, den, rcp_den; };
+G_HD CurveK curve_k(float curve) {
   float hp = gm::g_powf((fabsf(curve) + 1e-20f) * 1.2f, 0.41f) * 0.91f;
   float fp = hp / (1.0f - hp);
-  if (fabsf(fp) < 1e-6f) return progress;
-  return gm::g_expm1f(fp * progress) / gm::g_expm1f(fp);
+  float den = gm::g_expm1f(fp);
+  return {fp, den, 1.0f / den};
 }
-G_HD float max_curve(float progress, float curve) {
+// expm1f(fp * progress) / expm1f(fp) through the reciprocal: every curve of the instruments (|curve| = 0.3, 0.8, 0.83) gives
+// fp in [1.4, 10] and a quotient in [0, 1] that is 0 or above 1e-26 (progress is 0 or above 1e-22, see maxenv_value), never
+// subnormal, so g_div_by returns the IEEE quotient.
+G_HD float max_curve_pos(float progress, CurveK k) {
+  if (fabsf(k.fp) < 1e-6f) return progress;
+  return gm::g_div_by(gm::g_expm1f(k.fp * progress), k.den, k.rcp_den);
+}
+G_HD float max_curve(float progress, float curve, CurveK k) {  // k = curve_k(curve)
   progress = clampf(progress, 0.0f, 1.0f);
   if (fabsf(curve) < 1e-6f) return progress;
   if (curve < 0.0f) {
     // reference computes gp for the negative curve first, discards it, then recurses
     float q = clampf(1.0f - progress, 0.0f, 1.0f);
-    return 1.0f - max_curve_pos(q, -curve);
+    return 1.0f - max_curve_pos(q, k);
   }
-  return max_curve_pos(progress, curve);
+  return max_curve_pos(progress, k);
 }
+G_HD float max_curve(float progress, float curve) { return max_curve(progress, curve, curve_k(curve)); }
 // Two-segment MaxCurveEnvelope (all users: hihat2.rs:442, tom2.rs:443) from initial value 0.
 struct MaxEnv2 {
   float target[2], dur[2], curve[2];
@@ -185,27 +196,45 @@ G_HD void maxenv_init(MaxEnv2& e, float t0, float d0ms, float c0, float t1, floa
 G_HD void maxenv_trigger(MaxEnv2& e, double t) { e.active = 1; e.seg = 0; e.seg_start = t; e.seg_start_val = 0.0f; e.cur_val = 0.0f; }
 G_HD void maxenv_set_dur_ms(MaxEnv2& e, int i, float ms) { e.dur[i] = fmaxf(ms / 1000.0f, 0.0f); }
 G_HD bool maxenv_complete(const MaxEnv2& e) { return !e.active && e.seg >= 2; }
-G_HD float maxenv_value(MaxEnv2& e, double now) {  // max_curve.rs:133-174
+// The constants of one segment that depend only on its duration and curve.  The planner stores both segments' in the
+// span, so that the front end does not recompute them every frame.
+struct SegK { float rcp_dur; CurveK ck; };
+G_HD SegK maxenv_seg_k(const MaxEnv2& e, bool s1) {
+  const float dur = s1 ? e.dur[1] : e.dur[0];
+  return {dur > 0.0f ? 1.0f / dur : 0.0f, curve_k(s1 ? e.curve[1] : e.curve[0])};
+}
+// max_curve.rs:133-174; kf(s1) gives the SegK of segment s1 (segments are picked by select, so that a copy of the
+// envelope stays in registers)
+template <class KF> G_HD float maxenv_value_k(MaxEnv2& e, double now, const KF& kf) {
   if (!e.active) return e.cur_val;
   for (;;) {
     if (e.seg >= 2) { e.active = 0; return e.cur_val; }
-    int s = e.seg;
+    const bool s1 = e.seg != 0;
     float el = (float)(now - e.seg_start);
-    float dur = e.dur[s];
+    const float dur = s1 ? e.dur[1] : e.dur[0], target = s1 ? e.target[1] : e.target[0];
     if (el >= dur) {
-      e.seg_start_val = e.target[s];
-      e.cur_val = e.target[s];
+      e.seg_start_val = target;
+      e.cur_val = target;
       e.seg_start += (double)dur;
       e.seg += 1;
       continue;
     }
-    float progress = dur > 0.0f ? el / dur : 1.0f;
-    float cp = max_curve(progress, e.curve[s]);
-    float range = e.target[s] - e.seg_start_val;
+    const SegK k = kf(s1);
+    // el / dur through the reciprocal.  Here 0 <= el < dur, and el is 0 or a difference of two clock values of which the
+    // smaller is at least 1 / sr (or 0 and then el >= 1 / sr): el >= 2^-70, dur <= 4 s, so the quotient is 0 or far above the
+    // subnormal range and g_div_by returns the IEEE quotient.
+    float progress = dur > 0.0f ? gm::g_div_by(el, dur, k.rcp_dur) : 1.0f;
+    float cp = max_curve(progress, s1 ? e.curve[1] : e.curve[0], k.ck);
+    float range = target - e.seg_start_val;
     e.cur_val = e.seg_start_val + range * cp;
     return e.cur_val;
   }
 }
+G_HD float maxenv_value(MaxEnv2& e, double now) { return maxenv_value_k(e, now, [&](bool s1) { return maxenv_seg_k(e, s1); }); }
+// both segments' constants, for a span (the durations and curves do not change within one)
+struct MaxEnvK { SegK s[2]; };
+G_HD MaxEnvK maxenv_k(const MaxEnv2& e) { return {{maxenv_seg_k(e, false), maxenv_seg_k(e, true)}}; }
+G_HD float maxenv_value(MaxEnv2& e, double now, const MaxEnvK& k) { return maxenv_value_k(e, now, [&](bool s1) { return s1 ? k.s[1] : k.s[0]; }); }
 
 // ---- SipHash-1-3(k=0) of one u64 (Rust DefaultHasher; oscillator.rs:187-196, morph_osc.rs:42-47)
 G_HD uint64_t rotl64(uint64_t x, int b) { return (x << b) | (x >> (64 - b)); }
@@ -247,28 +276,71 @@ G_HD float osc_sine_fast(float idx, float freq, float sr, float rcp_sr) {
   const float two_pi = 2.0f * PI_F;
   return gm::g_sinf_fast(gm::g_div_by(idx * freq * two_pi, sr, rcp_sr));
 }
-// additive "triangle": odd harmonics, gain 1/i^2 (powf(i,2) is exact so 1/(i*i) matches), Gibbs taper (:106-131)
+// 1 / (i * i) for odd i < 2 INV_SQ_N: the same f32 quotient, tabulated on the device (i is uniform across the warp)
+G_HD float inv_sq_odd(int i, float fi) {
+#ifdef __CUDA_ARCH__
+  return c_inv_sq[i >> 1];
+#else
+  return 1.0f / (fi * fi);
+#endif
+}
+template <bool FAST> G_HD float tri_partial(float idx, float hf, float sr, float rcp_sr) {
+  return FAST ? osc_sine_fast(idx, hf, sr, rcp_sr) : osc_sine<false>(idx, hf, sr);
+}
+// additive "triangle": odd harmonics, gain 1/i^2 (powf(i,2) is exact so 1/(i*i) matches), Gibbs taper (:106-131).
+// The reference's loop adds harmonic i = 1, 3, ... in increasing order and stops at the first with freq * i > nyquist; the
+// taper is 1 while freq * i <= 0.7 nyquist (below that hf / nyquist cannot round above 0.75).  For freq > 0 and sr > 0,
+// freq * i only grows with i, so the harmonics fall into three runs, each summed by a loop of its own with the reference's
+// operations in the reference's order:
+//   1. freq * i <= 0.7 nyquist and i < 2 INV_SQ_N: no taper (gain * 1 == gain), gain from the table;
+//   2. the tapered top with i < 2 INV_SQ_N, where hf > 0.7 nyquist always holds;
+//   3. i >= 2 INV_SQ_N (freq < nyquist / 2047, about 11 Hz at 44.1 kHz) or any other input: the reference's loop as written.
 template <bool FAST = false> G_HD float osc_triangle(float idx, float freq, float sr) {
   float output = 0.0f;
-  float nyquist = sr / 2.0f;
+  const float nyquist = sr / 2.0f;
   const float rcp_sr = 1.0f / sr;
+  const float rcp_nyq = 2.0f * rcp_sr;      // == RN(1 / nyquist): both are scaled by exactly 2
+  const float lim = 0.7f * nyquist;
   float q = nyquist / freq;
   int max_h = !(q == q) ? 0 : (q >= 2147483648.0f ? 2147483647 : (q <= -2147483648.0f ? (-2147483647 - 1) : (int)q));
-  for (int i = 1; i <= max_h; i += 2) {
+  const int cap = (freq > 0.0f && sr > 0.0f) ? (max_h < 2 * INV_SQ_N - 1 ? max_h : 2 * INV_SQ_N - 1) : 0;   // last odd i runs 1 and 2 may take
+  // n1 = number of harmonics of run 1 (i = 1, 3, ..., 2 n1 - 1): the guess from q is off by at most one harmonic
+  int n1 = 0;
+  if (cap >= 1) {
+    n1 = ((int)fminf(q * 0.7f, (float)cap) + 1) >> 1;
+    while (n1 > 0 && freq * (float)(2 * n1 - 1) > lim) n1--;
+    while (2 * n1 + 1 <= cap && !(freq * (float)(2 * n1 + 1) > lim)) n1++;
+  }
+#ifdef __CUDA_ARCH__
+#pragma unroll 4
+#endif
+  for (int h = 0; h < n1; h++) {
+    const int i = 2 * h + 1;
+    const float fi = (float)i;
+    output += inv_sq_odd(i, fi) * tri_partial<FAST>(idx, freq * fi, sr, rcp_sr);
+  }
+  int i = 2 * n1 + 1;
+  for (; i <= cap; i += 2) {
+    const float fi = (float)i;
+    const float hf = freq * fi;
+    if (hf > nyquist) return output;
+    // hf is in (0.7 nyquist, nyquist]: the quotient is near 1, never subnormal, so the hoisted reciprocal gives its exact bits
+    const float ratio = gm::g_div_by(hf, nyquist, rcp_nyq);
+    const float t = (ratio - 0.75f) / 0.25f;
+    const float taper = ratio > 0.75f ? 1.0f - t * t : 1.0f;
+    output += inv_sq_odd(i, fi) * taper * tri_partial<FAST>(idx, hf, sr, rcp_sr);
+  }
+  for (; i <= max_h; i += 2) {
     float fi = (float)i;
     if (freq * fi > nyquist) break;
-#ifdef __CUDA_ARCH__
-    float gain = i < 2 * INV_SQ_N ? c_inv_sq[i >> 1] : 1.0f / (fi * fi);   // same f32 quotient, tabulated (i is uniform across the warp)
-#else
     float gain = 1.0f / (fi * fi);
-#endif
     float hf = freq * fi;
     float taper = 1.0f;
-    if (hf > 0.7f * nyquist) {          // below that hf / nyquist cannot round above 0.75: skip the division (same result)
+    if (hf > 0.7f * nyquist) {
       float ratio = hf / nyquist;
       if (ratio > 0.75f) { float t = (ratio - 0.75f) / 0.25f; taper = 1.0f - t * t; }
     }
-    output += gain * taper * (FAST ? osc_sine_fast(idx, hf, sr, rcp_sr) : osc_sine<false>(idx, hf, sr));
+    output += gain * taper * tri_partial<FAST>(idx, hf, sr, rcp_sr);
   }
   return output;
 }
@@ -584,6 +656,7 @@ G_HD int phasemod_advance(PhaseMod& m, const double* tt, uint32_t kbase, int ja,
 // MaxCurveEnvelope transitions are path independent (each depends only on `now`), so the value at any frame can be
 // computed from a span-start snapshot, and the state after a range is the state after its last frame.
 G_HD float maxenv_value_pure(const MaxEnv2& e, double now) { MaxEnv2 t = e; return maxenv_value(t, now); }
+G_HD float maxenv_value_pure(const MaxEnv2& e, const MaxEnvK& k, double now) { MaxEnv2 t = e; return maxenv_value(t, now, k); }
 struct MaxEnvDone { const MaxEnv2* e; G_HD bool operator()(double now) const { MaxEnv2 t = *e; maxenv_value(t, now); return t.seg >= 2; } };
 // first frame in [ja, jb) whose tick leaves the envelope complete (seg >= 2); jb if none
 G_HD int maxenv_complete_frame(const MaxEnv2& e, const double* tt, uint32_t kbase, int ja, int jb) {

@@ -574,7 +574,7 @@ struct HatAud {
   Pink pink;
 };
 struct HatState { HatCtl c; HatAud a; };
-struct HatDer { float pitch_hz, tone_hz, vel035, volume; uint32_t pink_on, db24; };
+struct HatDer { float pitch_hz, tone_hz, vel035, volume; uint32_t pink_on, db24; MaxEnvK ek; };   // ek = maxenv_k(c.env)
 struct HatFront { float env; };
 enum { HAT_PLANES = 1 };
 G_HD float hat_pitch_hz(float p) { return denorm(p * p, 3500.0f, 10000.0f); }
@@ -634,9 +634,10 @@ G_HD HatDer hat_derive(const HatCtl& c) {
   d.vel035 = c.velocity;
   d.volume = c.cur[H_VOLUME];
   d.pink_on = c.pink_on; d.db24 = c.db24;
+  d.ek = maxenv_k(c.env);   // after hat_live: the durations are current
   return d;
 }
-G_HD HatFront hat_front(const HatCtl& c, const HatDer&, double now, float) { HatFront f; f.env = maxenv_value_pure(c.env, now); return f; }
+G_HD HatFront hat_front(const HatCtl& c, const HatDer& d, double now, float) { HatFront f; f.env = maxenv_value_pure(c.env, d.ek, now); return f; }
 G_D float hat_osc(float& phase_cycle, float freq, float sr, float pm) {  // PhaseModOsc::tick (:277-286); set_frequency floors at 0
   float inc = fmaxf(freq, 0.0f) / sr;
   phase_cycle = fmodf(phase_cycle + inc, 1.0f);
@@ -725,6 +726,7 @@ struct TomState { TomCtl c; TomAud a; };
 struct TomDer {
   float base_frequency, bend_scaled, tone, mix_control, rand_freq, fq, membrane, mm, vol;
   float w1, w2, w3;
+  MaxEnvK ek;   // maxenv_k(c.env)
 };
 struct TomFront { float env, noise, rnd; };
 enum { TOM_PLANES = 3 };
@@ -851,12 +853,13 @@ G_HD TomDer tom_derive(const TomCtl& c) {
   d.mm = d.membrane / 100.0f;
   d.vol = c.p[T_VOLUME] / 100.0f;
   d.w1 = clampf(-d.mix_control, 0.0f, 1.0f); d.w2 = clampf(1.0f - fabsf(d.mix_control), 0.0f, 1.0f); d.w3 = clampf(d.mix_control, 0.0f, 1.0f);
+  d.ek = maxenv_k(c.env);
   return d;
 }
 // pure part: envelope value and the two SipHash draws keyed by the MorphOsc counter (= frames since the trigger + 1)
-G_HD TomFront tom_front(const TomCtl& c, const TomDer&, double now, uint32_t k) {
+G_HD TomFront tom_front(const TomCtl& c, const TomDer& d, double now, uint32_t k) {
   TomFront f;
-  f.env = maxenv_value_pure(c.env, now);
+  f.env = maxenv_value_pure(c.env, d.ek, now);
   uint64_t counter = (uint64_t)(k - c.trig_k) + 1ull;
   f.noise = hash_noise(counter);
   f.rnd = hash_noise(counter + 0x12345678ull);
