@@ -92,9 +92,22 @@ int gooey_voice_batch_render_device(GooeyVoiceBatch* b, uint32_t frames, float* 
  * One GooeyRsBatch holds n independent `Engine`s.  Per engine: named instruments (`Engine::add_instrument(name,
  * Box::new(<Voice>::with_config(sr, cfg)))`), sequencers that name their instrument (`Sequencer::with_pattern /
  * with_velocity_pattern(bpm, sr, pattern, name)`), `set_bpm`, `set_master_gain` (default 0.25) and the global effect chain,
- * which starts as [SoftLimiter(1.0)] (`clear_global_effects`, `add_global_effect(SoftLimiter::new(th))`).
+ * which starts as [SoftLimiter(1.0)] (`clear_global_effects`, `add_global_effect(effect)`).
  * gooey_rs_batch_bounce = `bounce_to_buffer(&mut engine, BounceLength::Samples(samples))` of every engine in one device
- * pass: out_host[engine * samples + i], mono.  Bars / Beats lengths are converted by the host mirror (bounce.rs:20-32). */
+ * pass: out_host[engine * samples + i], mono.  Bars / Beats lengths are converted by the host mirror (bounce.rs:20-32).
+ *
+ * Global effects: gooey_rs_batch_add_effect appends `effect_id` (the FFI effect ids of gooey.h) built at the batch's
+ * sample rate from its constructor arguments after the sample rate, in the reference's order:
+ *   0 LowpassFilterEffect (cutoff, resonance) · 1 DelayEffect (timing = DelayTiming index, bpm, feedback, mix, cutoff) ·
+ *   2 TubeSaturation (drive, warmth, mix) · 3 TubeCompressor (threshold dB, ratio, attack ms, release ms, mix) ·
+ *   4 TiltFilterEffect () · 5 SoftLimiter (threshold) · 6 SpringReverbEffect (decay, mix, damping) ·
+ *   7 Waveshaper (drive, mix) · 8 FeedbackWaveshaper (drive, feedback, cutoff, mix) · 9 PlateReverbEffect (decay, mix, damping).
+ * Each effect runs its mono `process` (the channel-0 path; the compressor is its own side-chain).  Effects keep their
+ * state from one bounce to the next; clear_global_effects drops them.  set_bpm does not reach a DelayEffect: it keeps
+ * the tempo it was built with.  GOOEY_E_INVALID (chain unchanged) for a bad engine, an unknown id, n_args other than
+ * the kind's count, NULL args with n_args > 0, or a chain already GOOEY_RS_MAX_EFFECTS long.
+ * gooey_rs_batch_add_limiter(b, e, th) = gooey_rs_batch_add_effect(b, e, 5, &th, 1). */
+#define GOOEY_RS_MAX_EFFECTS 8
 typedef struct GooeyRsBatch GooeyRsBatch;
 int gooey_rs_batch_new(float sample_rate, uint32_t n_engines, int device, GooeyRsBatch** out_batch);
 void gooey_rs_batch_free(GooeyRsBatch* b);
@@ -106,6 +119,7 @@ float gooey_rs_batch_get_bpm(const GooeyRsBatch* b, uint32_t engine);
 int gooey_rs_batch_set_master_gain(GooeyRsBatch* b, uint32_t engine, float gain);
 int gooey_rs_batch_clear_global_effects(GooeyRsBatch* b, uint32_t engine);
 int gooey_rs_batch_add_limiter(GooeyRsBatch* b, uint32_t engine, float threshold);
+int gooey_rs_batch_add_effect(GooeyRsBatch* b, uint32_t engine, uint32_t effect_id, const float* args, uint32_t n_args);
 int gooey_rs_batch_bounce(GooeyRsBatch* b, uint32_t samples, float* out_host);
 int gooey_rs_batch_bounce_device(GooeyRsBatch* b, uint32_t samples, float* out_dev, size_t stride);
 /* Mono PCM WAV writer of bounce_to_wav (bounce.rs:80-133; ffi.rs:7942-7980): bit_depth 16 or 24, sample = round(s * (2^(bits-1) - 1)). */

@@ -37,6 +37,7 @@ def _L():
         L.gooey_rs_batch_set_master_gain.argtypes = [c.c_void_p, c.c_uint32, c.c_float]
         L.gooey_rs_batch_clear_global_effects.argtypes = [c.c_void_p, c.c_uint32]
         L.gooey_rs_batch_add_limiter.argtypes = [c.c_void_p, c.c_uint32, c.c_float]
+        L.gooey_rs_batch_add_effect.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_void_p, c.c_uint32]
         L.gooey_rs_batch_bounce.argtypes = [c.c_void_p, c.c_uint32, c.c_void_p]
         L.gooey_rs_batch_bounce_device.argtypes = [c.c_void_p, c.c_uint32, c.c_void_p, c.c_size_t]
         L.gooey_b200_write_wav.argtypes = [c.c_char_p, c.c_void_p, c.c_uint32, c.c_uint32, c.c_uint32]
@@ -145,11 +146,96 @@ def BassSynth(sample_rate=44100.0, config=None):
     return _Instrument(V.BASS, cfg)
 
 
-class SoftLimiter:
+class _GlobalEffect:
+    """A global effect as its constructor describes it: the FFI effect id (include/gooey.h) and the constructor arguments
+    after the sample rate, in the reference's order.  ``sample_rate`` is None for types built without one."""
+    ID = None
+    sample_rate = None
+
+    def ffi(self):
+        return self.ID, [float(a) for a in self.args]
+
+
+class LowpassFilterEffect(_GlobalEffect):
+    """effects/lowpass_filter.rs:55-81."""
+    ID = 0
+
+    def __init__(self, sample_rate, cutoff, resonance):
+        self.sample_rate, self.args = float(sample_rate), (cutoff, resonance)
+
+
+class DelayEffect(_GlobalEffect):
+    """effects/delay.rs: ``timing`` is the DelayTiming index (0 whole, 1 half, 2 quarter, 3 eighth, 4 sixteenth,
+    5-7 triplets, 8 sixteenth triplet).  The delay keeps the tempo it was built with."""
+    ID = 1
+
+    def __init__(self, sample_rate, timing, bpm, feedback, mix, cutoff):
+        self.sample_rate, self.args = float(sample_rate), (int(timing), bpm, feedback, mix, cutoff)
+
+
+class TubeSaturation(_GlobalEffect):
+    """effects/saturation.rs:68-91."""
+    ID = 2
+
+    def __init__(self, sample_rate, drive, warmth, mix):
+        self.sample_rate, self.args = float(sample_rate), (drive, warmth, mix)
+
+
+class TubeCompressor(_GlobalEffect):
+    """effects/compressor.rs:55-96 (threshold dB, ratio, attack ms, release ms, mix)."""
+    ID = 3
+
+    def __init__(self, sample_rate, threshold, ratio, attack, release, mix):
+        self.sample_rate, self.args = float(sample_rate), (threshold, ratio, attack, release, mix)
+
+
+class TiltFilterEffect(_GlobalEffect):
+    """effects/tilt_filter.rs."""
+    ID = 4
+
+    def __init__(self, sample_rate):
+        self.sample_rate, self.args = float(sample_rate), ()
+
+
+class SoftLimiter(_GlobalEffect):
     """effects/limiter.rs:43-78."""
+    ID = 5
 
     def __init__(self, threshold=1.0):
         self.threshold = float(threshold)
+        self.args = (self.threshold,)
+
+
+class SpringReverbEffect(_GlobalEffect):
+    """effects/reverb.rs."""
+    ID = 6
+
+    def __init__(self, sample_rate, decay, mix, damping):
+        self.sample_rate, self.args = float(sample_rate), (decay, mix, damping)
+
+
+class Waveshaper(_GlobalEffect):
+    """effects/waveshaper.rs."""
+    ID = 7
+
+    def __init__(self, drive, mix):
+        self.args = (drive, mix)
+
+
+class FeedbackWaveshaper(_GlobalEffect):
+    """effects/feedback_waveshaper.rs."""
+    ID = 8
+
+    def __init__(self, sample_rate, drive, feedback, cutoff, mix):
+        self.sample_rate, self.args = float(sample_rate), (drive, feedback, cutoff, mix)
+
+
+class PlateReverbEffect(_GlobalEffect):
+    """effects/plate_reverb.rs."""
+    ID = 9
+
+    def __init__(self, sample_rate, decay, mix, damping):
+        self.sample_rate, self.args = float(sample_rate), (decay, mix, damping)
 
 
 class EngineBatch:
@@ -227,9 +313,15 @@ class Engine:
         check(_L().gooey_rs_batch_clear_global_effects(self._batch._h, self._i))
 
     def add_global_effect(self, effect):
-        if not isinstance(effect, SoftLimiter):
-            raise GooeyError("this build supports SoftLimiter in the Rust-API global chain; use the FFI engine for delay / reverb / tilt")
-        check(_L().gooey_rs_batch_add_limiter(self._batch._h, self._i, c.c_float(effect.threshold)))
+        """Appends ``effect`` to the global chain.  The device builds it at the batch's sample rate, so an effect
+        constructed for another rate is refused rather than rendered differently."""
+        if not isinstance(effect, _GlobalEffect):
+            raise GooeyError(f"not a global effect: {type(effect).__name__}")
+        if effect.sample_rate is not None and np.float32(effect.sample_rate) != np.float32(self._batch.sample_rate):
+            raise GooeyError(f"{type(effect).__name__} built at {effect.sample_rate} Hz for an engine at {self._batch.sample_rate} Hz")
+        eid, args = effect.ffi()
+        a = np.array(args, np.float32)
+        check(_L().gooey_rs_batch_add_effect(self._batch._h, self._i, eid, a.ctypes.data if len(a) else None, len(a)))
 
 
 def bounce_to_buffer(engine, length):

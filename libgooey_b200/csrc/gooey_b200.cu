@@ -1,11 +1,12 @@
 // gooey_b200.cu — libgooey_b200.so: the C ABI (include/gooey_batch.h, include/gooey.h)
-// over the sm_100a kernels.  Single translation unit: the kernels are header
-// templates (kernels.cuh), this file instantiates them and owns the host side.
+// over the sm_100a kernels.  The kernels are header templates (kernels.cuh); this file instantiates them and owns the
+// host side.  The Rust-API effect chain's kernels are compiled apart, in rs_chain.cu.
 #include <mutex>
 #include <memory>
 #include "pool.cuh"
 #include "patch.h"
 #include "halfband_design.h"
+#include "rs_chain.cuh"
 
 namespace gh {
 
@@ -56,6 +57,7 @@ static void use_device(int device) {
     float hb[8];
     gd::design_halfband8(hb);
     GH_CUDA(cudaMemcpyToSymbol(gd::c_hb, hb, sizeof hb));
+    gd::rs_chain_set_halfband(hb);
     {
       static float inv_sq[gd::INV_SQ_N];
       for (int k = 0; k < gd::INV_SQ_N; k++) { volatile float fi = (float)(2 * k + 1); volatile float sq = fi * fi; inv_sq[k] = 1.0f / sq; }

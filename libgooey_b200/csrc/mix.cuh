@@ -653,6 +653,7 @@ __device__ __forceinline__ void mix_event(MixState& s, const MixCfg& cfg, const 
   }
 }
 
+#ifndef GOOEY_RS_CHAIN_TU   // rs_chain.cu compiles only its own kernels
 // One engine per thread.  Voice rows come in and the mix goes out through 32 engines x 32 frames shared-memory tiles,
 // so every global access is a 128-byte row segment.
 constexpr int MIX_CH = 7;
@@ -995,6 +996,7 @@ __global__ void __launch_bounds__(256) quantize_pcm16_kernel(const float* __rest
     *reinterpret_cast<short4*>(dst) = q;
   } else for (int k = 0; k < nq; k++) dst[k] = pcm16_of(src[k]);
 }
+#endif  // GOOEY_RS_CHAIN_TU
 #endif  // __CUDACC__
 
 }  // namespace gd

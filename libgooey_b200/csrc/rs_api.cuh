@@ -6,8 +6,11 @@
 // and starts the sequencers, snaps the master gain, and calls tick N times with an f64 clock starting at 0.
 // Here thousands of such engines are bounced in one pass: the host resolves every sequencer into trigger events, the
 // voice kernels render every instrument of every engine, and rs_mix_kernel does the per-engine sum / master / limiter.
+// Engines whose chain holds anything but at most RS_MAX_LIM limiters get 0 limiters there, and rs_chain_kernel
+// (rs_chain.cuh) runs their whole chain afterwards.
 #pragma once
 #include "engine.cuh"
+#include "rs_chain.cuh"
 #include "../../include/gooey_batch.h"
 
 namespace gd {
@@ -21,6 +24,7 @@ struct RsMixLaunch {
   float* out; long long out_stride; int frames; int n_engines;
 };
 constexpr int RS_MAX_LIM = 4;
+static_assert(GOOEY_RS_MAX_EFFECTS == RS_MAX_FX, "the C ABI's chain length is the kernel's");
 
 // One thread per (engine, 4 frames): the voice rows of an engine are summed in insertion order (the reference iterates a
 // HashMap, whose order is unspecified), `+ 0.0` for the empty loop mixer, master gain, limiters.
@@ -59,26 +63,114 @@ struct GooeyRsBatch {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   struct Inst { std::string name; uint32_t type; uint32_t slot; };
   struct Seq { gh::HostSeq seq; std::string target; };
+  struct Fx { uint32_t kind; gd::FxDyn init; };                    // the effect as its constructor left it
   struct Eng {
     float bpm = 120.0f;
     std::vector<Inst> insts;
     std::vector<Seq> seqs;
     float master_cur = 0.25f, master_tgt = 0.25f;                 // SmoothedParam(0.25, 0, 2, sr, 30 ms)
-    std::vector<float> limiters = std::vector<float>(1, 1.0f);    // Engine::new pushes SoftLimiter(1.0)
+    std::vector<Fx> fx;
+    uint32_t fresh = 0;                                           // bit k: position k was constructed since it last reached the state pool
+    Eng() { const float one = 1.0f; Fx f; f.kind = gd::FXK_LIMITER; gd::rs_fx_construct(f.init, f.kind, &one, 0.0f); fx.push_back(f); fresh = 1; }   // Engine::new pushes SoftLimiter(1.0)
+    bool limiter_only() const { if (fx.size() > (size_t)gd::RS_MAX_LIM) return false; for (const Fx& f : fx) if (f.kind != gd::FXK_LIMITER) return false; return true; }
   };
   std::vector<Eng> engines;
   gh::VoiceBank bank;
   gh::ClockWindow clock;
   gh::DevBuf<float> d_voices, d_out, d_master, d_lim_th, d_lim_inv;
   gh::DevBuf<uint32_t> d_first, d_nlim;
+  // global effect chains (rs_chain.cuh): the state pool [engine][position] and one ring arena per position, [word][ring_pitch]
+  gd::FxGeom geo;
+  gh::DevBuf<gd::FxDyn> d_fx_state, d_fx_fresh;
+  gh::DevBuf<float> ring[gd::RS_MAX_FX]; uint32_t ring_words[gd::RS_MAX_FX] = {0}; long long ring_pitch = 0;
+  gh::DevBuf<uint32_t> d_chain_rows, d_chain_nfx, d_fx_where, d_ring_clear;
+  gh::DevBuf<uint8_t> d_chain_kinds;
+  cudaEvent_t ev_c0 = nullptr, ev_c1 = nullptr;
+  double chain_units = 0.0;                                       // engine-frames of the last bounce's rs_chain_kernel (0: not launched)
+  // arena `k` grows to `words` words per engine, keeping what it holds
+  void ensure_ring(int k, uint32_t words) {
+    if (words <= ring_words[k]) return;
+    gh::DevBuf<float> nb;
+    nb.alloc((size_t)words * (size_t)ring_pitch);
+    GH_CUDA(cudaMemsetAsync(nb.p, 0, (size_t)words * (size_t)ring_pitch * 4, stream));
+    if (ring_words[k]) GH_CUDA(cudaMemcpyAsync(nb.p, ring[k].p, (size_t)ring_words[k] * (size_t)ring_pitch * 4, cudaMemcpyDeviceToDevice, stream));
+    GH_CUDA(cudaStreamSynchronize(stream));
+    std::swap(ring[k].p, nb.p); std::swap(ring[k].n, nb.n);
+    ring_words[k] = words;
+  }
   ~GooeyRsBatch() {
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
+    if (ev_c0) cudaEventDestroy(ev_c0);
+    if (ev_c1) cudaEventDestroy(ev_c1);
     if (stream) cudaStreamDestroy(stream);
   }
 };
 
 namespace gh {
+
+// Lays out the chain engines for rs_chain_kernel (warps of one signature, padded with ~0u), grows the ring arenas to
+// the kinds each position holds, and moves the effects constructed since the last bounce into the state pool with
+// their ring columns zeroed.  Returns the number of warps (0: no engine has a chain beyond limiters).
+static uint32_t chain_prepare(GooeyRsBatch* b, const std::map<std::vector<uint8_t>, std::vector<uint32_t>>& chains) {
+  if (chains.empty()) return 0;
+  cudaStream_t st = b->stream;
+  const uint32_t ne = (uint32_t)b->engines.size();
+  if (!b->d_fx_state.p) {
+    b->ring_pitch = (((long long)ne + 31) / 32) * 32;
+    if ((b->ring_pitch / 32) % 2 == 0) b->ring_pitch += 32;        // odd multiple of 32 (DESIGN §3)
+    b->d_fx_state.alloc((size_t)ne * gd::RS_MAX_FX);
+    b->geo = make_fx_geom(b->sr);
+    GH_CUDA(cudaEventCreate(&b->ev_c0));
+    GH_CUDA(cudaEventCreate(&b->ev_c1));
+  }
+  std::vector<uint32_t> rows, nfx, where;
+  std::vector<uint8_t> kinds;
+  std::vector<gd::FxDyn> fresh;
+  std::vector<uint32_t> need(gd::RS_MAX_FX, 0);
+  std::vector<std::vector<uint32_t>> clear(gd::RS_MAX_FX);
+  for (const auto& c : chains) {
+    const std::vector<uint8_t>& sig = c.first;
+    for (size_t k = 0; k < sig.size(); k++) need[k] = std::max(need[k], gd::rs_fx_ring_words(b->geo, sig[k]));
+    for (size_t i = 0; i < c.second.size(); i += 32) {
+      for (size_t j = 0; j < 32; j++) rows.push_back(i + j < c.second.size() ? c.second[i + j] : ~0u);
+      nfx.push_back((uint32_t)sig.size());
+      for (int k = 0; k < gd::RS_MAX_FX; k++) kinds.push_back(k < (int)sig.size() ? sig[k] : (uint8_t)gd::FXK_NONE);
+    }
+    for (uint32_t e : c.second) {
+      GooeyRsBatch::Eng& E = b->engines[e];
+      for (size_t k = 0; k < E.fx.size(); k++) {
+        if (!((E.fresh >> k) & 1u)) continue;
+        fresh.push_back(E.fx[k].init);
+        where.push_back(e * gd::RS_MAX_FX + (uint32_t)k);
+        if (gd::rs_fx_ring_words(b->geo, E.fx[k].kind)) clear[k].push_back(e);
+      }
+      E.fresh = 0;
+    }
+  }
+  for (int k = 0; k < gd::RS_MAX_FX; k++) b->ensure_ring(k, need[k]);
+  for (int k = 0; k < gd::RS_MAX_FX; k++) {
+    if (clear[k].empty()) continue;
+    b->d_ring_clear.upload(clear[k].data(), clear[k].size(), st);
+    const int n = (int)clear[k].size();
+    ring_clear_kernel<<<dim3((n + 127) / 128, std::min<uint32_t>(b->ring_words[k], 4096u)), 128, 0, st>>>(b->ring[k].p, b->ring_pitch, b->ring_words[k], b->d_ring_clear.p, n);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    GH_CUDA(cudaGetLastError());
+    GH_CUDA(cudaStreamSynchronize(st));     // d_ring_clear is reused by the next position
+  }
+  if (!fresh.empty()) {
+    b->d_fx_fresh.upload(fresh.data(), fresh.size(), st);
+    b->d_fx_where.upload(where.data(), where.size(), st);
+    const int n = (int)fresh.size();
+    gd::rs_fx_init_launch(b->d_fx_state.p, b->d_fx_fresh.p, b->d_fx_where.p, n, st);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    GH_CUDA(cudaGetLastError());
+  }
+  b->d_chain_rows.upload(rows.data(), rows.size(), st);
+  b->d_chain_nfx.upload(nfx.data(), nfx.size(), st);
+  b->d_chain_kinds.upload(kinds.data(), kinds.size(), st);
+  return (uint32_t)nfx.size();
+}
 
 static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, size_t out_stride) {
   use_device(b->device);
@@ -89,15 +181,23 @@ static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, siz
   std::vector<uint32_t> first(ne + 1, 0), nlim(ne);
   std::vector<float> master(ne), lth((size_t)ne * gd::RS_MAX_LIM, 1.0f), linv((size_t)ne * gd::RS_MAX_LIM, 1.0f);
   std::vector<SeqFire> fires;
+  std::map<std::vector<uint8_t>, std::vector<uint32_t>> chains;   // chain signature -> its engines
   uint32_t row = 0;
   for (uint32_t e = 0; e < ne; e++) {
     GooeyRsBatch::Eng& E = b->engines[e];
     first[e] = row;
-    // prepare_for_bounce (engine/mod.rs:464-477): sequencers reset + start, master gain snapped
+    // prepare_for_bounce (engine/mod.rs:464-477): sequencers reset + start, master gain snapped; the effects are left as they are
     E.master_cur = E.master_tgt;
     master[e] = E.master_cur;
-    nlim[e] = (uint32_t)E.limiters.size();
-    for (size_t k = 0; k < E.limiters.size(); k++) { const float th = fmaxf(E.limiters[k], 0.001f); lth[e * gd::RS_MAX_LIM + k] = th; linv[e * gd::RS_MAX_LIM + k] = 1.0f / th; }
+    if (E.limiter_only()) {
+      nlim[e] = (uint32_t)E.fx.size();
+      for (size_t k = 0; k < E.fx.size(); k++) { memcpy(&lth[e * gd::RS_MAX_LIM + k], &E.fx[k].init.w[0], 4); memcpy(&linv[e * gd::RS_MAX_LIM + k], &E.fx[k].init.w[1], 4); }
+    } else {
+      nlim[e] = 0;
+      std::vector<uint8_t> sig;
+      for (const auto& f : E.fx) sig.push_back((uint8_t)f.kind);
+      chains[sig].push_back(e);
+    }
     std::vector<std::vector<gd::VoiceEvent>> ev(E.insts.size());
     for (auto& x : ev) x.push_back(make_event(0, gd::EV_SET_TIME, 0, 0.0f, 0));
     for (auto& s : E.seqs) {
@@ -123,6 +223,7 @@ static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, siz
   b->d_master.upload(master.data(), master.size(), st);
   b->d_lim_th.upload(lth.data(), lth.size(), st);
   b->d_lim_inv.upload(linv.data(), linv.size(), st);
+  const uint32_t n_chain_warps = chain_prepare(b, chains);
   GH_CUDA(cudaStreamSynchronize(st));   // the host vectors above are temporaries
   GH_CUDA(cudaEventRecord(b->ev0, st));
   b->bank.launch(st, b->ev0, b->rc, tt, (int)frames, b->d_voices.p, (long long)vstride);
@@ -134,7 +235,34 @@ static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, siz
   gd::rs_mix_kernel<<<grid, 256, 0, st>>>(M);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   GH_CUDA(cudaGetLastError());
+  b->chain_units = 0.0;
+  if (n_chain_warps) {
+    gd::RsChainLaunch C;
+    C.out = out_dev; C.out_stride = (long long)out_stride; C.frames = (int)frames;
+    C.rows = b->d_chain_rows.p; C.warp_kinds = b->d_chain_kinds.p; C.warp_nfx = b->d_chain_nfx.p;
+    C.state = b->d_fx_state.p;
+    for (int k = 0; k < gd::RS_MAX_FX; k++) C.ring[k] = b->ring[k].p;
+    C.ring_pitch = b->ring_pitch; C.rc = b->rc; C.geo = b->geo;
+    GH_CUDA(cudaEventRecord(b->ev_c0, st));
+    gd::rs_chain_launch(C, n_chain_warps, st);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    GH_CUDA(cudaGetLastError());
+    GH_CUDA(cudaEventRecord(b->ev_c1, st));
+    size_t n = 0;
+    for (const auto& c : chains) n += c.second.size();
+    b->chain_units = (double)n * frames;
+  }
   GH_CUDA(cudaEventRecord(b->ev1, st));
+}
+// after the stream has been synchronised: the chain kernel's time and engine-frames into the kernel statistics
+static void rs_collect_stats(GooeyRsBatch* b) {
+  if (b->chain_units == 0.0) return;
+  float ms = 0.0f;
+  GH_CUDA(cudaEventElapsedTime(&ms, b->ev_c0, b->ev_c1));
+  std::lock_guard<std::mutex> lk(kernel_stats_mutex());
+  KernelStat& k = kernel_stats()["rs_chain_kernel"];
+  k.launches++; k.ms += ms; k.voice_frames += b->chain_units;
+  b->chain_units = 0.0;
 }
 
 }  // namespace gh
@@ -201,15 +329,23 @@ int gooey_rs_batch_set_master_gain(GooeyRsBatch* b, uint32_t engine, float gain)
   return GOOEY_E_OK;
   GOOEY_CATCH
 }
-int gooey_rs_batch_clear_global_effects(GooeyRsBatch* b, uint32_t engine) { GOOEY_TRY RS_ENGINE(b, engine); E.limiters.clear(); return GOOEY_E_OK; GOOEY_CATCH }
-int gooey_rs_batch_add_limiter(GooeyRsBatch* b, uint32_t engine, float threshold) {
+int gooey_rs_batch_clear_global_effects(GooeyRsBatch* b, uint32_t engine) { GOOEY_TRY RS_ENGINE(b, engine); E.fx.clear(); E.fresh = 0; return GOOEY_E_OK; GOOEY_CATCH }
+int gooey_rs_batch_add_effect(GooeyRsBatch* b, uint32_t engine, uint32_t effect_id, const float* args, uint32_t n_args) {
   GOOEY_TRY
   RS_ENGINE(b, engine);
-  if (E.limiters.size() >= (size_t)gd::RS_MAX_LIM) { set_error("too many global effects"); return GOOEY_E_INVALID; }
-  E.limiters.push_back(threshold);
+  if (effect_id >= 10) { set_error("unknown global effect id"); return GOOEY_E_INVALID; }
+  if (n_args != gd::RS_FX_ARGS[effect_id]) { set_error("wrong number of constructor arguments for this global effect"); return GOOEY_E_INVALID; }
+  if (!args && n_args) { set_error("null argument"); return GOOEY_E_INVALID; }
+  if (E.fx.size() >= (size_t)gd::RS_MAX_FX) { set_error("too many global effects"); return GOOEY_E_INVALID; }
+  GooeyRsBatch::Fx f;
+  f.kind = effect_id;
+  gd::rs_fx_construct(f.init, effect_id, args, b->sr);
+  E.fresh |= 1u << E.fx.size();
+  E.fx.push_back(f);
   return GOOEY_E_OK;
   GOOEY_CATCH
 }
+int gooey_rs_batch_add_limiter(GooeyRsBatch* b, uint32_t engine, float threshold) { return gooey_rs_batch_add_effect(b, engine, gd::FXK_LIMITER, &threshold, 1); }
 int gooey_rs_batch_bounce_device(GooeyRsBatch* b, uint32_t samples, float* out_dev, size_t stride) {
   GOOEY_TRY
   if (!b || !out_dev || stride < samples) { set_error("bad arguments"); return GOOEY_E_INVALID; }
@@ -217,6 +353,7 @@ int gooey_rs_batch_bounce_device(GooeyRsBatch* b, uint32_t samples, float* out_d
   rs_bounce_impl(b, samples, out_dev, stride);
   GH_CUDA(cudaStreamSynchronize(b->stream));
   GH_CUDA(cudaEventElapsedTime(&gh::g_last_kernel_ms, b->ev0, b->ev1));
+  gh::rs_collect_stats(b);
   return GOOEY_E_OK;
   GOOEY_CATCH
 }
@@ -231,6 +368,7 @@ int gooey_rs_batch_bounce(GooeyRsBatch* b, uint32_t samples, float* out_host) {
   GH_CUDA(cudaMemcpy2DAsync(out_host, (size_t)samples * 4, b->d_out.p, stride * 4, (size_t)samples * 4, b->engines.size(), cudaMemcpyDeviceToHost, b->stream));
   GH_CUDA(cudaStreamSynchronize(b->stream));
   GH_CUDA(cudaEventElapsedTime(&gh::g_last_kernel_ms, b->ev0, b->ev1));
+  gh::rs_collect_stats(b);
   return GOOEY_E_OK;
   GOOEY_CATCH
 }

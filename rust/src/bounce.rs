@@ -45,13 +45,48 @@ pub struct EngineSpec {
     pub instruments: Vec<(String, GooeyVoicePatch)>,
     pub sequencers: Vec<SequencerSpec>,
     pub master_gain: f32,
-    /// thresholds of the SoftLimiters in the global chain; `Engine::new` starts with `[1.0]`
-    pub limiters: Vec<f32>,
+    /// the global chain in order; `Engine::new` starts with `[SoftLimiter(1.0)]`
+    pub global_effects: Vec<GlobalEffect>,
 }
 
 impl EngineSpec {
     pub fn new() -> Self {
-        Self { bpm: 120.0, instruments: Vec::new(), sequencers: Vec::new(), master_gain: 0.25, limiters: vec![1.0] }
+        Self { bpm: 120.0, instruments: Vec::new(), sequencers: Vec::new(), master_gain: 0.25, global_effects: vec![GlobalEffect::SoftLimiter(1.0)] }
+    }
+}
+
+/// One global effect, by its reference type and constructor arguments after the sample rate (the device builds it at
+/// the batch's sample rate).  `DelayEffect`'s first argument is the `DelayTiming` index (3 = eighth).
+#[derive(Clone, Copy, Debug)]
+pub enum GlobalEffect {
+    LowpassFilterEffect { cutoff: f32, resonance: f32 },
+    DelayEffect { timing: u32, bpm: f32, feedback: f32, mix: f32, cutoff: f32 },
+    TubeSaturation { drive: f32, warmth: f32, mix: f32 },
+    TubeCompressor { threshold_db: f32, ratio: f32, attack_ms: f32, release_ms: f32, mix: f32 },
+    TiltFilterEffect,
+    SoftLimiter(f32),
+    SpringReverbEffect { decay: f32, mix: f32, damping: f32 },
+    Waveshaper { drive: f32, mix: f32 },
+    FeedbackWaveshaper { drive: f32, feedback: f32, cutoff: f32, mix: f32 },
+    PlateReverbEffect { decay: f32, mix: f32, damping: f32 },
+}
+
+impl GlobalEffect {
+    /// (FFI effect id, constructor arguments) as `gooey_rs_batch_add_effect` takes them
+    fn ffi(&self) -> (u32, Vec<f32>) {
+        use GlobalEffect::*;
+        match *self {
+            LowpassFilterEffect { cutoff, resonance } => (0, vec![cutoff, resonance]),
+            DelayEffect { timing, bpm, feedback, mix, cutoff } => (1, vec![timing as f32, bpm, feedback, mix, cutoff]),
+            TubeSaturation { drive, warmth, mix } => (2, vec![drive, warmth, mix]),
+            TubeCompressor { threshold_db, ratio, attack_ms, release_ms, mix } => (3, vec![threshold_db, ratio, attack_ms, release_ms, mix]),
+            TiltFilterEffect => (4, vec![]),
+            SoftLimiter(threshold) => (5, vec![threshold]),
+            SpringReverbEffect { decay, mix, damping } => (6, vec![decay, mix, damping]),
+            Waveshaper { drive, mix } => (7, vec![drive, mix]),
+            FeedbackWaveshaper { drive, feedback, cutoff, mix } => (8, vec![drive, feedback, cutoff, mix]),
+            PlateReverbEffect { decay, mix, damping } => (9, vec![decay, mix, damping]),
+        }
     }
 }
 
@@ -82,8 +117,9 @@ impl EngineBatch {
             }
             check(unsafe { gooey_rs_batch_set_master_gain(raw, e, s.master_gain) })?;
             check(unsafe { gooey_rs_batch_clear_global_effects(raw, e) })?;
-            for th in &s.limiters {
-                check(unsafe { gooey_rs_batch_add_limiter(raw, e, *th) })?;
+            for fx in &s.global_effects {
+                let (id, args) = fx.ffi();
+                check(unsafe { gooey_rs_batch_add_effect(raw, e, id, args.as_ptr(), args.len() as u32) })?;
             }
         }
         Ok(batch)

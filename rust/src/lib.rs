@@ -3,7 +3,7 @@
 //!
 //! The reference resolves nothing ahead of time: `Engine::tick` walks sequencers and instruments sample by sample.
 //! Here the host describes each engine (instruments as `with_config` argument lists, sequencer patterns, master gain,
-//! limiter chain) once; the library resolves the sequencer schedule into per-voice trigger tables (bit-exact with
+//! global effect chain) once; the library resolves the sequencer schedule into per-voice trigger tables (bit-exact with
 //! `Sequencer::tick_with_settings`) and renders every engine of the batch in one pass on a B200.
 //!
 //! This crate cannot be compiled in the repository's own image (no Rust toolchain there); it is the binding a libgooey
@@ -51,6 +51,7 @@ extern "C" {
     pub fn gooey_rs_batch_set_master_gain(b: *mut GooeyRsBatch, engine: u32, gain: c_float) -> c_int;
     pub fn gooey_rs_batch_clear_global_effects(b: *mut GooeyRsBatch, engine: u32) -> c_int;
     pub fn gooey_rs_batch_add_limiter(b: *mut GooeyRsBatch, engine: u32, threshold: c_float) -> c_int;
+    pub fn gooey_rs_batch_add_effect(b: *mut GooeyRsBatch, engine: u32, effect_id: u32, args: *const c_float, n_args: u32) -> c_int;
     pub fn gooey_rs_batch_bounce(b: *mut GooeyRsBatch, samples: u32, out_host: *mut c_float) -> c_int;
 
     pub fn gooey_voice_batch_new(sample_rate: c_float, n: u32, patches: *const GooeyVoicePatch, device: c_int, out: *mut *mut GooeyVoiceBatch) -> c_int;
