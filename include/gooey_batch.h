@@ -34,7 +34,8 @@ extern "C" {
 #define GOOEY_INSTRUMENT_BASS 4u
 /* libgooey_b200 voice kinds beyond the five sequenced instruments (GooeyVoicePatch.instrument):
  * the poly synth (params = PolyConfig, 14 normalized values, src/instruments/poly_synth.rs:20-47) and the granulator
- * (GranulatorConfig::default; buffer and parameters arrive as events). */
+ * (GranulatorConfig::default; buffer, seed and parameters arrive as events: gooey_voice_batch_set_buffer / _share_buffer /
+ * _set_seed / _set_param below). */
 #define GOOEY_B200_VOICE_POLY 5u
 #define GOOEY_B200_VOICE_GRANULATOR 6u
 
@@ -64,8 +65,10 @@ int gooey_b200_device_count(void);
 uint64_t gooey_b200_launch_count(void);
 /* Device time (ms, CUDA events on the launching stream) of the most recent render call's kernels. */
 float gooey_b200_last_kernel_ms(void);
-/* Accumulated device time of one back-end kernel ("wave_kernel<KickW>" / "<SnareW>" / "<HatW>" / "<TomW>") since load or
- * the last reset: launches, summed launch durations (ms, CUDA events on the launching stream) and voice-frames written. */
+/* Accumulated device time of one back-end kernel ("wave_kernel<KickW>" / "<SnareW>" / "<HatW>" / "<TomW>",
+ * "coop_kernel<TomC>", "back_kernel", and for poly synths "poly_wave_kernel" or, under GOOEY_B200_BACKEND=serial,
+ * "slow_kernel<PolyV>") since load or the last reset: launches, summed launch durations (ms, CUDA events on the launching
+ * stream) and voice-frames written. */
 int gooey_b200_kernel_stat(const char* kernel, uint64_t* launches, double* total_ms, double* voice_frames);
 /* ';'-separated names of the kernels that have statistics (thread-local storage, valid until the next call) */
 const char* gooey_b200_kernel_stat_names(void);
@@ -75,12 +78,34 @@ void gooey_b200_kernel_stats_reset(void);
 int gooey_voice_batch_new(float sample_rate, uint32_t n_voices, const GooeyVoicePatch* patches, int device,
                           GooeyVoiceBatch** out_batch);
 void gooey_voice_batch_free(GooeyVoiceBatch* b);
-/* `voice.trigger_with_velocity(t_frame, velocity)` at frame `frame` (frames count from the batch's current position). */
+/* `voice.trigger_with_velocity(t_frame, velocity)` at frame `frame` (frames count from the batch's current position).
+ * A poly voice has no such trigger and ignores it: it sounds only through gooey_voice_batch_note_on. */
 int gooey_voice_batch_trigger(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, float velocity);
 /* Same trigger for every voice; velocities may be NULL (=1.0). */
 int gooey_voice_batch_trigger_all(GooeyVoiceBatch* b, uint32_t frame, const float* velocities);
-/* FFI-style normalized parameter edit (`gooey_engine_set_*_param` ids) taking effect at `frame`; snap != 0 also snaps. */
+/* FFI-style normalized parameter edit (`gooey_engine_set_*_param` ids) taking effect at `frame`; snap != 0 also snaps.
+ * Poly voices: ids 0-13 = PolySynth::set_param (PolyConfig order); granulators: ids 0-11 as gooey_engine_granulator_set_param
+ * (with snap = gooey_engine_granulator_snap_params).  The value is clamped to 0..1 and glides to its target unless snapped.
+ * Unknown ids are ignored.  (Until libgooey_b200 played poly voices and granulators in batches, this call did nothing for
+ * those two kinds.) */
 int gooey_voice_batch_set_param(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, uint32_t param, float value, int snap);
+/* Poly voices and granulators.  Each call queues its events at `frame`, counted like gooey_voice_batch_trigger's.
+ * GOOEY_E_INVALID, with a message and nothing queued, for a voice out of range, a voice of another kind, or the refusals
+ * named below.
+ *   note_on      PolySynth::trigger_note(note, velocity): note 0-127 (the reference's u8; above 127 is refused), velocity
+ *                unclamped.  A seventh note steals the oldest of the six sub-voices.
+ *   release      PolySynth::release_all.
+ *   set_buffer   Granulator::set_buffer: copies `len` samples at `sample_rate` to the device.  Refused: samples NULL,
+ *                len 0, a non-finite sample, or a sample_rate that is not finite and > 0.  Kills the voice's grains.
+ *   share_buffer libgooey_b200 addition: dst_voice plays the buffer most recently set on or shared to src_voice (also a
+ *                granulator; refused if it holds none) without a second device copy, so 1600 granulators over one 60 s
+ *                source keep one copy.  The batch keeps each buffer while a voice or a queued event refers to it.
+ *   set_seed     Granulator::set_seed (0 selects the reference's fixed non-zero seed). */
+int gooey_voice_batch_note_on(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, uint32_t note, float velocity);
+int gooey_voice_batch_release(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame);
+int gooey_voice_batch_set_buffer(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, const float* samples, uint32_t len, float sample_rate);
+int gooey_voice_batch_share_buffer(GooeyVoiceBatch* b, uint32_t dst_voice, uint32_t frame, uint32_t src_voice);
+int gooey_voice_batch_set_seed(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, uint32_t seed);
 /* Render `frames` samples of every voice: out_host[v * frames + i] (host memory; copies are part of the call). */
 int gooey_voice_batch_render(GooeyVoiceBatch* b, uint32_t frames, float* out_host);
 /* Same as 16-bit PCM, `(s * 32767).round() as i16` (bounce.rs:105-113), quantised on the device: out_host[v * frames + i]. */

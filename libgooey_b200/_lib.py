@@ -49,6 +49,11 @@ def lib():
         L.gooey_voice_batch_trigger.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_float]
         L.gooey_voice_batch_trigger_all.argtypes = [c.c_void_p, c.c_uint32, c.POINTER(c.c_float)]
         L.gooey_voice_batch_set_param.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_uint32, c.c_float, c.c_int]
+        L.gooey_voice_batch_note_on.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_uint32, c.c_float]
+        L.gooey_voice_batch_release.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32]
+        L.gooey_voice_batch_set_buffer.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_void_p, c.c_uint32, c.c_float]
+        L.gooey_voice_batch_share_buffer.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_uint32]
+        L.gooey_voice_batch_set_seed.argtypes = [c.c_void_p, c.c_uint32, c.c_uint32, c.c_uint32]
         L.gooey_voice_batch_render.argtypes = [c.c_void_p, c.c_uint32, c.c_void_p]
         L.gooey_voice_batch_render_device.argtypes = [c.c_void_p, c.c_uint32, c.c_void_p, c.c_size_t]
         _lib = L

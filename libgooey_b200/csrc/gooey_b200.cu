@@ -1,12 +1,14 @@
 // gooey_b200.cu — libgooey_b200.so: the C ABI (include/gooey_batch.h, include/gooey.h)
 // over the sm_100a kernels.  The kernels are header templates (kernels.cuh); this file instantiates them and owns the
-// host side.  The Rust-API effect chain's kernels are compiled apart, in rs_chain.cu.
+// host side.  The Rust-API effect chain's kernels and the poly synth's warp-per-voice kernel are compiled apart, in
+// rs_chain.cu and poly_wave.cu.
 #include <mutex>
 #include <memory>
 #include "pool.cuh"
 #include "patch.h"
 #include "halfband_design.h"
 #include "rs_chain.cuh"
+#include "poly_wave.cuh"
 
 namespace gh {
 
@@ -66,6 +68,7 @@ static void use_device(int device) {
     double mf[128];   // music/note.rs:81-83 midi_to_freq in f64, with the platform libm
     for (int n = 0; n < 128; n++) mf[n] = 440.0 * pow(2.0, ((double)n - 69.0) / 12.0);
     GH_CUDA(cudaMemcpyToSymbol(gd::c_midi_freq, mf, sizeof mf));
+    gd::poly_wave_set_midi_freq(mf);
     g_dev_ready[device] = 1;
   }
 }
@@ -130,7 +133,7 @@ struct VoiceBank {
     grans.launch(parent, start, rc, tt, frames, out, stride);
   }
   // call after the launching stream has been synchronised
-  void collect_stats() { kicks.collect_stats(); snares.collect_stats(); hats.collect_stats(); toms.collect_stats(); }
+  void collect_stats() { kicks.collect_stats(); snares.collect_stats(); hats.collect_stats(); toms.collect_stats(); polys.collect_stats(); }
   // frames per output chunk of the last launch (identical for every bucket) and the per-chunk completion fence
   int chunk_frames(int frames) const { return TypeRunner<gd::KickV>::chunk_of(frames); }
   void wait_chunk(cudaStream_t s, int i) { kicks.wait_chunk(s, i); snares.wait_chunk(s, i); hats.wait_chunk(s, i); toms.wait_chunk(s, i); basses.wait_chunk(s, i); polys.wait_chunk(s, i); grans.wait_chunk(s, i); }
@@ -143,6 +146,11 @@ using namespace gh;
 // =================================================================================================
 // Voice batch
 // =================================================================================================
+namespace gh {
+// A granulator's source buffer as the host hands it to the device: shared by every voice that plays it.
+struct GranSource { std::shared_ptr<DevBuf<float>> buf; uint32_t len = 0; float sr = 0.0f; };
+}  // namespace gh
+
 struct GooeyVoiceBatch {
   int device = 0;
   float sr = 44100.0f;
@@ -155,6 +163,12 @@ struct GooeyVoiceBatch {
   std::vector<uint8_t> vtype;
   std::vector<uint32_t> vslot;
   std::vector<std::vector<gd::VoiceEvent>> pending;   // per voice, frames relative to the next render
+  // Granulator sources per voice.  A buffer stays alive while the device state points at it (gran_live) or a queued
+  // EV_GRAN_BUFFER names it (gran_queued, frames relative to the next render, in call order); gran_latest is the buffer
+  // of the most recent set_buffer / share_buffer call, which share_buffer hands on.
+  std::vector<gh::GranSource> gran_live, gran_latest;
+  std::vector<std::vector<std::pair<uint32_t, gh::GranSource>>> gran_queued;
+  std::vector<gh::GranSource> gran_retired;           // replaced during the last render: freed when the next one starts
   VoiceBank bank;
   DevBuf<float> d_out;
   DevBuf<int16_t> d_pcm;
@@ -173,6 +187,7 @@ static void voice_batch_render_impl(GooeyVoiceBatch* b, uint32_t frames, float* 
   cudaStream_t st = b->stream;
   if ((uint64_t)b->k + frames >= 0xffffffffull) throw std::runtime_error("engine clock index overflow");
   const double* tt = b->clock.view(clock_table(b->sr), b->k, (uint64_t)b->k + frames, st);
+  b->gran_retired.clear();                           // every render call has synchronised its stream before returning
   b->bank.reset();
   std::vector<gd::VoiceEvent> now, later;
   for (uint32_t v = 0; v < b->n; v++) {
@@ -182,6 +197,17 @@ static void voice_batch_render_impl(GooeyVoiceBatch* b, uint32_t frames, float* 
     for (auto& e : ev) { if (e.frame < frames) now.push_back(e); else { e.frame -= frames; later.push_back(e); } }
     b->bank.add(b->vtype[v], b->vslot[v], v, now);
     ev = later;
+    if (!b->gran_queued.empty() && !b->gran_queued[v].empty()) {   // sources whose EV_GRAN_BUFFER this call applies
+      auto& q = b->gran_queued[v];
+      std::stable_sort(q.begin(), q.end(), [](const std::pair<uint32_t, GranSource>& a, const std::pair<uint32_t, GranSource>& c) { return a.first < c.first; });
+      std::vector<std::pair<uint32_t, GranSource>> keep;
+      for (auto& e : q) {
+        if (e.first >= frames) { keep.emplace_back(e.first - frames, e.second); continue; }
+        if (b->gran_live[v].buf) b->gran_retired.push_back(b->gran_live[v]);   // still read before the event's frame
+        b->gran_live[v] = e.second;
+      }
+      q.swap(keep);
+    }
   }
   GH_CUDA(cudaEventRecord(b->ev0, st));
   b->bank.launch(st, b->ev0, b->rc, tt, (int)frames, out_dev, (long long)stride);
@@ -236,6 +262,7 @@ int gooey_voice_batch_new(float sample_rate, uint32_t n_voices, const GooeyVoice
   GH_CUDA(cudaEventCreate(&b->ev0));
   GH_CUDA(cudaEventCreate(&b->ev1));
   b->vtype.resize(n_voices); b->vslot.resize(n_voices); b->pending.resize(n_voices);
+  b->gran_live.resize(n_voices); b->gran_latest.resize(n_voices); b->gran_queued.resize(n_voices);
   for (uint32_t v = 0; v < n_voices; v++) {
     int slot = b->bank.create(patches[v], sample_rate);
     if (slot < 0) { set_error("unsupported instrument id in voice patch"); return GOOEY_E_INVALID; }
@@ -276,6 +303,79 @@ int gooey_voice_batch_set_param(GooeyVoiceBatch* b, uint32_t voice, uint32_t fra
   bool known = ffi_param_to_events(b->vtype[voice], param, value,
                                    [&](uint32_t kind, uint32_t p, float v) { b->pending[voice].push_back(make_event(frame, kind, p, v)); });
   if (known && snap) b->pending[voice].push_back(make_event(frame, gd::EV_SNAP, 0, 0.0f));
+  return GOOEY_E_OK;
+  GOOEY_CATCH
+}
+
+// ---- poly synth and granulator voices: the events of PolySynth::trigger_note / release_all and Granulator::set_buffer /
+// set_seed.  A refused call queues nothing.
+static int voice_of_kind(GooeyVoiceBatch* b, uint32_t voice, uint32_t kind, const char* what) {
+  if (!b || voice >= b->n) { set_error("bad batch/voice"); return GOOEY_E_INVALID; }
+  if (b->vtype[voice] != kind) {
+    set_error(std::string(what) + ": voice " + std::to_string(voice) + " is not a " + (kind == GOOEY_B200_VOICE_POLY ? "poly synth" : "granulator"));
+    return GOOEY_E_INVALID;
+  }
+  return GOOEY_E_OK;
+}
+static void gran_queue(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, const gh::GranSource& src) {   // gran_attach's order (engine_api.cuh)
+  const uint64_t ptr = (uint64_t)(uintptr_t)src.buf->p;
+  float lo; uint32_t lo_bits = (uint32_t)ptr; memcpy(&lo, &lo_bits, 4);
+  b->pending[voice].push_back(make_event(frame, gd::EV_GRAN_BUFFER, 0, lo, (uint32_t)(ptr >> 32)));   // kills all grains, like set_buffer
+  b->pending[voice].push_back(make_event(frame, gd::EV_SET_AUX, gd::AUX_GRAN_BUFINFO, src.sr, src.len));
+  b->gran_queued[voice].emplace_back(frame, src);
+  b->gran_latest[voice] = src;
+}
+
+int gooey_voice_batch_note_on(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, uint32_t note, float velocity) {
+  GOOEY_TRY
+  if (int rc = voice_of_kind(b, voice, GOOEY_B200_VOICE_POLY, "note_on")) return rc;
+  if (note > 127) { set_error("note_on: note " + std::to_string(note) + " is above 127"); return GOOEY_E_INVALID; }
+  b->pending[voice].push_back(make_event(frame, gd::EV_POLY_NOTE, note, velocity));   // velocity as trigger_note takes it: unclamped
+  return GOOEY_E_OK;
+  GOOEY_CATCH
+}
+
+int gooey_voice_batch_release(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame) {
+  GOOEY_TRY
+  if (int rc = voice_of_kind(b, voice, GOOEY_B200_VOICE_POLY, "release")) return rc;
+  b->pending[voice].push_back(make_event(frame, gd::EV_POLY_RELEASE, 0, 0.0f));
+  return GOOEY_E_OK;
+  GOOEY_CATCH
+}
+
+int gooey_voice_batch_set_buffer(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, const float* samples, uint32_t len, float sample_rate) {
+  GOOEY_TRY
+  if (int rc = voice_of_kind(b, voice, GOOEY_B200_VOICE_GRANULATOR, "set_buffer")) return rc;
+  if (!samples || len == 0) { set_error("set_buffer: empty buffer"); return GOOEY_E_INVALID; }
+  if (!std::isfinite(sample_rate) || !(sample_rate > 0.0f)) { set_error("set_buffer: sample_rate must be finite and > 0"); return GOOEY_E_INVALID; }   // SampleBuffer::from_mono
+  for (uint32_t i = 0; i < len; i++)
+    if (!std::isfinite(samples[i])) { set_error("set_buffer: sample " + std::to_string(i) + " is not finite"); return GOOEY_E_INVALID; }
+  use_device(b->device);
+  gh::GranSource src;
+  src.buf = std::make_shared<DevBuf<float>>();
+  src.buf->alloc(len);
+  GH_CUDA(cudaMemcpy(src.buf->p, samples, (size_t)len * 4, cudaMemcpyHostToDevice));
+  src.len = len; src.sr = sample_rate;
+  gran_queue(b, voice, frame, src);
+  return GOOEY_E_OK;
+  GOOEY_CATCH
+}
+
+int gooey_voice_batch_share_buffer(GooeyVoiceBatch* b, uint32_t dst_voice, uint32_t frame, uint32_t src_voice) {
+  GOOEY_TRY
+  if (int rc = voice_of_kind(b, dst_voice, GOOEY_B200_VOICE_GRANULATOR, "share_buffer")) return rc;
+  if (int rc = voice_of_kind(b, src_voice, GOOEY_B200_VOICE_GRANULATOR, "share_buffer")) return rc;
+  if (!b->gran_latest[src_voice].buf) { set_error("share_buffer: voice " + std::to_string(src_voice) + " holds no buffer"); return GOOEY_E_INVALID; }
+  const gh::GranSource src = b->gran_latest[src_voice];
+  gran_queue(b, dst_voice, frame, src);
+  return GOOEY_E_OK;
+  GOOEY_CATCH
+}
+
+int gooey_voice_batch_set_seed(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, uint32_t seed) {
+  GOOEY_TRY
+  if (int rc = voice_of_kind(b, voice, GOOEY_B200_VOICE_GRANULATOR, "set_seed")) return rc;
+  b->pending[voice].push_back(make_event(frame, gd::EV_GRAN_SEED, 0, 0.0f, seed));
   return GOOEY_E_OK;
   GOOEY_CATCH
 }

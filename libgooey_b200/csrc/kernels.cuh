@@ -402,7 +402,7 @@ __global__ void __launch_bounds__(BLOCK) back_kernel(const VoiceLaunch L) {
   }
 }
 
-#ifndef GOOEY_RS_CHAIN_TU   // rs_chain.cu compiles only its own kernels
+#ifndef GOOEY_OWN_KERNELS_TU   // rs_chain.cu and poly_wave.cu compile only their own kernels
 // The LFO pool of a batch (engine/lfo.rs:170-185): one thread per (engine, enabled LFO) walks the call's frames —
 // value = sin(phase * 2 * pi); phase += inc, wrapped at 1; out = offset + value * amount — and leaves the final phase.
 __global__ void __launch_bounds__(64) lfo_kernel(LfoStream* __restrict__ streams, int n, float* __restrict__ planes, long long pitch, int frames) {

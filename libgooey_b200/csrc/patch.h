@@ -45,6 +45,14 @@ template <class AddFn> static bool ffi_param_to_events(uint32_t instrument, uint
       if (param >= 16) return false;
       add(gd::EV_SET_TARGET, param, clamp01(value));   // BASS_PARAM_* ids follow the smoother order (ffi.rs:1904-1934)
       return true;
+    case GOOEY_B200_VOICE_POLY:                          // PolySynth::set_param: ids 0-13 in PolyConfig order (poly_synth.rs)
+      if (param >= gd::P_NP) return false;
+      add(gd::EV_SET_TARGET, param, clamp01(value));
+      return true;
+    case GOOEY_B200_VOICE_GRANULATOR:                    // gooey_engine_granulator_set_param: ids 0-11 in GranulatorConfig order
+      if (param >= gd::G_NP) return false;
+      add(gd::EV_SET_TARGET, param, clamp01(value));
+      return true;
     default: return false;
   }
 }

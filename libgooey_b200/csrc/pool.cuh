@@ -7,7 +7,8 @@
 // TypeRunner<V>: the per-render list of (slot, output row, events) for one type bucket and the
 // A -> (B | C pipelined over time chunks) + S launch sequence of kernels.cuh.  Type bucketing keeps
 // warps type-homogeneous (no cross-instrument divergence).  choose_back() fixes which kernel plays C for the drums;
-// the bass, the granulator and the poly synth have one path each (their warp kernels, or kernel S).
+// the bass, the granulator and the poly synth have one path each (their warp kernels, or kernel S for LFO-routed
+// basses), apart from the serial reference below.
 #pragma once
 #include <algorithm>
 #include <atomic>
@@ -20,6 +21,7 @@
 #include "coop.cuh"
 #include "gran_wave.cuh"
 #include "bass_wave.cuh"
+#include "poly_wave.cuh"
 #include "../../include/gooey_batch.h"
 
 namespace gh {
@@ -146,7 +148,8 @@ ClockTable& clock_table(float sr);
 //   tom, >= COOP_FROM voices                      coop_kernel<TomC, COOP_NV>   (coop.cuh)
 //   kick / snare / hi-hat / tom, fewer voices     wave_kernel<...W>           (wave.cuh)
 //   kick / snare / hi-hat, >= SERIAL_FROM voices  back_kernel<V, 32>          (kernels.cuh)
-// GOOEY_B200_BACKEND=serial puts every drum on back_kernel: the per-sample-order reference of the parity tests.
+// GOOEY_B200_BACKEND=serial puts every drum on back_kernel and every poly synth on slow_kernel<PolyV> (instead of
+// poly_wave_kernel): the per-sample-order references of the parity tests.
 enum class Back { Wave, Coop, Serial };
 // The cooperative back end issues ~3x fewer instructions per voice-frame but walks a block through barrier-separated phases,
 // so a voice's timeline is slower than in the warp-per-voice back end while voices are too few to fill the device with CTAs:
@@ -223,6 +226,7 @@ template <class V> struct TypeRunner {
   std::vector<double> timed_units;       // voice-frames of that launch
   std::vector<cudaEvent_t> evChunk;      // evChunk[i]: frames of chunk i are final in the output (fast-path voices)
   int launched_chunks = 0;               // chunks of the most recent launch (0 = one undivided launch)
+  int timed_launches = 0;                // timed launches of the most recent undivided launch not yet collected (poly synths)
   const char* backend_name = "back_kernel";   // the back-end kernel of the most recent launch (kernel statistics key)
   static int chunk_of(int frames) { return std::min(CHUNK_FRAMES, (frames + 31) & ~31); }
   // Makes `s` wait until every voice of this bucket has written frames [i * chunk, (i + 1) * chunk) of the last launch.
@@ -270,20 +274,22 @@ template <class V> struct TypeRunner {
   // After the launch's streams have been synchronised: add the back-end launches of the last call to the global table.
   void collect_stats() {
     const char* name = backend_name;
-    if (launched_chunks <= 0) return;
+    const int timed = V::FAST ? launched_chunks : timed_launches;
+    if (timed <= 0) return;
     std::lock_guard<std::mutex> lk(kernel_stats_mutex());
     KernelStat& k = kernel_stats()[name];
-    for (int i = 0; i < launched_chunks; i++) {
+    for (int i = 0; i < timed; i++) {
       float ms = 0.0f;
       if (cudaEventElapsedTime(&ms, evT0[i], evT1[i]) != cudaSuccess) { cudaGetLastError(); continue; }
       k.launches++; k.ms += ms; k.voice_frames += timed_units[i];
     }
-    launched_chunks = -launched_chunks;   // collected once
+    if (V::FAST) launched_chunks = -launched_chunks;   // collected once
+    else timed_launches = 0;
   }
   // Forks from `parent` (after `start`), runs the bucket on its own streams, joins back into `parent`.
   void launch(cudaStream_t parent, cudaEvent_t start, const gd::RateCtx& rc, const double* tt, int frames, float* out, long long stride) {
     const int cnt = n();
-    launched_chunks = 0;
+    launched_chunks = 0; timed_launches = 0;
     if (cnt == 0 || frames <= 0) return;
     ensure_streams();
     GH_CUDA(cudaStreamWaitEvent(sC, start, 0));
@@ -396,7 +402,22 @@ template <class V> struct TypeRunner {
           fprintf(stderr, "[gooey trace]   bass_wave_kernel: %d voices x %d frames, %.1f ms\n", cnt, frames, ms);
           cudaEventDestroy(t0); cudaEventDestroy(t1);
         }
-      } else if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);   // LFO-routed basses, poly synths
+      } else if (std::is_same<V, gd::PolyV>::value) {                        // timed: the kernel statistics show which back end ran
+        if (evT0.empty()) { cudaEvent_t e0, e1; GH_CUDA(cudaEventCreate(&e0)); GH_CUDA(cudaEventCreate(&e1)); evT0.push_back(e0); evT1.push_back(e1); timed_units.push_back(0.0); }
+        timed_units[0] = (double)cnt * frames;
+        GH_CUDA(cudaEventRecord(evT0[0], sC));
+        if (serial_backend()) {
+          if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);
+          else GH_LAUNCH((gd::slow_kernel<V, 128>), (cnt + 127) / 128, 128, sC, L);
+          backend_name = "slow_kernel<PolyV>";
+        } else {
+          gd::poly_wave_launch(L, sC);                                          // one warp per poly synth, lane = frame (poly_wave.cu)
+          backend_name = "poly_wave_kernel";
+        }
+        GH_CUDA(cudaGetLastError());
+        GH_CUDA(cudaEventRecord(evT1[0], sC));
+        timed_launches = 1;
+      } else if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);   // LFO-routed basses
       else GH_LAUNCH((gd::slow_kernel<V, 128>), (cnt + 127) / 128, 128, sC, L);
       g_launches.fetch_add(1, std::memory_order_relaxed);
       GH_CUDA(cudaGetLastError());

@@ -1,5 +1,5 @@
 // rs_chain.cu — the kernels of rs_chain.cuh and their launchers.
-#define GOOEY_RS_CHAIN_TU
+#define GOOEY_OWN_KERNELS_TU
 #include "device_rt.h"
 #include "rs_chain.cuh"
 

@@ -8,9 +8,10 @@ import ctypes
 
 import numpy as np
 
-from ._lib import VoicePatch, check, lib
+from ._lib import GooeyError, VoicePatch, check, lib
 
 KICK, SNARE, HIHAT, TOM, BASS = 0, 1, 2, 3, 4
+POLY, GRANULATOR = 5, 6     # libgooey_b200 voice kinds (include/gooey_batch.h GOOEY_B200_VOICE_*)
 
 # Reference presets (normalized), in each Config's `new_full` argument order.
 KICK_PRESETS = {  # src/instruments/kick.rs:257-350
@@ -50,6 +51,13 @@ BASS_PRESETS = {  # BassConfig::{acid,sub,reese,stab} in field order (src/instru
     "sub": [0.18, 1.00, 0.15, 0.00, 0.00, 0.00, 0.70, 0.05, 0.10, 0.30, 0.20, 0.60, 0.15, 0.00, 0.85],
     "reese": [0.18, 0.30, 0.80, 0.80, 0.50, 0.05, 0.35, 0.30, 0.50, 0.40, 0.15, 0.55, 0.12, 0.60, 0.80],
     "stab": [0.30, 0.20, 0.90, 0.00, 0.00, 0.90, 0.20, 0.40, 0.90, 0.08, 0.05, 0.20, 0.08, 0.20, 0.80],
+}
+POLY_PRESETS = {  # PolyConfig::{default,pad,pluck,keys,strings} in field order (src/instruments/poly_synth.rs:49-142)
+    "default": [0.0, 0.2, 0.6, 0.15, 0.3, 0.55, 0.7, 0.7, 0.8, 0.5, 0.65, 0.4, 0.75, 0.7],
+    "pad": [0.0, 0.4, 0.45, 0.2, 0.2, 0.8, 0.75, 0.8, 0.85, 0.75, 0.7, 0.5, 0.8, 0.6],
+    "pluck": [0.3, 0.1, 0.7, 0.25, 0.6, 0.0, 0.75, 0.0, 0.65, 0.0, 0.7, 0.1, 0.65, 0.7],
+    "keys": [0.5, 0.15, 0.55, 0.1, 0.4, 0.35, 0.7, 0.5, 0.75, 0.3, 0.65, 0.3, 0.7, 0.7],
+    "strings": [0.0, 0.5, 0.5, 0.1, 0.15, 0.85, 0.7, 0.9, 0.85, 0.8, 0.7, 0.6, 0.8, 0.5],
 }
 
 
@@ -99,6 +107,29 @@ class VoiceBatch:
 
     def set_param(self, voice, param, value, frame=0, snap=False):
         check(lib().gooey_voice_batch_set_param(self._h, voice, frame, param, ctypes.c_float(value), int(snap)))
+
+    # Poly voices: PolySynth::trigger_note / release_all.  Granulators: Granulator::set_buffer / set_seed, and
+    # share_buffer, which plays another granulator's buffer without a second device copy.  Each raises GooeyError on a
+    # refusal (wrong voice kind, note above 127, invalid buffer), and a refused call queues nothing.
+    def note_on(self, voice, note, velocity=1.0, frame=0):
+        if not 0 <= int(note) <= 127:
+            raise GooeyError(f"note_on: note {note} is outside 0..127")
+        check(lib().gooey_voice_batch_note_on(self._h, voice, frame, int(note), ctypes.c_float(velocity)))
+
+    def release(self, voice, frame=0):
+        check(lib().gooey_voice_batch_release(self._h, voice, frame))
+
+    def set_buffer(self, voice, samples, sample_rate, frame=0):
+        buf = np.ascontiguousarray(samples, dtype=np.float32)
+        if buf.ndim != 1 or buf.size == 0:
+            raise GooeyError("set_buffer: samples must be a non-empty 1-D array")
+        check(lib().gooey_voice_batch_set_buffer(self._h, voice, frame, buf.ctypes.data, buf.size, ctypes.c_float(sample_rate)))
+
+    def share_buffer(self, dst_voice, src_voice, frame=0):
+        check(lib().gooey_voice_batch_share_buffer(self._h, dst_voice, frame, src_voice))
+
+    def set_seed(self, voice, seed, frame=0):
+        check(lib().gooey_voice_batch_set_seed(self._h, voice, frame, int(seed) & 0xFFFFFFFF))
 
     def render(self, frames, out=None):
         if out is None:

@@ -58,6 +58,11 @@ extern "C" {
     pub fn gooey_voice_batch_free(b: *mut GooeyVoiceBatch);
     pub fn gooey_voice_batch_trigger(b: *mut GooeyVoiceBatch, voice: u32, frame: u32, velocity: c_float) -> c_int;
     pub fn gooey_voice_batch_set_param(b: *mut GooeyVoiceBatch, voice: u32, frame: u32, param: u32, value: c_float, snap: c_int) -> c_int;
+    pub fn gooey_voice_batch_note_on(b: *mut GooeyVoiceBatch, voice: u32, frame: u32, note: u32, velocity: c_float) -> c_int;
+    pub fn gooey_voice_batch_release(b: *mut GooeyVoiceBatch, voice: u32, frame: u32) -> c_int;
+    pub fn gooey_voice_batch_set_buffer(b: *mut GooeyVoiceBatch, voice: u32, frame: u32, samples: *const c_float, len: u32, sample_rate: c_float) -> c_int;
+    pub fn gooey_voice_batch_share_buffer(b: *mut GooeyVoiceBatch, dst_voice: u32, frame: u32, src_voice: u32) -> c_int;
+    pub fn gooey_voice_batch_set_seed(b: *mut GooeyVoiceBatch, voice: u32, frame: u32, seed: u32) -> c_int;
     pub fn gooey_voice_batch_render(b: *mut GooeyVoiceBatch, frames: u32, out_host: *mut c_float) -> c_int;
 
     pub fn gooey_b200_write_wav(path: *const c_char, samples: *const c_float, n: u32, sample_rate: u32, bit_depth: u32) -> c_int;
