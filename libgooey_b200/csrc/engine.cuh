@@ -312,18 +312,14 @@ struct EngineBank {
   DevBuf<gd::VoiceEvent> d_mix_eventss[2];
   std::recursive_mutex mu;   // every use of the bank's shared buffers / streams, held for a whole render call
   float last_ms = 0.0f;
-  // timing brackets of the effect mixer of piece p of the last render (on mix_stream) and its engine-frames
-  std::vector<cudaEvent_t> mixT0, mixT1; std::vector<double> mix_units; int mix_timed = 0;
-  void collect_mix_stats() {     // after the streams have been synchronised
+  KernelTimer mix_timer;                  // the effect mixer of each piece of the last render (on mix_stream)
+  void collect_stats() {                  // after the streams have been synchronised
+    mix_timer.collect();
+    voices.collect_stats();
+    if (!h_chain_units) return;
     std::lock_guard<std::mutex> lk(kernel_stats_mutex());
-    KernelStat& k = kernel_stats()["mix_kernel"];
-    for (int i = 0; i < mix_timed; i++) {
-      float ms = 0.0f;
-      if (cudaEventElapsedTime(&ms, mixT0[i], mixT1[i]) != cudaSuccess) { cudaGetLastError(); continue; }
-      k.launches++; k.ms += ms; k.voice_frames += mix_units[i];
-    }
-    mix_timed = 0;
-    if (h_chain_units) { KernelStat& c = kernel_stats()["chain_fast_kernel"]; c.launches++; c.voice_frames += (double)h_chain_units; h_chain_units = 0; }
+    KernelStat& c = kernel_stats()["chain_fast_kernel"];
+    c.launches++; c.voice_frames += (double)h_chain_units; h_chain_units = 0;
   }
   EngineBank(int dev, float sr_) : device(dev), sr(sr_) {
     rc = gd::make_rate_ctx(sr); geo = make_fx_geom(sr);
@@ -912,6 +908,7 @@ inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, 
   GH_CUDA(cudaEventRecord(B.ev_piece, st));
   GH_CUDA(cudaStreamWaitEvent(ms, B.ev_piece, 0));             // the mix stream starts after everything queued so far (uploads, ring set-up)
   GH_CUDA(cudaEventRecord(B.ev0, st));
+  B.mix_timer.clear();
   std::vector<gd::VoiceEvent> cur, mflat;
   std::vector<uint32_t> mbegin;
   std::vector<size_t> vpos((size_t)n * 7, 0), mpos(n, 0);
@@ -1011,14 +1008,12 @@ inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, 
         GH_CUDA(cudaFuncSetAttribute(gd::chain_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gd::CHAIN_SMEM));
       }
     }
-    if (B.mixT0.size() <= pc) { cudaEvent_t a, b; GH_CUDA(cudaEventCreate(&a)); GH_CUDA(cudaEventCreate(&b)); B.mixT0.push_back(a); B.mixT1.push_back(b); B.mix_units.push_back(0.0); }
-    GH_CUDA(cudaEventRecord(B.mixT0[pc], ms));
+    B.mix_timer.begin(ms);
     // settled tilt / delay / spring chains: whole warps of engines go to the pipelined chain kernel, mix_kernel takes the rest
     const bool chain_fast = getenv("GOOEY_B200_NO_CHAIN_FAST") == nullptr;     // (tests compare the two paths bit for bit)
     if (chain_fast && M.premix) { gd::chain_fast_kernel<<<(n + 31) / 32, 32, gd::CHAIN_SMEM, ms>>>(M); g_launches.fetch_add(1, std::memory_order_relaxed); }
     gd::mix_kernel<<<(n + 31) / 32, 32, gd::MIX_DYN_SMEM, ms>>>(M);
-    GH_CUDA(cudaEventRecord(B.mixT1[pc], ms));
-    B.mix_units[pc] = (double)n * nf; B.mix_timed = (int)pc + 1;
+    B.mix_timer.end(ms, "mix_kernel", (double)n * nf);
     g_launches.fetch_add(3, std::memory_order_relaxed);
     GH_CUDA(cudaGetLastError());
     GH_CUDA(cudaEventRecord(B.ev_mixed[vb], ms));

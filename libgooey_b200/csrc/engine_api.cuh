@@ -671,8 +671,7 @@ static int batch_render_impl(GooeyEngine* const* engines, uint32_t n, uint32_t f
       std::lock_guard<std::mutex> g(g_ms_mutex);
       gh::g_last_kernel_ms = accumulate_ms ? std::max(gh::g_last_kernel_ms, ms) : ms;
     }
-    B.collect_mix_stats();
-    B.voices.collect_stats();
+    B.collect_stats();
     return GOOEY_E_OK;
   } catch (const gh::BadBatch& ex) {
     gh::set_error(ex.what());

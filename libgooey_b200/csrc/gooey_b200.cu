@@ -5,7 +5,6 @@
 #include <mutex>
 #include <memory>
 #include "pool.cuh"
-#include "patch.h"
 #include "halfband_design.h"
 #include "rs_chain.cuh"
 #include "poly_wave.cuh"
@@ -72,72 +71,6 @@ static void use_device(int device) {
     g_dev_ready[device] = 1;
   }
 }
-
-// Every voice-type bucket of one device-resident set of voices.
-struct VoiceBank {
-  TypeRunner<gd::KickV> kicks;
-  TypeRunner<gd::SnareV> snares;
-  TypeRunner<gd::HatV> hats;
-  TypeRunner<gd::TomV> toms;
-  TypeRunner<gd::BassV> basses;
-  TypeRunner<gd::PolyV> polys;
-  TypeRunner<gd::GranV> grans;
-  void reset() { kicks.reset(); snares.reset(); hats.reset(); toms.reset(); basses.reset(); polys.reset(); grans.reset(); }
-  // returns the pool slot of a new voice built from `p` (the reference's `<Voice>::with_config`); -1 = bad instrument
-  int create(const GooeyVoicePatch& p, float sr) {
-    switch (p.instrument) {
-      case GOOEY_INSTRUMENT_KICK: { gd::KickState s; init_from_patch(s, p, sr); return kicks.pool.alloc(s); }
-      case GOOEY_INSTRUMENT_SNARE: { gd::SnareState s; init_from_patch(s, p, sr); return snares.pool.alloc(s); }
-      case GOOEY_INSTRUMENT_HIHAT: { gd::HatState s; init_from_patch(s, p, sr); return hats.pool.alloc(s); }
-      case GOOEY_INSTRUMENT_TOM: { gd::TomState s; init_from_patch(s, p, sr); return toms.pool.alloc(s); }
-      case GOOEY_INSTRUMENT_BASS: { gd::BassState s; init_from_patch(s, p, sr); return basses.pool.alloc(s); }
-      case GOOEY_B200_VOICE_POLY: { gd::PolyState s; memset(&s, 0, sizeof s); gd::poly_init(s, p.params, sr); return polys.pool.alloc(s); }   // params = PolyConfig (14 values)
-      case GOOEY_B200_VOICE_GRANULATOR: { gd::GranState s; memset(&s, 0, sizeof s); gd::gran_init(s, sr); return grans.pool.alloc(s); }
-      default: return -1;
-    }
-  }
-  void set_mod(const float* planes, long long pitch, int frame0) {
-    kicks.mod_planes = snares.mod_planes = hats.mod_planes = toms.mod_planes = basses.mod_planes = planes;
-    kicks.mod_pitch = snares.mod_pitch = hats.mod_pitch = toms.mod_pitch = basses.mod_pitch = pitch;
-    kicks.mod_frame0 = snares.mod_frame0 = hats.mod_frame0 = toms.mod_frame0 = basses.mod_frame0 = frame0;
-  }
-  void add(uint32_t type, uint32_t slot, uint32_t row, const std::vector<gd::VoiceEvent>& ev, const std::vector<gd::ModRoute>* routes = nullptr) {
-    switch (type) {
-      case GOOEY_INSTRUMENT_KICK: kicks.add(slot, row, ev, routes); break;
-      case GOOEY_INSTRUMENT_SNARE: snares.add(slot, row, ev, routes); break;
-      case GOOEY_INSTRUMENT_HIHAT: hats.add(slot, row, ev, routes); break;
-      case GOOEY_INSTRUMENT_TOM: toms.add(slot, row, ev, routes); break;
-      case GOOEY_INSTRUMENT_BASS: basses.add(slot, row, ev, routes); break;
-      case GOOEY_B200_VOICE_POLY: polys.add(slot, row, ev); break;
-      case GOOEY_B200_VOICE_GRANULATOR: grans.add(slot, row, ev); break;
-    }
-  }
-  void release(uint32_t type, int slot) {
-    switch (type) {
-      case GOOEY_INSTRUMENT_KICK: kicks.pool.release(slot); break;
-      case GOOEY_INSTRUMENT_SNARE: snares.pool.release(slot); break;
-      case GOOEY_INSTRUMENT_HIHAT: hats.pool.release(slot); break;
-      case GOOEY_INSTRUMENT_TOM: toms.pool.release(slot); break;
-      case GOOEY_INSTRUMENT_BASS: basses.pool.release(slot); break;
-      case GOOEY_B200_VOICE_POLY: polys.pool.release(slot); break;
-      case GOOEY_B200_VOICE_GRANULATOR: grans.pool.release(slot); break;
-    }
-  }
-  void launch(cudaStream_t parent, cudaEvent_t start, const gd::RateCtx& rc, const double* tt, int frames, float* out, long long stride) {
-    kicks.launch(parent, start, rc, tt, frames, out, stride);
-    snares.launch(parent, start, rc, tt, frames, out, stride);
-    hats.launch(parent, start, rc, tt, frames, out, stride);
-    toms.launch(parent, start, rc, tt, frames, out, stride);
-    basses.launch(parent, start, rc, tt, frames, out, stride);
-    polys.launch(parent, start, rc, tt, frames, out, stride);
-    grans.launch(parent, start, rc, tt, frames, out, stride);
-  }
-  // call after the launching stream has been synchronised
-  void collect_stats() { kicks.collect_stats(); snares.collect_stats(); hats.collect_stats(); toms.collect_stats(); polys.collect_stats(); }
-  // frames per output chunk of the last launch (identical for every bucket) and the per-chunk completion fence
-  int chunk_frames(int frames) const { return TypeRunner<gd::KickV>::chunk_of(frames); }
-  void wait_chunk(cudaStream_t s, int i) { kicks.wait_chunk(s, i); snares.wait_chunk(s, i); hats.wait_chunk(s, i); toms.wait_chunk(s, i); basses.wait_chunk(s, i); polys.wait_chunk(s, i); grans.wait_chunk(s, i); }
-};
 
 }  // namespace gh
 

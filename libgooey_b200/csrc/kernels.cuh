@@ -17,6 +17,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include "voices2.cuh"
+#include "../../include/gooey_batch.h"
 
 namespace gd {
 
@@ -36,9 +37,10 @@ template <class S> __device__ __forceinline__ void store_words(const S& s, uint3
 }
 
 // ------------------------------------------------------------------------------------------- voice traits ----
+// ID: the instrument id (GooeyVoicePatch::instrument) that selects the type.
 struct KickV {
   using State = KickState; using Ctl = KickCtl; using Aud = KickAud; using Span = KickSpan;
-  static constexpr bool FAST = true; static constexpr int NPL = KICK_PLANES;
+  static constexpr bool FAST = true; static constexpr int NPL = KICK_PLANES; static constexpr uint32_t ID = GOOEY_INSTRUMENT_KICK;
   struct Run { KickDer d; int j_act; };
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return kick_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) {
@@ -66,7 +68,7 @@ struct KickV {
 };
 struct SnareV {
   using State = SnareState; using Ctl = SnareCtl; using Aud = SnareAud; using Span = SnareSpan;
-  static constexpr bool FAST = true; static constexpr int NPL = SNARE_PLANES;
+  static constexpr bool FAST = true; static constexpr int NPL = SNARE_PLANES; static constexpr uint32_t ID = GOOEY_INSTRUMENT_SNARE;
   struct Run { SnareDer d; int j_act; };
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return snare_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) {
@@ -92,7 +94,7 @@ struct SnareV {
 };
 struct HatV {
   using State = HatState; using Ctl = HatCtl; using Aud = HatAud; using Span = HatSpan;
-  static constexpr bool FAST = true; static constexpr int NPL = HAT_PLANES;
+  static constexpr bool FAST = true; static constexpr int NPL = HAT_PLANES; static constexpr uint32_t ID = GOOEY_INSTRUMENT_HIHAT;
   struct Run { HatDer d; int j_env; float env_final; };
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return hat_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) {
@@ -115,7 +117,7 @@ struct HatV {
 };
 struct TomV {
   using State = TomState; using Ctl = TomCtl; using Aud = TomAud; using Span = TomSpan;
-  static constexpr bool FAST = true; static constexpr int NPL = TOM_PLANES;
+  static constexpr bool FAST = true; static constexpr int NPL = TOM_PLANES; static constexpr uint32_t ID = GOOEY_INSTRUMENT_TOM;
   struct Run { TomDer d; int j_env; float env_final; };
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return tom_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx& rc) {
@@ -141,13 +143,13 @@ struct TomV {
     return tom_back(a, r.d, f, j >= r.j_env, rc);
   }
 };
-struct BassV { using State = BassState; static constexpr bool FAST = false;
+struct BassV { using State = BassState; static constexpr bool FAST = false; static constexpr uint32_t ID = GOOEY_INSTRUMENT_BASS;
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return bass_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) { bass_event(s, e, tt); } };
-struct PolyV { using State = PolyState; static constexpr bool FAST = false;
+struct PolyV { using State = PolyState; static constexpr bool FAST = false; static constexpr uint32_t ID = GOOEY_B200_VOICE_POLY;
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return poly_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) { poly_event(s, e, tt); } };
-struct GranV { using State = GranState; static constexpr bool FAST = false;
+struct GranV { using State = GranState; static constexpr bool FAST = false; static constexpr uint32_t ID = GOOEY_B200_VOICE_GRANULATOR;
   static __device__ __forceinline__ float tick(State& s, const double* tt, const RateCtx& rc) { return gran_tick(s, tt, rc); }
   static __device__ __forceinline__ void slow_event(State& s, const VoiceEvent& e, const double* tt, const RateCtx&) { gran_event(s, e, tt); } };
 

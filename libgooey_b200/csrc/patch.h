@@ -98,5 +98,13 @@ inline void init_from_patch(gd::BassState& s, const GooeyVoicePatch& p, float sr
   gd::bass_init(s, p.params, sr);
   if (p.aux & 0x100) s.cur[gd::B_TUNING] = s.tgt[gd::B_TUNING] = clamp01(p.params[23]);
 }
+inline void init_from_patch(gd::PolyState& s, const GooeyVoicePatch& p, float sr) {   // params = PolyConfig (14 values)
+  memset(&s, 0, sizeof s);
+  gd::poly_init(s, p.params, sr);
+}
+inline void init_from_patch(gd::GranState& s, const GooeyVoicePatch&, float sr) {
+  memset(&s, 0, sizeof s);
+  gd::gran_init(s, sr);
+}
 
 }  // namespace gh

@@ -16,13 +16,14 @@
 #include <type_traits>
 #include <set>
 #include <mutex>
+#include <tuple>
 #include "device_rt.h"
 #include "wave.cuh"
 #include "coop.cuh"
 #include "gran_wave.cuh"
 #include "bass_wave.cuh"
 #include "poly_wave.cuh"
-#include "../../include/gooey_batch.h"
+#include "patch.h"
 
 namespace gh {
 
@@ -32,6 +33,45 @@ extern std::atomic<uint64_t> g_launches;
 struct KernelStat { uint64_t launches = 0; double ms = 0.0; double voice_frames = 0.0; };
 std::map<std::string, KernelStat>& kernel_stats();
 std::mutex& kernel_stats_mutex();
+// Times launches for kernel_stats(): begin() and end() bracket one launch on its stream with reusable events.  collect()
+// runs once the caller has synchronised those streams; it adds the bracketed launches to the table and forgets them.
+// clear() forgets them uncounted.
+struct KernelTimer {
+  struct Rec { cudaEvent_t t0, t1; const char* key; double units; };
+  std::vector<Rec> recs;
+  size_t n = 0;                          // records bracketed since the last collect() / clear()
+  KernelTimer() = default;
+  KernelTimer(const KernelTimer&) = delete;
+  ~KernelTimer() { for (const Rec& r : recs) { cudaEventDestroy(r.t0); cudaEventDestroy(r.t1); } }
+  void begin(cudaStream_t s) {
+    if (n == recs.size()) { Rec r{}; GH_CUDA(cudaEventCreate(&r.t0)); GH_CUDA(cudaEventCreate(&r.t1)); recs.push_back(r); }
+    GH_CUDA(cudaEventRecord(recs[n].t0, s));
+  }
+  void end(cudaStream_t s, const char* key, double units) {   // units: voice-frames (or engine-frames) of the launch
+    Rec& r = recs[n++];
+    r.key = key; r.units = units;
+    GH_CUDA(cudaEventRecord(r.t1, s));
+  }
+  void clear() { n = 0; }
+  // after a synchronise: the device time of record i, or -1 when it cannot be read (the error is cleared)
+  float elapsed(size_t i) const {
+    float ms = 0.0f;
+    if (cudaEventElapsedTime(&ms, recs[i].t0, recs[i].t1) == cudaSuccess) return ms;
+    cudaGetLastError();
+    return -1.0f;
+  }
+  float ms() const { float sum = 0.0f; for (size_t i = 0; i < n; i++) sum += std::max(elapsed(i), 0.0f); return sum; }
+  void collect() {
+    std::lock_guard<std::mutex> lk(kernel_stats_mutex());
+    for (size_t i = 0; i < n; i++) {
+      const float ms = elapsed(i);
+      if (ms < 0.0f) continue;
+      KernelStat& k = kernel_stats()[recs[i].key];
+      k.launches++; k.ms += ms; k.voice_frames += recs[i].units;
+    }
+    n = 0;
+  }
+};
 
 __global__ void scatter_words_kernel(uint32_t* __restrict__ dst, long long cap, const uint32_t* __restrict__ src, const uint32_t* __restrict__ slots,
                                      int n, int words) {
@@ -143,13 +183,15 @@ struct ClockWindow {
 };
 ClockTable& clock_table(float sr);
 
-// ---- the drum back ends (kernel C of the A -> (B | C) + S sequence) ----
-// Which kernel renders a drum bucket depends on the voice type and on how many voices of the type one launch holds:
+// ---- the back ends (kernel C of the A -> (B | C) + S sequence) ----
+// launch_back<V>() launches the back end of a bucket and returns its kernel-statistics key.  Which kernel renders a drum
+// bucket depends on the voice type and on how many voices of the type one launch holds (choose_back):
 //   tom, >= COOP_FROM voices                      coop_kernel<TomC, COOP_NV>   (coop.cuh)
 //   kick / snare / hi-hat / tom, fewer voices     wave_kernel<...W>           (wave.cuh)
 //   kick / snare / hi-hat, >= SERIAL_FROM voices  back_kernel<V, 32>          (kernels.cuh)
-// GOOEY_B200_BACKEND=serial puts every drum on back_kernel and every poly synth on slow_kernel<PolyV> (instead of
-// poly_wave_kernel): the per-sample-order references of the parity tests.
+// The other types have one back end each: bass_wave_kernel (slow_kernel<BassV> for LFO-routed basses), poly_wave_kernel
+// and gran_wave_kernel.  GOOEY_B200_BACKEND=serial puts every drum on back_kernel and every poly synth on
+// slow_kernel<PolyV> (instead of poly_wave_kernel): the per-sample-order references of the parity tests.
 enum class Back { Wave, Coop, Serial };
 // The cooperative back end issues ~3x fewer instructions per voice-frame but walks a block through barrier-separated phases,
 // so a voice's timeline is slower than in the warp-per-voice back end while voices are too few to fill the device with CTAs:
@@ -205,6 +247,37 @@ template <class K> inline void same_carveout(K kernel) {
 }
 #define GH_LAUNCH(kernel, grid, block, stream, ...) do { same_carveout(kernel); kernel<<<grid, block, 0, stream>>>(__VA_ARGS__); } while (0)
 
+// The per-sample kernel S as a bucket's back end: one-warp CTAs up to 148 * 32 * 4 voices, 128-thread CTAs above.
+template <class V> inline void slow_launch(const gd::VoiceLaunch& L, cudaStream_t s) {
+  if (L.n <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (L.n + 31) / 32, 32, s, L);
+  else GH_LAUNCH((gd::slow_kernel<V, 128>), (L.n + 127) / 128, 128, s, L);
+}
+// The drums; the other types specialise it below.
+template <class V> inline const char* launch_back(const gd::VoiceLaunch& L, cudaStream_t s) {
+  const Back back = choose_back<V>(L.n);
+  if (back == Back::Coop) { coop_launch(L.n, s, L); return "coop_kernel<TomC>"; }
+  if (back == Back::Wave) {
+    GH_LAUNCH((gd::wave::wave_kernel<typename WaveOf<V>::W>), L.n, 32, s, L);   // one voice per one-warp CTA
+    return WaveOf<V>::name;
+  }
+  GH_LAUNCH((gd::back_kernel<V, 32>), (L.n + 31) / 32, 32, s, L);             // one voice per lane, one warp per CTA
+  return "back_kernel";
+}
+template <> inline const char* launch_back<gd::BassV>(const gd::VoiceLaunch& L, cudaStream_t s) {
+  if (L.routes) { slow_launch<gd::BassV>(L, s); return "slow_kernel<BassV>"; }   // LFO-routed basses
+  GH_LAUNCH((gd::bass_wave_kernel<2>), (L.n + 1) / 2, 64, s, L);                 // one warp per bass voice, lane = frame (bass_wave.cuh)
+  return "bass_wave_kernel";
+}
+template <> inline const char* launch_back<gd::PolyV>(const gd::VoiceLaunch& L, cudaStream_t s) {
+  if (serial_backend()) { slow_launch<gd::PolyV>(L, s); return "slow_kernel<PolyV>"; }
+  gd::poly_wave_launch(L, s);                                                      // one warp per poly synth, lane = frame (poly_wave.cu)
+  return "poly_wave_kernel";
+}
+template <> inline const char* launch_back<gd::GranV>(const gd::VoiceLaunch& L, cudaStream_t s) {
+  GH_LAUNCH((gd::gran_wave_kernel<4>), (L.n + 3) / 4, 128, s, L);                 // one warp per granulator, grains on lanes (gran_wave.cuh)
+  return "gran_wave_kernel";
+}
+
 // Frames per front/back pipeline stage.
 constexpr int CHUNK_FRAMES = 8192;
 // One type bucket of one render call.
@@ -222,22 +295,21 @@ template <class V> struct TypeRunner {
   DevBuf<float> d_planes[2];
   cudaStream_t sB = nullptr, sC = nullptr, sS = nullptr;
   cudaEvent_t evA = nullptr, evB[2] = {nullptr, nullptr}, evC[2] = {nullptr, nullptr}, evDoneC = nullptr, evDoneS = nullptr;
-  std::vector<cudaEvent_t> evT0, evT1;   // timing brackets of the back-end launch of chunk i (on sC)
-  std::vector<double> timed_units;       // voice-frames of that launch
+  KernelTimer timer;                     // the back-end launches of the most recent launch (on sC)
   std::vector<cudaEvent_t> evChunk;      // evChunk[i]: frames of chunk i are final in the output (fast-path voices)
   int launched_chunks = 0;               // chunks of the most recent launch (0 = one undivided launch)
-  int timed_launches = 0;                // timed launches of the most recent undivided launch not yet collected (poly synths)
-  const char* backend_name = "back_kernel";   // the back-end kernel of the most recent launch (kernel statistics key)
   static int chunk_of(int frames) { return std::min(CHUNK_FRAMES, (frames + 31) & ~31); }
   // Makes `s` wait until every voice of this bucket has written frames [i * chunk, (i + 1) * chunk) of the last launch.
   void wait_chunk(cudaStream_t s, int i) {
     if (n() == 0) return;
     if (launched_chunks == 0) { GH_CUDA(cudaStreamWaitEvent(s, evDoneC, 0)); return; }
     GH_CUDA(cudaStreamWaitEvent(s, evDoneS, 0));
-    GH_CUDA(cudaStreamWaitEvent(s, evChunk[std::min(i, std::abs(launched_chunks) - 1)], 0));
+    GH_CUDA(cudaStreamWaitEvent(s, evChunk[std::min(i, launched_chunks - 1)], 0));
   }
 
   int n() const { return (int)slots.size(); }
+  // a new voice built from `p` (the reference's `<Voice>::with_config`): its pool slot
+  int create(const GooeyVoicePatch& p, float sr) { State s; init_from_patch(s, p, sr); return pool.alloc(s); }
   void reset() { slots.clear(); rows.clear(); ev_flat.clear(); ev_begin.clear(); ev_begin.push_back(0); span_off.clear(); span_off.push_back(0);
                  routes_flat.clear(); route_begin.clear(); route_begin.push_back(0); }
   // events must be ordered by frame and lie inside the call
@@ -265,31 +337,17 @@ template <class V> struct TypeRunner {
     cudaEvent_t evs[] = {evA, evB[0], evB[1], evC[0], evC[1], evDoneC, evDoneS};
     for (auto e : evs) if (e) cudaEventDestroy(e);
     for (auto e : evChunk) cudaEventDestroy(e);
-    for (auto e : evT0) cudaEventDestroy(e);
-    for (auto e : evT1) cudaEventDestroy(e);
     if (sB) cudaStreamDestroy(sB);
     if (sC) cudaStreamDestroy(sC);
     if (sS) cudaStreamDestroy(sS);
   }
   // After the launch's streams have been synchronised: add the back-end launches of the last call to the global table.
-  void collect_stats() {
-    const char* name = backend_name;
-    const int timed = V::FAST ? launched_chunks : timed_launches;
-    if (timed <= 0) return;
-    std::lock_guard<std::mutex> lk(kernel_stats_mutex());
-    KernelStat& k = kernel_stats()[name];
-    for (int i = 0; i < timed; i++) {
-      float ms = 0.0f;
-      if (cudaEventElapsedTime(&ms, evT0[i], evT1[i]) != cudaSuccess) { cudaGetLastError(); continue; }
-      k.launches++; k.ms += ms; k.voice_frames += timed_units[i];
-    }
-    if (V::FAST) launched_chunks = -launched_chunks;   // collected once
-    else timed_launches = 0;
-  }
+  void collect_stats() { timer.collect(); }
   // Forks from `parent` (after `start`), runs the bucket on its own streams, joins back into `parent`.
   void launch(cudaStream_t parent, cudaEvent_t start, const gd::RateCtx& rc, const double* tt, int frames, float* out, long long stride) {
     const int cnt = n();
-    launched_chunks = 0; timed_launches = 0;
+    launched_chunks = 0;
+    timer.clear();
     if (cnt == 0 || frames <= 0) return;
     ensure_streams();
     GH_CUDA(cudaStreamWaitEvent(sC, start, 0));
@@ -304,12 +362,12 @@ template <class V> struct TypeRunner {
     L.state = pool.d.p; L.n = cnt; L.n_pad = pool.cap;
     L.slots = d_slots.p; L.rows = d_rows.p; L.row0 = 0;
     L.events = d_events.p; L.ev_begin = d_ev_begin.p; L.tt = tt; L.frames = frames; L.out = out; L.stride = stride; L.rc = rc;
-    const bool modulated = !routes_flat.empty() && mod_planes;
-    if (modulated) {
+    if (!routes_flat.empty() && mod_planes) {
       d_routes.upload(routes_flat.data(), routes_flat.size(), sC);
       d_route_begin.upload(route_begin.data(), route_begin.size(), sC);
       L.routes = d_routes.p; L.route_begin = d_route_begin.p; L.mod_planes = mod_planes; L.mod_pitch = mod_pitch; L.mod_frame0 = mod_frame0;
     }
+    const char* key = nullptr;
     if constexpr (V::FAST) {
       using Span = typename V::Span;
       d_span_off.upload(span_off.data(), span_off.size(), sC);
@@ -332,7 +390,6 @@ template <class V> struct TypeRunner {
       g_launches.fetch_add(1, std::memory_order_relaxed);
       GH_CUDA(cudaGetLastError());
       GH_CUDA(cudaEventRecord(evDoneS, sS));
-      const Back back = choose_back<V>(cnt);
       int i = 0;
       for (int c0 = 0; c0 < frames; c0 += chunk, i++) {
         const int b = i & 1;
@@ -344,87 +401,71 @@ template <class V> struct TypeRunner {
         GH_CUDA(cudaGetLastError());
         GH_CUDA(cudaEventRecord(evB[b], sB));
         GH_CUDA(cudaStreamWaitEvent(sC, evB[b], 0));
-        if ((int)evT0.size() <= i) { cudaEvent_t e0, e1; GH_CUDA(cudaEventCreate(&e0)); GH_CUDA(cudaEventCreate(&e1)); evT0.push_back(e0); evT1.push_back(e1); timed_units.push_back(0.0); }
-        timed_units[i] = (double)cnt * L.chunk_frames;
-        GH_CUDA(cudaEventRecord(evT0[i], sC));
-        switch (back) {
-          case Back::Coop:
-            if constexpr (std::is_same<V, gd::TomV>::value) coop_launch(cnt, sC, L);
-            backend_name = "coop_kernel<TomC>";
-            break;
-          case Back::Wave:
-            GH_LAUNCH((gd::wave::wave_kernel<typename WaveOf<V>::W>), cnt, 32, sC, L);   // one voice per one-warp CTA
-            backend_name = WaveOf<V>::name;
-            break;
-          case Back::Serial:
-            GH_LAUNCH((gd::back_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);             // one voice per lane, one warp per CTA
-            backend_name = "back_kernel";
-            break;
-        }
+        timer.begin(sC);
+        key = launch_back<V>(L, sC);
         GH_CUDA(cudaGetLastError());
-        GH_CUDA(cudaEventRecord(evT1[i], sC));
+        timer.end(sC, key, (double)cnt * L.chunk_frames);
         GH_CUDA(cudaEventRecord(evC[b], sC));
         if ((int)evChunk.size() <= i) { cudaEvent_t e; GH_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming)); evChunk.push_back(e); }
         GH_CUDA(cudaEventRecord(evChunk[i], sC));
         g_launches.fetch_add(2, std::memory_order_relaxed);
       }
       launched_chunks = i;
-      GH_CUDA(cudaEventRecord(evDoneC, sC));
-      GH_CUDA(cudaStreamWaitEvent(parent, evDoneC, 0));
-      GH_CUDA(cudaStreamWaitEvent(parent, evDoneS, 0));
-      if (getenv("GOOEY_B200_TRACE_TYPES")) {      // diagnostic (serialises the buckets): time of the time-parallel chain and of the per-sample kernel, voices on the latter
-        cudaEvent_t t0, t1, t2;
-        cudaEventCreate(&t0); cudaEventCreate(&t1); cudaEventCreate(&t2);
-        cudaEventRecord(t1, sC); cudaEventRecord(t2, sS);
-        GH_CUDA(cudaStreamSynchronize(sC)); GH_CUDA(cudaStreamSynchronize(sS));
+    } else {
+      timer.begin(sC);
+      key = launch_back<V>(L, sC);
+      GH_CUDA(cudaGetLastError());
+      timer.end(sC, key, (double)cnt * frames);
+      g_launches.fetch_add(1, std::memory_order_relaxed);
+    }
+    GH_CUDA(cudaEventRecord(evDoneC, sC));
+    GH_CUDA(cudaStreamWaitEvent(parent, evDoneC, 0));
+    if (V::FAST) GH_CUDA(cudaStreamWaitEvent(parent, evDoneS, 0));
+    if (getenv("GOOEY_B200_TRACE_TYPES")) {      // diagnostic (serialises the buckets): the back end's device time, drum voices on the per-sample kernel
+      GH_CUDA(cudaStreamSynchronize(sC)); GH_CUDA(cudaStreamSynchronize(sS));
+      std::string per_sample;
+      if constexpr (V::FAST) {
         std::vector<uint8_t> mode(cnt);
         GH_CUDA(cudaMemcpy(mode.data(), d_mode.p, cnt, cudaMemcpyDeviceToHost));
-        int slow = 0; for (uint8_t m : mode) slow += m != 0;
-        float ms_all = 0.0f;
-        cudaEventElapsedTime(&ms_all, evT0[0], t1);
-        float ms_slow_end = 0.0f;
-        cudaEventElapsedTime(&ms_slow_end, evT0[0], t2);
-        fprintf(stderr, "[gooey trace]   %s: %d voices x %d frames, %d on the per-sample path; back ends done %.1f ms, per-sample kernel done %.1f ms after the first back-end launch\n",
-                backend_name, cnt, frames, slow, ms_all, ms_slow_end);
-        cudaEventDestroy(t0); cudaEventDestroy(t1); cudaEventDestroy(t2);
+        int slow = 0;
+        for (uint8_t m : mode) slow += m != 0;
+        per_sample = ", " + std::to_string(slow) + " on the per-sample path";
       }
-    } else {
-      if constexpr (std::is_same<V, gd::GranV>::value) {
-        GH_LAUNCH((gd::gran_wave_kernel<4>), (cnt + 3) / 4, 128, sC, L);       // one warp per granulator, grains on lanes (gran_wave.cuh)
-      } else if (std::is_same<V, gd::BassV>::value && !modulated) {           // one warp per bass voice, lane = frame (bass_wave.cuh)
-        const bool ttrace = getenv("GOOEY_B200_TRACE_TYPES") != nullptr;
-        cudaEvent_t t0 = nullptr, t1 = nullptr;
-        if (ttrace) { cudaEventCreate(&t0); cudaEventCreate(&t1); cudaEventRecord(t0, sC); }
-        GH_LAUNCH((gd::bass_wave_kernel<2>), (cnt + 1) / 2, 64, sC, L);
-        if (ttrace) {
-          cudaEventRecord(t1, sC); GH_CUDA(cudaStreamSynchronize(sC));
-          float ms = 0.0f; cudaEventElapsedTime(&ms, t0, t1);
-          fprintf(stderr, "[gooey trace]   bass_wave_kernel: %d voices x %d frames, %.1f ms\n", cnt, frames, ms);
-          cudaEventDestroy(t0); cudaEventDestroy(t1);
-        }
-      } else if (std::is_same<V, gd::PolyV>::value) {                        // timed: the kernel statistics show which back end ran
-        if (evT0.empty()) { cudaEvent_t e0, e1; GH_CUDA(cudaEventCreate(&e0)); GH_CUDA(cudaEventCreate(&e1)); evT0.push_back(e0); evT1.push_back(e1); timed_units.push_back(0.0); }
-        timed_units[0] = (double)cnt * frames;
-        GH_CUDA(cudaEventRecord(evT0[0], sC));
-        if (serial_backend()) {
-          if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);
-          else GH_LAUNCH((gd::slow_kernel<V, 128>), (cnt + 127) / 128, 128, sC, L);
-          backend_name = "slow_kernel<PolyV>";
-        } else {
-          gd::poly_wave_launch(L, sC);                                          // one warp per poly synth, lane = frame (poly_wave.cu)
-          backend_name = "poly_wave_kernel";
-        }
-        GH_CUDA(cudaGetLastError());
-        GH_CUDA(cudaEventRecord(evT1[0], sC));
-        timed_launches = 1;
-      } else if (cnt <= 148 * 32 * 4) GH_LAUNCH((gd::slow_kernel<V, 32>), (cnt + 31) / 32, 32, sC, L);   // LFO-routed basses
-      else GH_LAUNCH((gd::slow_kernel<V, 128>), (cnt + 127) / 128, 128, sC, L);
-      g_launches.fetch_add(1, std::memory_order_relaxed);
-      GH_CUDA(cudaGetLastError());
-      GH_CUDA(cudaEventRecord(evDoneC, sC));
-      GH_CUDA(cudaStreamWaitEvent(parent, evDoneC, 0));
+      fprintf(stderr, "[gooey trace]   %s: %d voices x %d frames, back end %.1f ms%s\n", key, cnt, frames, timer.ms(), per_sample.c_str());
     }
   }
 };
+
+// Every voice-type bucket of one device-resident set of voices: one TypeRunner per type of Vs, addressed by the
+// instrument id of its voices (V::ID).
+template <class... Vs> struct VoiceBankOf {
+  std::tuple<TypeRunner<Vs>...> runners;
+  template <class F> void each(F f) { (f(std::get<TypeRunner<Vs>>(runners)), ...); }
+  // f(the runner of instrument `id`); nothing when no type has that id
+  template <class F> void with(uint32_t id, F f) { (void)((id == Vs::ID && (f(std::get<TypeRunner<Vs>>(runners)), true)) || ...); }
+  void reset() { each([](auto& r) { r.reset(); }); }
+  // returns the pool slot of a new voice built from `p`; -1 = bad instrument
+  int create(const GooeyVoicePatch& p, float sr) {
+    int slot = -1;
+    with(p.instrument, [&](auto& r) { slot = r.create(p, sr); });
+    return slot;
+  }
+  void set_mod(const float* planes, long long pitch, int frame0) {
+    each([&](auto& r) { r.mod_planes = planes; r.mod_pitch = pitch; r.mod_frame0 = frame0; });
+  }
+  void add(uint32_t type, uint32_t slot, uint32_t row, const std::vector<gd::VoiceEvent>& ev, const std::vector<gd::ModRoute>* routes = nullptr) {
+    with(type, [&](auto& r) { r.add(slot, row, ev, routes); });
+  }
+  void release(uint32_t type, int slot) { with(type, [&](auto& r) { r.pool.release(slot); }); }
+  void launch(cudaStream_t parent, cudaEvent_t start, const gd::RateCtx& rc, const double* tt, int frames, float* out, long long stride) {
+    each([&](auto& r) { r.launch(parent, start, rc, tt, frames, out, stride); });
+  }
+  // call after the launching stream has been synchronised
+  void collect_stats() { each([](auto& r) { r.collect_stats(); }); }
+  // frames per output chunk of the last launch (identical for every bucket) and the per-chunk completion fence
+  int chunk_frames(int frames) const { return TypeRunner<gd::KickV>::chunk_of(frames); }
+  void wait_chunk(cudaStream_t s, int i) { each([&](auto& r) { r.wait_chunk(s, i); }); }
+};
+using VoiceBank = VoiceBankOf<gd::KickV, gd::SnareV, gd::HatV, gd::TomV, gd::BassV, gd::PolyV, gd::GranV>;
 
 }  // namespace gh

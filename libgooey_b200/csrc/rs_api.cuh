@@ -85,8 +85,7 @@ struct GooeyRsBatch {
   gh::DevBuf<float> ring[gd::RS_MAX_FX]; uint32_t ring_words[gd::RS_MAX_FX] = {0}; long long ring_pitch = 0;
   gh::DevBuf<uint32_t> d_chain_rows, d_chain_nfx, d_fx_where, d_ring_clear;
   gh::DevBuf<uint8_t> d_chain_kinds;
-  cudaEvent_t ev_c0 = nullptr, ev_c1 = nullptr;
-  double chain_units = 0.0;                                       // engine-frames of the last bounce's rs_chain_kernel (0: not launched)
+  gh::KernelTimer chain_timer;                                    // the last bounce's rs_chain_kernel
   // arena `k` grows to `words` words per engine, keeping what it holds
   void ensure_ring(int k, uint32_t words) {
     if (words <= ring_words[k]) return;
@@ -101,8 +100,6 @@ struct GooeyRsBatch {
   ~GooeyRsBatch() {
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
-    if (ev_c0) cudaEventDestroy(ev_c0);
-    if (ev_c1) cudaEventDestroy(ev_c1);
     if (stream) cudaStreamDestroy(stream);
   }
 };
@@ -121,8 +118,6 @@ static uint32_t chain_prepare(GooeyRsBatch* b, const std::map<std::vector<uint8_
     if ((b->ring_pitch / 32) % 2 == 0) b->ring_pitch += 32;        // odd multiple of 32 (DESIGN §3)
     b->d_fx_state.alloc((size_t)ne * gd::RS_MAX_FX);
     b->geo = make_fx_geom(b->sr);
-    GH_CUDA(cudaEventCreate(&b->ev_c0));
-    GH_CUDA(cudaEventCreate(&b->ev_c1));
   }
   std::vector<uint32_t> rows, nfx, where;
   std::vector<uint8_t> kinds;
@@ -235,7 +230,7 @@ static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, siz
   gd::rs_mix_kernel<<<grid, 256, 0, st>>>(M);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   GH_CUDA(cudaGetLastError());
-  b->chain_units = 0.0;
+  b->chain_timer.clear();
   if (n_chain_warps) {
     gd::RsChainLaunch C;
     C.out = out_dev; C.out_stride = (long long)out_stride; C.frames = (int)frames;
@@ -243,26 +238,15 @@ static void rs_bounce_impl(GooeyRsBatch* b, uint32_t frames, float* out_dev, siz
     C.state = b->d_fx_state.p;
     for (int k = 0; k < gd::RS_MAX_FX; k++) C.ring[k] = b->ring[k].p;
     C.ring_pitch = b->ring_pitch; C.rc = b->rc; C.geo = b->geo;
-    GH_CUDA(cudaEventRecord(b->ev_c0, st));
+    size_t n = 0;
+    for (const auto& c : chains) n += c.second.size();
+    b->chain_timer.begin(st);
     gd::rs_chain_launch(C, n_chain_warps, st);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     GH_CUDA(cudaGetLastError());
-    GH_CUDA(cudaEventRecord(b->ev_c1, st));
-    size_t n = 0;
-    for (const auto& c : chains) n += c.second.size();
-    b->chain_units = (double)n * frames;
+    b->chain_timer.end(st, "rs_chain_kernel", (double)n * frames);
   }
   GH_CUDA(cudaEventRecord(b->ev1, st));
-}
-// after the stream has been synchronised: the chain kernel's time and engine-frames into the kernel statistics
-static void rs_collect_stats(GooeyRsBatch* b) {
-  if (b->chain_units == 0.0) return;
-  float ms = 0.0f;
-  GH_CUDA(cudaEventElapsedTime(&ms, b->ev_c0, b->ev_c1));
-  std::lock_guard<std::mutex> lk(kernel_stats_mutex());
-  KernelStat& k = kernel_stats()["rs_chain_kernel"];
-  k.launches++; k.ms += ms; k.voice_frames += b->chain_units;
-  b->chain_units = 0.0;
 }
 
 }  // namespace gh
@@ -353,7 +337,7 @@ int gooey_rs_batch_bounce_device(GooeyRsBatch* b, uint32_t samples, float* out_d
   rs_bounce_impl(b, samples, out_dev, stride);
   GH_CUDA(cudaStreamSynchronize(b->stream));
   GH_CUDA(cudaEventElapsedTime(&gh::g_last_kernel_ms, b->ev0, b->ev1));
-  gh::rs_collect_stats(b);
+  b->chain_timer.collect();
   return GOOEY_E_OK;
   GOOEY_CATCH
 }
@@ -368,7 +352,7 @@ int gooey_rs_batch_bounce(GooeyRsBatch* b, uint32_t samples, float* out_host) {
   GH_CUDA(cudaMemcpy2DAsync(out_host, (size_t)samples * 4, b->d_out.p, stride * 4, (size_t)samples * 4, b->engines.size(), cudaMemcpyDeviceToHost, b->stream));
   GH_CUDA(cudaStreamSynchronize(b->stream));
   GH_CUDA(cudaEventElapsedTime(&gh::g_last_kernel_ms, b->ev0, b->ev1));
-  gh::rs_collect_stats(b);
+  b->chain_timer.collect();
   return GOOEY_E_OK;
   GOOEY_CATCH
 }
