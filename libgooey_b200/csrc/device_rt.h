@@ -1,13 +1,15 @@
 // device_rt.h — small CUDA runtime helpers shared by the host-side classes:
-// error latch, device buffers, pinned buffers, SoA state upload.
+// error latch, device buffers, once-per-device kernel attributes.
 #pragma once
 #include <cstdio>
 #include <cstdlib>
 #include <cuda_runtime.h>
 #include <cstdint>
-#include <cstdio>
 #include <cstring>
+#include <mutex>
+#include <set>
 #include <string>
+#include <tuple>
 #include <vector>
 #include <stdexcept>
 
@@ -54,18 +56,15 @@ template <class T> struct DevBuf {
   void zero(cudaStream_t s) { if (p && n) GH_CUDA(cudaMemsetAsync(p, 0, n * sizeof(T), s)); }
 };
 
-// AoS host states -> word-interleaved SoA on the device: dev[w * n_pad + v].
-template <class S> void upload_states(DevBuf<uint32_t>& dev, const std::vector<S>& host, int n_pad, cudaStream_t s) {
-  static_assert(sizeof(S) % 4 == 0, "state must be a whole number of 32-bit words");
-  constexpr size_t W = sizeof(S) / 4;
-  std::vector<uint32_t> t(W * (size_t)n_pad, 0u);
-  for (size_t v = 0; v < host.size(); v++) {
-    const uint32_t* w = reinterpret_cast<const uint32_t*>(&host[v]);
-    for (size_t i = 0; i < W; i++) t[i * n_pad + v] = w[i];
-  }
-  dev.alloc(t.size());
-  GH_CUDA(cudaMemcpyAsync(dev.p, t.data(), t.size() * 4, cudaMemcpyHostToDevice, s));
-  GH_CUDA(cudaStreamSynchronize(s));  // t is a temporary
+// cudaFuncSetAttribute(kernel, attr, value) on the current device, once per (device, kernel, attribute).  Thread safe: the
+// groups of a batch that spans several devices are rendered by one host thread each.
+inline void func_attr_once(const void* kernel, cudaFuncAttribute attr, int value) {
+  static std::mutex mu;
+  static std::set<std::tuple<int, const void*, int>> done;
+  int dev = 0;
+  GH_CUDA(cudaGetDevice(&dev));
+  std::lock_guard<std::mutex> lk(mu);
+  if (done.insert({dev, kernel, (int)attr}).second) GH_CUDA(cudaFuncSetAttribute(kernel, attr, value));
 }
 
 inline int pad32(int n) { return (n + 31) & ~31; }

@@ -5,7 +5,6 @@
 #pragma once
 #include <chrono>
 #include <cmath>
-#include <map>
 #include <memory>
 #include <functional>
 #include "pool.cuh"
@@ -268,7 +267,7 @@ struct EngineBank {
   Pool<gd::MixState> mix_pool;
   std::vector<gd::MixCfg> cfgs;           // by mix slot (host authoritative)
   DevBuf<gd::MixCfg> d_cfg;
-  DevBuf<float> ring[gd::MAX_FX]; uint32_t ring_words[gd::MAX_FX] = {0}; long long ring_cap = 0;
+  DevBuf<float> ring[gd::MAX_FX]; uint32_t ring_words[gd::MAX_FX] = {0};
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_piece = nullptr;
   // The mix of piece p runs on its own stream while the voices of piece p + 1 render into the other voice buffer.
@@ -311,7 +310,6 @@ struct EngineBank {
   std::vector<float> h_peaks;
   DevBuf<gd::VoiceEvent> d_mix_eventss[2];
   std::recursive_mutex mu;   // every use of the bank's shared buffers / streams, held for a whole render call
-  float last_ms = 0.0f;
   KernelTimer mix_timer;                  // the effect mixer of each piece of the last render (on mix_stream)
   void collect_stats() {                  // after the streams have been synchronised
     mix_timer.collect();
@@ -375,28 +373,34 @@ inline void EngineBank::clear_dirty_rings(cudaStream_t st) {
   ring_dirty.clear();
 }
 
+// An engine's voice channels: the five strips, the poly synth, the granulator.  Channel c renders into row c * n_lpad + engine
+// of a render's voice buffer, and its default instrument is the one with id c.
+constexpr int N_STRIPS = 5, CH_POLY = 5, CH_GRAN = 6, N_CH = 7;
+
 }  // namespace gh
+
+extern const float GOOEY_POLY_PRESETS[5][14];   // PolySynthConfig presets by ffi preset id (engine_api.cuh)
 
 // ---- the engine handle (opaque to C callers) --------------------------------------------------------------------------
 struct GooeyEngine {
   gh::EngineBank* bank = nullptr;
   float sr = 44100.0f, bpm = 120.0f, swing = 0.5f;
   uint32_t k = 0;                       // engine clock index (current_time = tt[k])
-  struct Strip {
+  // Every voice channel: its instrument, pool slot and the events queued for the next render.  The strips are always launched.
+  // The poly synth's and granulator's FFI calls act immediately in the reference (ffi.rs:5571-5648, 7702-7827); here they
+  // queue events that are applied before frame 0 of the next render — the same instant, since nothing ticks in between.
+  // These two are only launched once the host has touched them (until then they contribute exactly +0.0).
+  struct Voice {
     uint32_t type = 0; int slot = -1;
+    bool launched = false;
+    std::vector<gd::VoiceEvent> pending;
+  } voice[gh::N_CH];
+  struct Strip {                        // what only the strips have
     gh::HostSeq seq;
     bool muted = false, soloed = false, trig_pending = false;
     float trig_vel = 1.0f;
-    std::vector<gd::VoiceEvent> pending;
     gh::ChannelBlender blender; bool blend_enabled = false; float blend_x = 0.5f, blend_y = 0.5f;   // ffi.rs:598-600
-  } strip[5];
-  // poly synth and granulator: their FFI calls act immediately in the reference (ffi.rs:5571-5648, 7702-7827); here they
-  // queue events that are applied before frame 0 of the next render — the same instant, since nothing ticks in between.
-  // The voices are only launched once the host has touched them (until then they contribute exactly +0.0).
-  struct Aux {
-    int slot = -1; bool used = false;
-    std::vector<gd::VoiceEvent> pending;
-  } poly, gran;
+  } strip[gh::N_STRIPS];
   std::shared_ptr<gh::DevBuf<float>> gran_buf;    // may be shared by many engines (gooey_b200_granulator_share_buffer)
   uint32_t gran_len = 1; float gran_sr = 44100.0f;
   int mix_slot = -1;
@@ -498,24 +502,18 @@ inline void engine_fail(GooeyEngine* e, const std::string& msg) {   // sticky er
   if (e->error_cb && !e->error_cb_fired) { e->error_cb_fired = true; e->error_cb(e->error_ctx, e->error.c_str()); }
 }
 
-// `<Voice>::new(sample_rate)` of each channel instrument: kick(tight) / snare(tight) / hihat(short) / Tom2::new / bass(acid)
-// (ffi.rs:809-850 and :2320-2326; kick.rs:772, snare.rs:764, hihat2.rs:350, tom2.rs:199, bass.rs:608)
+// `<Voice>::new(sample_rate)` of each channel instrument: kick(tight) / snare(tight) / hihat(short) / Tom2::new / bass(acid) /
+// PolySynth (default config) / Granulator (ffi.rs:809-850 and :2320-2326; kick.rs:772, snare.rs:764, hihat2.rs:350, tom2.rs:199,
+// bass.rs:608)
 inline GooeyVoicePatch default_patch(uint32_t type) {
-  static const float KICK_TIGHT[18] = {0.22f, 0.00f, 1.00f, 0.00f, 0.12f, 0.70f, 0.01f, 0.85f, 0.64f, 1.00f, 0.07f, 0.01f, 0.02f, 0.20f, 0.00f, 0.47f, 0.12f, 0.02f};
-  static const float BASS_ACID[15] = {0.24f, 0.40f, 0.80f, 0.00f, 0.00f, 0.10f, 0.15f, 0.70f, 0.85f, 0.15f, 0.08f, 0.35f, 0.10f, 0.30f, 0.80f};
   GooeyVoicePatch p;
   memset(&p, 0, sizeof p);
   p.instrument = type;
   switch (type) {
-    case GOOEY_INSTRUMENT_KICK: memcpy(p.params, KICK_TIGHT, sizeof KICK_TIGHT); break;
-    case GOOEY_INSTRUMENT_SNARE: {  // SnareConfig::tight() = SnareConfig::new(0.2, 0.4, 0.7, 0.5, 0.029, 0.3, 0.8) (snare.rs:99-132, 270-280)
-      const float d = 0.029f;
-      const float s[19] = {0.2f, 0.4f, 0.7f, 0.5f, d, 0.3f, 0.8f, d * 0.8f, 0.091f, d * 0.6f, d, 0.495f, 0.053f, 1.0f, 0.5f, 0.0f, 0.0f, 0.125f, 0.02f};
-      memcpy(p.params, s, sizeof s);
-    } break;
+    case GOOEY_INSTRUMENT_KICK: case GOOEY_INSTRUMENT_SNARE: case GOOEY_INSTRUMENT_BASS: preset_flat(type, 0, p.params); break;
     case GOOEY_INSTRUMENT_HIHAT: { const float h[5] = {0.76f, 0.05f, 0.00f, 1.00f, 1.0f}; memcpy(p.params, h, sizeof h); } break;
-    case GOOEY_INSTRUMENT_BASS: memcpy(p.params, BASS_ACID, sizeof BASS_ACID); break;
-    default: break;   // tom: Tom2::new
+    case GOOEY_B200_VOICE_POLY: memcpy(p.params, GOOEY_POLY_PRESETS[0], sizeof GOOEY_POLY_PRESETS[0]); break;
+    default: break;   // tom: Tom2::new; the granulator takes no patch
   }
   return p;
 }
@@ -525,23 +523,11 @@ inline GooeyEngine* engine_create(int device, float sr) {
   std::lock_guard<std::recursive_mutex> lk(B.mu);
   std::unique_ptr<GooeyEngine> e(new GooeyEngine);
   e->bank = &B; e->sr = sr; e->transport.sr = sr;
-  GooeyVoicePatch p[5];
-  for (uint32_t t = 0; t < 5; t++) p[t] = default_patch(t);
-  for (int ch = 0; ch < 5; ch++) {
-    e->strip[ch].type = p[ch].instrument;
-    e->strip[ch].slot = B.voices.create(p[ch], sr);
-    e->strip[ch].seq.init(120.0f, sr);
-    e->strip[ch].blender.default_for_type(p[ch].instrument);
+  for (int c = 0; c < N_CH; c++) {
+    const GooeyVoicePatch p = default_patch((uint32_t)c);
+    e->voice[c] = {p.instrument, B.voices.create(p, sr), c < N_STRIPS, {}};
   }
-  {
-    GooeyVoicePatch q;
-    memset(&q, 0, sizeof q);
-    static const float POLY_DEFAULT[14] = {0.0f, 0.2f, 0.6f, 0.15f, 0.3f, 0.55f, 0.7f, 0.7f, 0.8f, 0.5f, 0.65f, 0.4f, 0.75f, 0.7f};   // PolySynthConfig::default (poly_synth.rs:49-66)
-    q.instrument = GOOEY_B200_VOICE_POLY; memcpy(q.params, POLY_DEFAULT, sizeof POLY_DEFAULT);
-    e->poly.slot = B.voices.create(q, sr);
-    q.instrument = GOOEY_B200_VOICE_GRANULATOR;
-    e->gran.slot = B.voices.create(q, sr);
-  }
+  for (int c = 0; c < N_STRIPS; c++) { e->strip[c].seq.init(120.0f, sr); e->strip[c].blender.default_for_type(e->voice[c].type); }
   gd::MixState ms;
   memset(&ms, 0, sizeof ms);
   for (int c = 0; c < gd::N_VOICE_CH; c++) { ms.ch_gain[c] = {1.0f, 1.0f}; ms.ch_mute[c] = {1.0f, 1.0f}; ms.ch_pan[c] = {0.5f, 0.5f}; }
@@ -577,9 +563,7 @@ inline void engine_destroy(GooeyEngine* e) {
   if (!e) return;
   EngineBank& B = *e->bank;
   std::lock_guard<std::recursive_mutex> lk(B.mu);
-  for (int ch = 0; ch < 5; ch++) B.voices.release(e->strip[ch].type, e->strip[ch].slot);
-  B.voices.release(GOOEY_B200_VOICE_POLY, e->poly.slot);
-  B.voices.release(GOOEY_B200_VOICE_GRANULATOR, e->gran.slot);
+  for (const auto& v : e->voice) B.voices.release(v.type, v.slot);
   bool holds_pcm = (bool)e->gran_buf;
   for (auto& l : e->loops) holds_pcm = holds_pcm || l.buf;
   for (auto& r : e->samplers) holds_pcm = holds_pcm || r.registered;
@@ -619,280 +603,340 @@ inline float lfo_beats(uint32_t d) { const float B[8] = {16.0f, 8.0f, 4.0f, 2.0f
 
 // First FFI touch of the poly synth / granulator of an engine: from now on the voice is launched with the engine.  It was
 // not ticked so far (an untouched poly synth / granulator is bit-exactly silent and its state does not move), so its
-// clock is set to the engine's and, for the granulator, the placeholder buffer is attached.
-inline void aux_touch(GooeyEngine* e, bool is_gran) {
-  GooeyEngine::Aux& a = is_gran ? e->gran : e->poly;
-  if (a.used) return;
-  a.used = true;
-  a.pending.push_back(make_event(0, gd::EV_SET_TIME, 1, 0.0f, e->k));
-  if (is_gran) {
-    const uint64_t ptr = (uint64_t)(uintptr_t)e->bank->d_silent.p;
-    float lo; uint32_t lo_bits = (uint32_t)ptr; memcpy(&lo, &lo_bits, 4);
-    a.pending.push_back(make_event(0, gd::EV_GRAN_BUFFER, 0, lo, (uint32_t)(ptr >> 32)));
-    a.pending.push_back(make_event(0, gd::EV_SET_AUX, gd::AUX_GRAN_BUFINFO, 44100.0f, 1));
-    e->cfg.src_gran = 1;
-  } else e->cfg.src_poly = 1;
+// clock is set to the engine's and, for the granulator, the placeholder buffer is attached.  Returns the channel's pending events.
+inline std::vector<gd::VoiceEvent>& aux_touch(GooeyEngine* e, int ch) {
+  GooeyEngine::Voice& v = e->voice[ch];
+  if (v.launched) return v.pending;
+  v.launched = true;
+  v.pending.push_back(make_event(0, gd::EV_SET_TIME, 1, 0.0f, e->k));
+  if (ch == CH_GRAN) { gran_buffer_events(v.pending, 0, e->bank->d_silent.p, 44100.0f, 1); e->cfg.src_gran = 1; }
+  else e->cfg.src_poly = 1;
   std::lock_guard<std::recursive_mutex> lk(e->bank->mu);
   e->bank->cfgs[e->mix_slot] = e->cfg;
+  return v.pending;
 }
 
-// Renders `frames` frames of every engine of `E` (all on one bank) into out_dev: mono rows [n][stride] (the bounce
-// downmix 0.5 (l + r)) or interleaved stereo rows [n][stride >= 2 frames].  `bounce`: apply the reference's bounce
-// preamble first (ffi.rs:7840-7854): clock to 0, sequencers reset + start, strips / graph / master snapped.
-// on_piece (optional): called after the mix of frames [f0, f0 + nf) has been enqueued, with the event that marks it done.
-using PieceHook = std::function<void(uint32_t f0, uint32_t nf, cudaEvent_t mixed)>;
-inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, int out_mode, bool bounce, float* out_dev, size_t stride,
-                           const PieceHook* on_piece = nullptr) {
-  if (E.empty() || frames == 0) return;
-  EngineBank& B = *E[0]->bank;
-  std::lock_guard<std::recursive_mutex> lk(B.mu);
-  GH_CUDA(cudaSetDevice(B.device));
-  cudaStream_t st = B.stream;
-  const int n = (int)E.size();
-  const int n_lpad = pad32(n);
-  // ---- schedule resolution (host): per voice and per engine event lists over the whole call ----
-  std::vector<std::vector<gd::VoiceEvent>> vev((size_t)n * 7), mev(n);   // per engine: 5 strips, poly, granulator
-  bool any_poly = false, any_gran = false;
+using PieceHook = std::function<void(uint32_t f0, uint32_t nf, cudaEvent_t mixed)>;   // see engines_render
+
+// Appends the events of `ev` from `pos` on that lie before frame `end` to `out`, rebased to frame f0, and advances `pos` past them.
+inline void take_piece(const std::vector<gd::VoiceEvent>& ev, size_t& pos, uint32_t f0, uint32_t end, std::vector<gd::VoiceEvent>& out) {
+  for (; pos < ev.size() && ev[pos].frame < end; pos++) { gd::VoiceEvent x = ev[pos]; x.frame -= f0; out.push_back(x); }
+}
+
+// GOOEY_B200_TRACE=1: per piece, the host time of its launch phases and the device times of its voice and mix stages, on
+// stderr (diagnostic)
+struct PieceTrace {
+  using Clock = std::chrono::steady_clock;
+  const bool on = getenv("GOOEY_B200_TRACE") != nullptr;
+  std::vector<cudaEvent_t> tv0, tv1, tm0, tm1;   // per piece: voice stage start / end (voice stream), mix stage start / end (mix stream)
+  Clock::time_point host[3];                     // the current piece: start, event lists built, voices launched
+  void host_mark(int k) { if (on) host[k] = Clock::now(); }
+  void mark(std::vector<cudaEvent_t>& v, cudaStream_t s) { if (!on) return; cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, s); v.push_back(e); }
+  void host_line(size_t pc) const {
+    if (!on) return;
+    auto msf = [](Clock::time_point a, Clock::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
+    fprintf(stderr, "[gooey trace] host, piece %zu: wait + event lists %.1f ms, voice launches %.1f ms, mixer launches %.1f ms\n", pc, msf(host[0], host[1]), msf(host[1], host[2]), msf(host[2], Clock::now()));
+  }
+  void device_lines(cudaStream_t st, const std::vector<uint32_t>& cuts) {   // once every piece has been enqueued on `st`
+    if (!on) return;
+    GH_CUDA(cudaStreamSynchronize(st));
+    for (size_t pc = 0; pc < tv0.size(); pc++) {
+      float a = 0, b = 0, c = 0, d = 0;
+      cudaEventElapsedTime(&a, tv0[0], tv0[pc]); cudaEventElapsedTime(&b, tv0[pc], tv1[pc]); cudaEventElapsedTime(&c, tv0[0], tm0[pc]); cudaEventElapsedTime(&d, tm0[pc], tm1[pc]);
+      fprintf(stderr, "[gooey trace] piece %zu frames %u: voices start %.1f ms, take %.1f ms; mix start %.1f ms, takes %.1f ms\n", pc, cuts[pc] - (pc ? cuts[pc - 1] : 0), a, b, c, d);
+    }
+    for (auto* v : {&tv0, &tv1, &tm0, &tm1}) for (auto e : *v) cudaEventDestroy(e);
+  }
+};
+
+// One engines_render call.  Its stages run in the order they are declared; each fills the members listed above it.
+struct EngineRender {
+  EngineBank& B;
+  const std::vector<GooeyEngine*>& E;
+  const uint32_t frames;
+  const bool bounce;
+  const int n, n_lpad;
+  const cudaStream_t st;
+  // schedule: the call's events of every voice channel ([engine * N_CH + channel]) and of every engine's mixer
+  std::vector<std::vector<gd::VoiceEvent>> vev, mev;
+  uint32_t chan_mask = 0;                 // bit c: some engine launches channel c
+  uint64_t kmin = ~0ull, kmax = 0;        // the engines' clock range
+  // external sources: one stereo row pair per loop mixer / sounding rack
+  struct ExtRef { int engine, rack; };
+  std::vector<int> loop_refs; std::vector<ExtRef> rack_refs;
+  uint32_t ext_pairs = 0;
+  // device state
+  const double* tt = nullptr;
+  size_t vstride = 0;                     // row pitch of the voice buffers
+  bool two_bufs = false;                  // more than one piece: the mix of piece p overlaps the voices of piece p + 1
+  std::vector<uint32_t> cuts;             // the end frame of every piece
+  // LFO pool
+  std::vector<std::vector<gd::ModRoute>> vroutes;   // [engine * N_CH + channel]; only strips are routed
+  struct LfoRef { int engine, lfo; };
+  std::vector<LfoRef> lfo_refs;
+  const float* lfo_planes = nullptr;
+  // pieces
+  gd::MixLaunch M;                        // filled once; every piece sets events, ev_begin, voice_buf, frames, out and ext
+  float* out = nullptr;
+  std::vector<size_t> vpos, mpos;         // the next event of every voice / mix event list
+  std::vector<gd::VoiceEvent> cur, mflat;
+  std::vector<uint32_t> mbegin;
+  PieceTrace trace;
+
+  EngineRender(EngineBank& B_, const std::vector<GooeyEngine*>& E_, uint32_t frames_, bool bounce_)
+      : B(B_), E(E_), frames(frames_), bounce(bounce_), n((int)E_.size()), n_lpad(pad32(n)), st(B_.stream),
+        vev((size_t)n * N_CH), mev(n), vpos((size_t)n * N_CH, 0), mpos(n, 0) {}
+
   // argument errors are found before any engine is touched (BadBatch -> GOOEY_E_INVALID, no sticky error)
-  {
+  void check_batch() const {
     std::set<const GooeyEngine*> seen;
-    for (int i = 0; i < n; i++) {
-      const GooeyEngine* e = E[i];
+    for (const GooeyEngine* e : E) {
       if (e->bank != &B) throw BadBatch("engines of one batch must share device and sample rate");
       if (!seen.insert(e).second) throw BadBatch("the same engine appears twice in one batch");
       if (!bounce && (uint64_t)e->k + frames >= 0xffffffffull) throw BadBatch("engine clock index would pass 2^32 frames (27 h at 44.1 kHz); bounce or recreate the engine");
     }
   }
-  uint64_t kmin = ~0ull, kmax = 0;
-  std::vector<SeqFire> fires;
-  for (int i = 0; i < n; i++) {
-    GooeyEngine* e = E[i];
-    if (bounce) {
-      e->k = 0;
-      for (auto& s : e->strip) { s.seq.reset(); s.seq.start(); }
-    }
-    kmin = std::min<uint64_t>(kmin, e->k);
-    kmax = std::max<uint64_t>(kmax, (uint64_t)e->k + frames);
-    auto& mx = mev[i];
-    mx = e->mix_pending; e->mix_pending.clear();
-    if (bounce) {
-      mx.push_back(make_event(0, gd::MX_SNAP, 0, 0.0f));       // voice strips snap to their current targets
-    }
-    // per-buffer mute / solo targets (ffi.rs:1099-1109, graph.rs update_mute_solo_targets)
-    bool any_solo = false;
-    for (auto& s : e->strip) any_solo |= s.soloed;
-    bool any_tsolo = false;
-    for (uint32_t t = 0; t < e->cfg.n_tracks; t++) any_tsolo |= e->track_soloed[t];
-    std::vector<gd::VoiceEvent> mute_ev;
-    for (int ch = 0; ch < 5; ch++) {
-      const auto& s = e->strip[ch];
-      mute_ev.push_back(make_event(0, gd::MX_SET, gd::MP_CH_MUTE + ch, s.soloed ? 1.0f : (any_solo ? 0.0f : (s.muted ? 0.0f : 1.0f))));
-    }
-    std::vector<gd::VoiceEvent> tmute_ev;
-    for (uint32_t t = 0; t < e->cfg.n_tracks; t++)
-      tmute_ev.push_back(make_event(0, gd::MX_SET, gd::MP_TR_MUTE + t, e->track_soloed[t] ? 1.0f : ((any_tsolo || e->track_muted[t]) ? 0.0f : 1.0f)));
-    if (bounce) {
-      // graph.snap_strip_params() refreshes the track mute targets and snaps; master_gain.snap(); the voice-strip
-      // mute targets are only written by render() afterwards, so they glide (ffi.rs:7846-7854, 1099-1109)
-      mx.insert(mx.end(), tmute_ev.begin(), tmute_ev.end());
-      mx.push_back(make_event(0, gd::MX_SNAP, 1, 0.0f));
-      mx.push_back(make_event(0, gd::MX_SNAP, 2, 0.0f));
-      mx.insert(mx.end(), mute_ev.begin(), mute_ev.end());
-    } else {
-      mx.insert(mx.end(), mute_ev.begin(), mute_ev.end());
-      mx.insert(mx.end(), tmute_ev.begin(), tmute_ev.end());
-    }
-    for (int ax = 0; ax < 2; ax++) {   // immediate-mode events first, then the bounce's clock reset
-      GooeyEngine::Aux& a = ax ? e->gran : e->poly;
-      if (!a.used) continue;
-      (ax ? any_gran : any_poly) = true;
-      auto& ev = vev[(size_t)i * 7 + 5 + ax];
-      ev = a.pending; a.pending.clear();
-      if (bounce) ev.push_back(make_event(0, gd::EV_SET_TIME, 0, 0.0f, 0));
-    }
-    struct MidiKey { uint32_t frame, seq, ch; float vel; };
+
+  // ---- per-engine schedule (host): event lists over the whole call ----
+  struct MidiKey { uint32_t frame, seq, ch; float vel; };
+  void schedule() {
+    std::vector<SeqFire> fires;
     std::vector<MidiKey> midi;
-    for (int ch = 0; ch < 5; ch++) {
-      auto& s = e->strip[ch];
-      auto& ev = vev[(size_t)i * 7 + ch];
-      ev.insert(ev.end(), s.pending.begin(), s.pending.end());
-      s.pending.clear();
+    for (int i = 0; i < n; i++) {
+      GooeyEngine* e = E[i];
+      if (bounce) {
+        e->k = 0;
+        for (auto& s : e->strip) { s.seq.reset(); s.seq.start(); }
+      }
+      kmin = std::min<uint64_t>(kmin, e->k);
+      kmax = std::max<uint64_t>(kmax, (uint64_t)e->k + frames);
+      mix_events(e, mev[i]);
+      midi.clear();
+      channel_events(e, &vev[(size_t)i * N_CH], midi, fires);
+      midi_export(e, midi);
+    }
+  }
+  // pending mixer edits, the bounce preamble's snaps and the per-buffer mute / solo targets (ffi.rs:1099-1109, graph.rs
+  // update_mute_solo_targets)
+  void mix_events(GooeyEngine* e, std::vector<gd::VoiceEvent>& mx) const {
+    mx = e->mix_pending; e->mix_pending.clear();
+    if (bounce) mx.push_back(make_event(0, gd::MX_SNAP, 0, 0.0f));       // voice strips snap to their current targets
+    bool any_solo = false, any_tsolo = false;
+    for (auto& s : e->strip) any_solo |= s.soloed;
+    for (uint32_t t = 0; t < e->cfg.n_tracks; t++) any_tsolo |= e->track_soloed[t];
+    auto strip_mutes = [&] {
+      for (int ch = 0; ch < N_STRIPS; ch++) {
+        const auto& s = e->strip[ch];
+        mx.push_back(make_event(0, gd::MX_SET, gd::MP_CH_MUTE + ch, s.soloed ? 1.0f : (any_solo ? 0.0f : (s.muted ? 0.0f : 1.0f))));
+      }
+    };
+    auto track_mutes = [&] {
+      for (uint32_t t = 0; t < e->cfg.n_tracks; t++)
+        mx.push_back(make_event(0, gd::MX_SET, gd::MP_TR_MUTE + t, e->track_soloed[t] ? 1.0f : ((any_tsolo || e->track_muted[t]) ? 0.0f : 1.0f)));
+    };
+    if (!bounce) { strip_mutes(); track_mutes(); return; }
+    // graph.snap_strip_params() refreshes the track mute targets and snaps; master_gain.snap(); the voice-strip
+    // mute targets are only written by render() afterwards, so they glide (ffi.rs:7846-7854, 1099-1109)
+    track_mutes();
+    mx.push_back(make_event(0, gd::MX_SNAP, 1, 0.0f));
+    mx.push_back(make_event(0, gd::MX_SNAP, 2, 0.0f));
+    strip_mutes();
+  }
+  // every launched channel: its pending events, then the bounce's clock reset; a strip then adds its manual trigger and its
+  // sequencer's fires (ffi.rs:1162-1198), and both go to the MIDI export
+  void channel_events(GooeyEngine* e, std::vector<gd::VoiceEvent>* out_ev, std::vector<MidiKey>& midi, std::vector<SeqFire>& fires) {
+    for (int ch = 0; ch < N_CH; ch++) {
+      GooeyEngine::Voice& v = e->voice[ch];
+      if (!v.launched) continue;
+      chan_mask |= 1u << ch;
+      auto& ev = out_ev[ch];
+      ev.insert(ev.end(), v.pending.begin(), v.pending.end());
+      v.pending.clear();
       // the bounce's clock reset comes after the pending edits: a voice swapped in since the last render carries a
       // "join the engine clock at k" event that must not outlive the reset (the clock window of a bounce is [0, frames])
       if (bounce) ev.push_back(make_event(0, gd::EV_SET_TIME, 0, 0.0f, 0));
+      if (ch >= N_STRIPS) continue;
+      auto& s = e->strip[ch];
       if (s.trig_pending) { s.trig_pending = false; ev.push_back(make_event(0, gd::EV_TRIGGER, 0, s.trig_vel)); midi.push_back({0u, 0u, (uint32_t)ch, s.trig_vel}); }
       fires.clear();
       s.seq.run(frames, fires);
-      if (e->seq_triggers_enabled) {
-        for (const SeqFire& f : fires) midi.push_back({f.frame, 1u, (uint32_t)ch, f.velocity});
-        for (const SeqFire& f : fires) {   // ffi.rs:1162-1198
-          // apply_sequencer_blend_setting (:1384-1402): the step's own blend, else the channel's pad position when blending is
-          // on; a blend that was applied is followed by snap_params (:1168-1171)
-          auto add = [&](const gd::VoiceEvent& x) { ev.push_back(x); };
-          if (f.has_blend) s.blender.apply(f.bx, f.by, f.frame, add);
-          else if (s.blend_enabled) s.blender.apply(s.blend_x, s.blend_y, f.frame, add);
-          if (f.has_blend || s.blend_enabled) ev.push_back(make_event(f.frame, gd::EV_SNAP, 0, 0.0f));
-          float mn, mxf;
-          if (f.has_note) { if (note_freq_range(s.type, mn, mxf)) ev.push_back(make_event(f.frame, gd::EV_NOTE_FREQ, 0, midi_to_norm(f.note, mn, mxf))); }
-          else ev.push_back(make_event(f.frame, gd::EV_RESTORE_FREQ, 0, 0.0f));
-          ev.push_back(make_event(f.frame, gd::EV_TRIGGER, 0, f.velocity));
-        }
-      }
-    }
-    // MIDI note-on export (ffi.rs:994-1004, 1079-1094, 1196): manual triggers first (offset 0, channel order), then the sequencer's
-    // in frame / channel order; the list is cleared by every render() call and capped at 64, and a bounce IS a run of 512-frame
-    // render() calls (ffi.rs:7855-7870), so after a bounce only the last chunk's events are pending, offsets relative to it.
-    {
-      std::stable_sort(midi.begin(), midi.end(), [](const MidiKey& a, const MidiKey& b) {
-        return a.frame != b.frame ? a.frame < b.frame : (a.seq != b.seq ? a.seq < b.seq : a.ch < b.ch); });
-      const uint32_t base = bounce ? ((frames - 1) / 512u) * 512u : 0u;
-      e->midi_events.clear();
-      for (const MidiKey& m : midi) {
-        if (m.frame < base) continue;
-        if (e->midi_events.size() >= 64) break;
-        e->midi_events.push_back({m.ch, m.vel, m.frame - base});
+      if (!e->seq_triggers_enabled) continue;
+      for (const SeqFire& f : fires) midi.push_back({f.frame, 1u, (uint32_t)ch, f.velocity});
+      for (const SeqFire& f : fires) {
+        // apply_sequencer_blend_setting (:1384-1402): the step's own blend, else the channel's pad position when blending is
+        // on; a blend that was applied is followed by snap_params (:1168-1171)
+        auto add = [&](const gd::VoiceEvent& x) { ev.push_back(x); };
+        if (f.has_blend) s.blender.apply(f.bx, f.by, f.frame, add);
+        else if (s.blend_enabled) s.blender.apply(s.blend_x, s.blend_y, f.frame, add);
+        if (f.has_blend || s.blend_enabled) ev.push_back(make_event(f.frame, gd::EV_SNAP, 0, 0.0f));
+        float mn, mxf;
+        if (f.has_note) { if (note_freq_range(v.type, mn, mxf)) ev.push_back(make_event(f.frame, gd::EV_NOTE_FREQ, 0, midi_to_norm(f.note, mn, mxf))); }
+        else ev.push_back(make_event(f.frame, gd::EV_RESTORE_FREQ, 0, 0.0f));
+        ev.push_back(make_event(f.frame, gd::EV_TRIGGER, 0, f.velocity));
       }
     }
   }
+  // MIDI note-on export (ffi.rs:994-1004, 1079-1094, 1196): manual triggers first (offset 0, channel order), then the sequencer's
+  // in frame / channel order; the list is cleared by every render() call and capped at 64, and a bounce IS a run of 512-frame
+  // render() calls (ffi.rs:7855-7870), so after a bounce only the last chunk's events are pending, offsets relative to it.
+  void midi_export(GooeyEngine* e, std::vector<MidiKey>& midi) const {
+    std::stable_sort(midi.begin(), midi.end(), [](const MidiKey& a, const MidiKey& b) {
+      return a.frame != b.frame ? a.frame < b.frame : (a.seq != b.seq ? a.seq < b.seq : a.ch < b.ch); });
+    const uint32_t base = bounce ? ((frames - 1) / 512u) * 512u : 0u;
+    e->midi_events.clear();
+    for (const MidiKey& m : midi) {
+      if (m.frame < base) continue;
+      if (e->midi_events.size() >= 64) break;
+      e->midi_events.push_back({m.ch, m.vel, m.frame - base});
+    }
+  }
+
   // ---- sample-playback sources: one descriptor per engine with a loaded loop / per rack with a sounding voice ----
-  B.h_loop_descs.clear(); B.h_rack_descs.clear();
-  struct ExtRef { int engine, rack; };
-  std::vector<int> loop_refs; std::vector<ExtRef> rack_refs;
-  std::vector<gd::SamplerHit> rack_hits; std::vector<size_t> rack_hit_off;
-  uint32_t ext_pairs = 0;
-  for (int i = 0; i < n; i++) {
-    GooeyEngine* e = E[i];
-    e->cfg.src_ext = 0;
-    for (int s = 0; s < gd::EXT_SOURCES; s++) e->cfg.ext_row[s] = 0;
-    // Mixer::tick writes the gate targets every sample from the mute / solo flags, which only change between calls (mod.rs:63-72)
-    bool any_lsolo = false, any_loaded = false;
-    for (auto& l : e->loops) { any_lsolo = any_lsolo || l.soloed; any_loaded = any_loaded || (l.buf && l.len > 0); }
-    for (auto& l : e->loops) gd::lsm_set(l.active, (any_lsolo ? l.soloed : !l.muted) ? 1.0f : 0.0f, 0.0f, 1.0f);
-    if (any_loaded) {
-      gd::LoopMixer m;
-      memset(&m, 0, sizeof m);
-      for (int c = 0; c < gd::LOOP_CHANNELS; c++) {
-        auto& l = e->loops[c];
-        l.describe(m.ch[c], e->loop_engine_bpm);
-        B.attach_stretcher(l, m.ch[c]);
+  void ext_sources() {
+    B.h_loop_descs.clear(); B.h_rack_descs.clear();
+    std::vector<gd::SamplerHit> rack_hits; std::vector<size_t> rack_hit_off;
+    for (int i = 0; i < n; i++) {
+      GooeyEngine* e = E[i];
+      e->cfg.src_ext = 0;
+      for (int s = 0; s < gd::EXT_SOURCES; s++) e->cfg.ext_row[s] = 0;
+      // Mixer::tick writes the gate targets every sample from the mute / solo flags, which only change between calls (mod.rs:63-72)
+      bool any_lsolo = false, any_loaded = false;
+      for (auto& l : e->loops) { any_lsolo = any_lsolo || l.soloed; any_loaded = any_loaded || (l.buf && l.len > 0); }
+      for (auto& l : e->loops) gd::lsm_set(l.active, (any_lsolo ? l.soloed : !l.muted) ? 1.0f : 0.0f, 0.0f, 1.0f);
+      if (any_loaded) {
+        gd::LoopMixer m;
+        memset(&m, 0, sizeof m);
+        for (int c = 0; c < gd::LOOP_CHANNELS; c++) {
+          auto& l = e->loops[c];
+          l.describe(m.ch[c], e->loop_engine_bpm);
+          B.attach_stretcher(l, m.ch[c]);
+        }
+        m.row = ext_pairs;
+        e->cfg.src_ext |= 1u; e->cfg.ext_row[0] = ext_pairs++;
+        B.h_loop_descs.push_back(m); loop_refs.push_back(i);
+      } else {
+        // nothing to read: the channels output exactly 0 and only their smoothers move (they tick every sample, :202-207)
+        for (auto& l : e->loops)
+          for (uint32_t f = 0; f < frames && (l.gain.c != l.gain.t || l.active.c != l.active.t); f++) { gd::lsm_tick(l.gain, B.rc.smooth15); gd::lsm_tick(l.active, B.rc.smooth15); }
       }
-      m.row = ext_pairs;
-      e->cfg.src_ext |= 1u; e->cfg.ext_row[0] = ext_pairs++;
-      B.h_loop_descs.push_back(m); loop_refs.push_back(i);
-    } else {
-      // nothing to read: the channels output exactly 0 and only their smoothers move (they tick every sample, :202-207)
-      for (auto& l : e->loops)
-        for (uint32_t f = 0; f < frames && (l.gain.c != l.gain.t || l.active.c != l.active.t); f++) { gd::lsm_tick(l.gain, B.rc.smooth15); gd::lsm_tick(l.active, B.rc.smooth15); }
-    }
-    // rack patterns: resolved on the host into pad hits (resolve_rack_patterns above)
-    gh::RackPattern* pats[gd::SAMPLER_RACKS];
-    std::vector<gh::RackHit> rhits[gd::SAMPLER_RACKS];
-    bool any_rack = false;
-    for (int r = 0; r < gd::SAMPLER_RACKS; r++) { pats[r] = e->samplers[r].registered ? &e->samplers[r].pat : nullptr; any_rack = any_rack || pats[r]; }
-    if (any_rack) gh::resolve_rack_patterns(e->transport, pats, gd::SAMPLER_RACKS, frames, bounce, e->seq_triggers_enabled, rhits);
-    else if (e->transport.running) e->transport.lazy += frames;       // nothing listens to the transport: it just advances
-    for (int r = 0; any_rack && r < gd::SAMPLER_RACKS; r++) {
-      auto& R = e->samplers[r];
-      if (!R.registered) continue;
-      std::vector<gd::SamplerHit> hits;
-      for (const gh::RackHit& h : rhits[r]) hits.push_back(gd::SamplerHit{h.frame, h.slot, h.velocity, 0u});
-      bool sounding = false;
-      for (const auto& v : R.voices) sounding = sounding || v.samples != nullptr;
-      if (!sounding && hits.empty()) continue;         // no active voice and no hit: the rack ticks to exactly 0 and its state does not move
-      gd::SamplerRack d;
-      memset(&d, 0, sizeof d);
-      memcpy(d.v, R.voices, sizeof d.v);
-      d.row = ext_pairs; d.rack = (uint32_t)r;
-      for (int k = 0; k < gd::SAMPLER_SLOTS; k++) {
-        const auto& S = R.slots[k];
-        if (S.buf) d.slots[k] = gd::SamplerSlotRef{S.buf->p, S.frames, S.channels, (double)S.sr / (double)e->sr};
+      // rack patterns: resolved on the host into pad hits (resolve_rack_patterns above)
+      gh::RackPattern* pats[gd::SAMPLER_RACKS];
+      std::vector<gh::RackHit> rhits[gd::SAMPLER_RACKS];
+      bool any_rack = false;
+      for (int r = 0; r < gd::SAMPLER_RACKS; r++) { pats[r] = e->samplers[r].registered ? &e->samplers[r].pat : nullptr; any_rack = any_rack || pats[r]; }
+      if (any_rack) gh::resolve_rack_patterns(e->transport, pats, gd::SAMPLER_RACKS, frames, bounce, e->seq_triggers_enabled, rhits);
+      else if (e->transport.running) e->transport.lazy += frames;       // nothing listens to the transport: it just advances
+      for (int r = 0; any_rack && r < gd::SAMPLER_RACKS; r++) {
+        auto& R = e->samplers[r];
+        if (!R.registered) continue;
+        std::vector<gd::SamplerHit> hits;
+        for (const gh::RackHit& h : rhits[r]) hits.push_back(gd::SamplerHit{h.frame, h.slot, h.velocity, 0u});
+        bool sounding = false;
+        for (const auto& v : R.voices) sounding = sounding || v.samples != nullptr;
+        if (!sounding && hits.empty()) continue;         // no active voice and no hit: the rack ticks to exactly 0 and its state does not move
+        gd::SamplerRack d;
+        memset(&d, 0, sizeof d);
+        memcpy(d.v, R.voices, sizeof d.v);
+        d.row = ext_pairs; d.rack = (uint32_t)r;
+        for (int k = 0; k < gd::SAMPLER_SLOTS; k++) {
+          const auto& S = R.slots[k];
+          if (S.buf) d.slots[k] = gd::SamplerSlotRef{S.buf->p, S.frames, S.channels, (double)S.sr / (double)e->sr};
+        }
+        d.next_age = R.next_age;
+        d.n_hits = (uint32_t)hits.size(); d.next_hit = 0; d.cur_frame = 0;
+        rack_hit_off.push_back(rack_hits.size());
+        rack_hits.insert(rack_hits.end(), hits.begin(), hits.end());
+        e->cfg.src_ext |= 2u << r; e->cfg.ext_row[1 + r] = ext_pairs++;
+        B.h_rack_descs.push_back(d); rack_refs.push_back({i, r});
       }
-      d.next_age = R.next_age;
-      d.n_hits = (uint32_t)hits.size(); d.next_hit = 0; d.cur_frame = 0;
-      rack_hit_off.push_back(rack_hits.size());
-      rack_hits.insert(rack_hits.end(), hits.begin(), hits.end());
-      e->cfg.src_ext |= 2u << r; e->cfg.ext_row[1 + r] = ext_pairs++;
-      B.h_rack_descs.push_back(d); rack_refs.push_back({i, r});
+      B.cfgs[e->mix_slot] = e->cfg;
     }
-    B.cfgs[e->mix_slot] = e->cfg;
+    if (!rack_hits.empty()) {                             // one flat hit table for the call; the descriptors point into it
+      B.d_rack_hits.upload(rack_hits.data(), rack_hits.size(), st);
+      for (size_t q = 0; q < B.h_rack_descs.size(); q++) if (B.h_rack_descs[q].n_hits) B.h_rack_descs[q].hits = B.d_rack_hits.p + rack_hit_off[q];
+    }
   }
-  if (!rack_hits.empty()) {                             // one flat hit table for the call; the descriptors point into it
-    B.d_rack_hits.upload(rack_hits.data(), rack_hits.size(), st);
-    for (size_t q = 0; q < B.h_rack_descs.size(); q++) if (B.h_rack_descs[q].n_hits) B.h_rack_descs[q].hits = B.d_rack_hits.p + rack_hit_off[q];
-  }
-  const double* tt = B.clock.view(clock_table(B.sr), kmin, kmax, st);
-  // ---- device state: pools, configs, rings ----
-  B.mix_pool.flush(st);
-  B.d_cfg.upload(B.cfgs.data(), B.cfgs.size(), st);
-  uint32_t need_words[gd::MAX_FX] = {0};
-  for (int i = 0; i < n; i++) {
-    const gd::MixCfg& c = E[i]->cfg;
+
+  // ---- device state: clock window, pools, configs, rings, piece geometry, buffers ----
+  void device_state() {
+    tt = B.clock.view(clock_table(B.sr), kmin, kmax, st);
+    B.mix_pool.flush(st);
+    B.d_cfg.upload(B.cfgs.data(), B.cfgs.size(), st);
+    uint32_t need_words[gd::MAX_FX] = {0};
+    for (int i = 0; i < n; i++) {
+      const gd::MixCfg& c = E[i]->cfg;
+      for (int s = 0; s < gd::MAX_FX; s++) {
+        const bool used = c.fx_kind[s] != gd::FXK_NONE && (s >= 4 || c.fx_enabled[s] != 0);
+        if (used) need_words[s] = std::max(need_words[s], ring_words_of(B.geo, c.fx_kind[s]));
+      }
+    }
+    B.clear_dirty_rings(st);
+    // every arena shares one row pitch (the mix pool's capacity); arenas that already exist are re-laid when it grows
     for (int s = 0; s < gd::MAX_FX; s++) {
-      const bool used = c.fx_kind[s] != gd::FXK_NONE && (s >= 4 || c.fx_enabled[s] != 0);
-      if (used) need_words[s] = std::max(need_words[s], ring_words_of(B.geo, c.fx_kind[s]));
+      const uint32_t words = std::max(need_words[s], B.ring_words[s]);
+      if (words) B.ensure_ring(s, words, B.mix_pool.cap);
     }
-  }
-  B.clear_dirty_rings(st);
-  // every arena shares one row pitch (the mix pool's capacity); arenas that already exist are re-laid when it grows
-  const long long ring_cap = B.mix_pool.cap;
-  for (int s = 0; s < gd::MAX_FX; s++) {
-    const uint32_t words = std::max(need_words[s], B.ring_words[s]);
-    if (words) B.ensure_ring(s, words, ring_cap);
-  }
-  std::vector<uint32_t> mix_slots(n);
-  for (int i = 0; i < n; i++) mix_slots[i] = (uint32_t)E[i]->mix_slot;
-  B.d_mix_slots.upload(mix_slots.data(), n, st);
-  // ---- pieces: bound the voice buffer (5 rows per engine) to ~2 GiB ----
-  const int n_ch = any_gran ? 7 : (any_poly ? 6 : 5);
-  const size_t rows = (size_t)n_ch * n_lpad;
-  size_t piece = ((size_t)2 << 30) / (rows * 4);
-  piece = std::min<size_t>(std::max<size_t>(piece & ~(size_t)31, 2048), 65536);
-  piece = std::min<size_t>(piece, (frames + 31) & ~31u);
-  const bool two_bufs = frames > piece || frames > 4096;      // more than one piece: overlap mix(p) with voices(p + 1)
-  // row pitch of the voice buffers: an odd multiple of 32 frames (the mixer reads 32 rows x 7 channels per tile; rows a power of
-  // two apart would all fall into the same cache sets)
-  const size_t vstride = ((piece / 32) & 1) ? piece : piece + 32;
-  B.d_voice_bufs[0].alloc(rows * vstride);
-  if (two_bufs) B.d_voice_bufs[1].alloc(rows * vstride);
-  if (ext_pairs) {
-    B.d_ext[0].alloc((size_t)2 * ext_pairs * vstride);
-    if (two_bufs) B.d_ext[1].alloc((size_t)2 * ext_pairs * vstride);
-    if (!B.h_loop_descs.empty()) B.d_loop_descs.upload(B.h_loop_descs.data(), B.h_loop_descs.size(), st);
-    if (!B.h_rack_descs.empty()) B.d_rack_descs.upload(B.h_rack_descs.data(), B.h_rack_descs.size(), st);
-  }
-  {
+    std::vector<uint32_t> mix_slots(n);
+    for (int i = 0; i < n; i++) mix_slots[i] = (uint32_t)E[i]->mix_slot;
+    B.d_mix_slots.upload(mix_slots.data(), n, st);
+    // pieces: bound the voice buffer (a row per engine and launched channel) to ~2 GiB
+    int n_ch = 0;
+    for (int c = 0; c < N_CH; c++) if (chan_mask >> c & 1u) n_ch = c + 1;
+    const size_t rows = (size_t)n_ch * n_lpad;
+    size_t piece = ((size_t)2 << 30) / (rows * 4);
+    piece = std::min<size_t>(std::max<size_t>(piece & ~(size_t)31, 2048), 65536);
+    piece = std::min<size_t>(piece, (frames + 31) & ~31u);
+    two_bufs = frames > piece || frames > 4096;
+    // row pitch of the voice buffers: an odd multiple of 32 frames (the mixer reads 32 rows x 7 channels per tile; rows a power of
+    // two apart would all fall into the same cache sets)
+    vstride = ((piece / 32) & 1) ? piece : piece + 32;
+    B.d_voice_bufs[0].alloc(rows * vstride);
+    if (two_bufs) B.d_voice_bufs[1].alloc(rows * vstride);
+    if (ext_pairs) {
+      B.d_ext[0].alloc((size_t)2 * ext_pairs * vstride);
+      if (two_bufs) B.d_ext[1].alloc((size_t)2 * ext_pairs * vstride);
+      if (!B.h_loop_descs.empty()) B.d_loop_descs.upload(B.h_loop_descs.data(), B.h_loop_descs.size(), st);
+      if (!B.h_rack_descs.empty()) B.d_rack_descs.upload(B.h_rack_descs.data(), B.h_rack_descs.size(), st);
+    }
     bool any_chain = false;
     for (int i = 0; i < n && !any_chain; i++) for (int q = 0; q < gd::MAX_FX; q++) any_chain = any_chain || (E[i]->cfg.fx_kind[q] != gd::FXK_NONE && E[i]->cfg.fx_enabled[q]);
     if (any_chain) B.d_premix.alloc((size_t)2 * n_lpad * vstride);
+    // Piece schedule.  Parameters edited through the FFI glide for ~10 smoother time constants (kick.rs: 15 ms -> ~6000
+    // samples) and the planner keeps a voice on the per-sample general path for a whole piece while anything glides, so the
+    // first pieces are short: a gliding voice re-enters the time-parallel path within a few thousand frames.
+    const uint32_t lead[10] = {2048, 2048, 2048, 2048, 2048, 2048, 4096, 4096, 8192, 16384};
+    uint32_t f = 0;
+    for (int k = 0; k < 10 && f + lead[k] < frames && lead[k] < piece; k++) { f += lead[k]; cuts.push_back(f); }
+    while (f + piece < frames) { f += (uint32_t)piece; cuts.push_back(f); }
+    cuts.push_back(frames);
   }
+
   // ---- LFO pool: one stream per enabled LFO; routed ones get a plane of per-frame values (computed on the device) ----
-  std::vector<std::vector<gd::ModRoute>> vroutes((size_t)n * 5);
-  struct LfoRef { int engine, lfo; };
-  std::vector<LfoRef> lfo_refs;
-  B.h_lfo_streams.clear();
-  int n_planes = 0;
-  for (int i = 0; i < n; i++) {
-    GooeyEngine* e = E[i];
-    for (int li = 0; li < 8; li++) {
-      if (!e->lfo_enabled[li]) continue;
-      gd::LfoStream sdesc;
-      volatile float bps = e->bpm / 60.0f;                                   // MusicalDivision::to_frequency (lfo.rs:27-33)
-      volatile float freq = bps / lfo_beats(e->lfos[li].division);
-      sdesc.phase = e->lfos[li].phase; sdesc.inc = freq / e->sr; sdesc.amount = e->lfos[li].amount; sdesc.offset = e->lfos[li].offset;
-      sdesc.plane = -1;
-      for (const auto& r : e->lfo_routes[li]) {
-        if (r.instrument >= 5) continue;                                     // voice_mut(channel) is None
-        uint32_t param, mode;
-        if (!lfo_route_target(e->strip[r.instrument].type, r.param, param, mode)) continue;
-        if (sdesc.plane < 0) sdesc.plane = n_planes++;
-        vroutes[(size_t)i * 5 + r.instrument].push_back(gd::ModRoute{param, mode, r.depth, (uint32_t)sdesc.plane});
+  void lfo_pool() {
+    vroutes.resize((size_t)n * N_CH);
+    B.h_lfo_streams.clear();
+    int n_planes = 0;
+    for (int i = 0; i < n; i++) {
+      GooeyEngine* e = E[i];
+      for (int li = 0; li < 8; li++) {
+        if (!e->lfo_enabled[li]) continue;
+        gd::LfoStream sdesc;
+        volatile float bps = e->bpm / 60.0f;                                   // MusicalDivision::to_frequency (lfo.rs:27-33)
+        volatile float freq = bps / lfo_beats(e->lfos[li].division);
+        sdesc.phase = e->lfos[li].phase; sdesc.inc = freq / e->sr; sdesc.amount = e->lfos[li].amount; sdesc.offset = e->lfos[li].offset;
+        sdesc.plane = -1;
+        for (const auto& r : e->lfo_routes[li]) {
+          if (r.instrument >= (uint32_t)N_STRIPS) continue;                    // voice_mut(channel) is None
+          uint32_t param, mode;
+          if (!lfo_route_target(e->voice[r.instrument].type, r.param, param, mode)) continue;
+          if (sdesc.plane < 0) sdesc.plane = n_planes++;
+          vroutes[(size_t)i * N_CH + r.instrument].push_back(gd::ModRoute{param, mode, r.depth, (uint32_t)sdesc.plane});
+        }
+        B.h_lfo_streams.push_back(sdesc);
+        lfo_refs.push_back({i, li});
       }
-      B.h_lfo_streams.push_back(sdesc);
-      lfo_refs.push_back({i, li});
     }
-  }
-  const float* lfo_planes = nullptr;
-  if (!B.h_lfo_streams.empty()) {
+    if (B.h_lfo_streams.empty()) return;
     B.d_lfo_streams.upload(B.h_lfo_streams.data(), B.h_lfo_streams.size(), st);
     if (n_planes) B.d_lfo_planes.alloc((size_t)n_planes * frames);
     gd::lfo_kernel<<<((int)B.h_lfo_streams.size() + 63) / 64, 64, 0, st>>>(B.d_lfo_streams.p, (int)B.h_lfo_streams.size(), B.d_lfo_planes.p, (long long)frames, (int)frames);
@@ -900,59 +944,59 @@ inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, 
     GH_CUDA(cudaGetLastError());
     if (n_planes) lfo_planes = B.d_lfo_planes.p;
   }
-  B.d_peaks.alloc((size_t)n * gd::N_PEAKS);
-  GH_CUDA(cudaMemsetAsync(B.d_peaks.p, 0, (size_t)n * gd::N_PEAKS * 4, st));
-  B.d_chain_units.alloc(1);
-  GH_CUDA(cudaMemsetAsync(B.d_chain_units.p, 0, sizeof(unsigned long long), st));
-  cudaStream_t ms = B.mix_stream;
-  GH_CUDA(cudaEventRecord(B.ev_piece, st));
-  GH_CUDA(cudaStreamWaitEvent(ms, B.ev_piece, 0));             // the mix stream starts after everything queued so far (uploads, ring set-up)
-  GH_CUDA(cudaEventRecord(B.ev0, st));
-  B.mix_timer.clear();
-  std::vector<gd::VoiceEvent> cur, mflat;
-  std::vector<uint32_t> mbegin;
-  std::vector<size_t> vpos((size_t)n * 7, 0), mpos(n, 0);
-  // Piece schedule.  Parameters edited through the FFI glide for ~10 smoother time constants (kick.rs: 15 ms -> ~6000
-  // samples) and the planner keeps a voice on the per-sample general path for a whole piece while anything glides, so the
-  // first pieces are short: a gliding voice re-enters the time-parallel path within a few thousand frames.
-  std::vector<uint32_t> cuts;
-  {
-    const uint32_t lead[10] = {2048, 2048, 2048, 2048, 2048, 2048, 4096, 4096, 8192, 16384};
-    uint32_t f = 0;
-    for (int k = 0; k < 10 && f + lead[k] < frames && lead[k] < piece; k++) { f += lead[k]; cuts.push_back(f); }
-    while (f + piece < frames) { f += (uint32_t)piece; cuts.push_back(f); }
-    cuts.push_back(frames);
+
+  // ---- the mixer's launch record and the call's meters; the mix stream starts after everything queued so far ----
+  void mixer_setup(int out_mode, float* out_dev, size_t stride) {
+    B.d_peaks.alloc((size_t)n * gd::N_PEAKS);
+    GH_CUDA(cudaMemsetAsync(B.d_peaks.p, 0, (size_t)n * gd::N_PEAKS * 4, st));
+    B.d_chain_units.alloc(1);
+    GH_CUDA(cudaMemsetAsync(B.d_chain_units.p, 0, sizeof(unsigned long long), st));
+    B.d_mix_fast.alloc(n); B.d_mix_consts.alloc(n);
+    out = out_dev;
+    memset(&M, 0, sizeof M);
+    M.state = B.mix_pool.d.p; M.n = n; M.state_cap = B.mix_pool.cap; M.slots = B.d_mix_slots.p; M.n_lpad = n_lpad;
+    M.cfg = B.d_cfg.p; M.voice_stride = (long long)vstride; M.chan_mask = chan_mask;
+    for (int s = 0; s < gd::MAX_FX; s++) M.ring[s] = B.ring[s].p;
+    M.ring_cap = B.mix_pool.cap;
+    M.out_stride = (long long)stride; M.out_mode = out_mode; M.out_rows = nullptr;
+    M.rc = B.rc; M.geo = B.geo;
+    M.center_l = gm::g_cosf(0.5f * 1.57079632679489661923f); M.center_r = gm::g_sinf(0.5f * 1.57079632679489661923f);
+    M.fast = B.d_mix_fast.p; M.consts = B.d_mix_consts.p;
+    M.peaks = B.d_peaks.p;
+    M.premix = B.d_premix.p; M.premix_stride = (long long)vstride;
+    M.ext_stride = (long long)vstride;
+    M.chain_units = B.d_chain_units.p;
+    // dynamic shared memory beyond 48 KB (with the static tiles)
+    func_attr_once((const void*)gd::mix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gd::MIX_DYN_SMEM);
+    func_attr_once((const void*)gd::chain_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gd::CHAIN_SMEM);
+    GH_CUDA(cudaEventRecord(B.ev_piece, st));
+    GH_CUDA(cudaStreamWaitEvent(B.mix_stream, B.ev_piece, 0));   // after the uploads and the ring set-up
+    GH_CUDA(cudaEventRecord(B.ev0, st));
+    B.mix_timer.clear();
   }
-  // GOOEY_B200_TRACE=1: per-piece device times of the voice stage and of the mix stage on stderr (diagnostic)
-  const bool trace = getenv("GOOEY_B200_TRACE") != nullptr;
-  std::vector<cudaEvent_t> tv0, tv1, tm0, tm1;
-  auto tev = [&](std::vector<cudaEvent_t>& v, cudaStream_t s2) { if (!trace) return; cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, s2); v.push_back(e); };
-  uint32_t f0 = 0;
-  for (size_t pc = 0; pc < cuts.size(); f0 = cuts[pc], pc++) {
-    const uint32_t nf = cuts[pc] - f0;
+
+  // ---- one piece, frames [f0, f0 + nf): voices and external sources on the voice stream, then the mixer on its own ----
+  void piece(size_t pc, const PieceHook* on_piece) {
+    const uint32_t f0 = pc ? cuts[pc - 1] : 0, nf = cuts[pc] - f0;
     const int vb = two_bufs ? (int)(pc & 1) : 0;
-    const auto h0 = std::chrono::steady_clock::now();
+    trace.host_mark(0);
     if (pc >= (two_bufs ? 2u : 1u)) GH_CUDA(cudaStreamWaitEvent(st, B.ev_mixed[vb], 0));   // voice buffer vb is free again
     B.voices.reset();
     for (int i = 0; i < n; i++)
-      for (int ch = 0; ch < 7; ch++) {
-        if (ch == 5 && !E[i]->poly.used) continue;
-        if (ch == 6 && !E[i]->gran.used) continue;
-        auto& ev = vev[(size_t)i * 7 + ch];
-        size_t& p = vpos[(size_t)i * 7 + ch];
+      for (int ch = 0; ch < N_CH; ch++) {
+        const GooeyEngine::Voice& v = E[i]->voice[ch];
+        const size_t q = (size_t)i * N_CH + ch;
+        if (!v.launched) continue;
         cur.clear();
-        while (p < ev.size() && ev[p].frame < f0 + nf) { gd::VoiceEvent x = ev[p++]; x.frame -= f0; cur.push_back(x); }
-        const uint32_t type = ch < 5 ? E[i]->strip[ch].type : (ch == 5 ? GOOEY_B200_VOICE_POLY : GOOEY_B200_VOICE_GRANULATOR);
-        const int slot = ch < 5 ? E[i]->strip[ch].slot : (ch == 5 ? E[i]->poly.slot : E[i]->gran.slot);
-        B.voices.add(type, (uint32_t)slot, (uint32_t)(ch * n_lpad + i), cur, (ch < 5 && lfo_planes && !vroutes[(size_t)i * 5 + ch].empty()) ? &vroutes[(size_t)i * 5 + ch] : nullptr);
+        take_piece(vev[q], vpos[q], f0, f0 + nf, cur);
+        B.voices.add(v.type, (uint32_t)v.slot, (uint32_t)(ch * n_lpad + i), cur, lfo_planes && !vroutes[q].empty() ? &vroutes[q] : nullptr);
       }
-    const auto h1 = std::chrono::steady_clock::now();
-    cudaEvent_t start = B.ev_piece;
-    GH_CUDA(cudaEventRecord(start, st));
+    trace.host_mark(1);
+    GH_CUDA(cudaEventRecord(B.ev_piece, st));
     // the clock index differs per engine only through e->k; voices carry their own k, the launch passes the table
-    tev(tv0, st);
+    trace.mark(trace.tv0, st);
     B.voices.set_mod(lfo_planes, (long long)frames, (int)f0);
-    B.voices.launch(st, start, B.rc, tt, (int)nf, B.d_voice_bufs[vb].p, (long long)vstride);
+    B.voices.launch(st, B.ev_piece, B.rc, tt, (int)nf, B.d_voice_bufs[vb].p, (long long)vstride);
     if (ext_pairs) {   // loop mixers and sampler racks of this piece, on the voice stream (the mixer waits for ev_voices)
       const gd::ExtTickCtx xc{B.sr, B.rc.smooth15};
       if (!B.h_loop_descs.empty()) {
@@ -967,47 +1011,28 @@ inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, 
       }
       GH_CUDA(cudaGetLastError());
     }
-    tev(tv1, st);
-    const auto h2 = std::chrono::steady_clock::now();
+    trace.mark(trace.tv1, st);
+    trace.host_mark(2);
     GH_CUDA(cudaEventRecord(B.ev_voices[vb], st));
-    GH_CUDA(cudaStreamWaitEvent(ms, B.ev_voices[vb], 0));
+    GH_CUDA(cudaStreamWaitEvent(B.mix_stream, B.ev_voices[vb], 0));
+    mix_piece(f0, nf, vb);
+    if (on_piece) (*on_piece)(f0, nf, B.ev_mixed[vb]);
+    trace.mark(trace.tm1, B.mix_stream);
+    trace.host_line(pc);
+  }
+  void mix_piece(uint32_t f0, uint32_t nf, int vb) {
+    cudaStream_t ms = B.mix_stream;
     mflat.clear(); mbegin.assign(1, 0);
-    for (int i = 0; i < n; i++) {
-      auto& ev = mev[i];
-      size_t& p = mpos[i];
-      while (p < ev.size() && ev[p].frame < f0 + nf) { gd::VoiceEvent x = ev[p++]; x.frame -= f0; mflat.push_back(x); }
-      mbegin.push_back((uint32_t)mflat.size());
-    }
+    for (int i = 0; i < n; i++) { take_piece(mev[i], mpos[i], f0, f0 + nf, mflat); mbegin.push_back((uint32_t)mflat.size()); }
     if (mflat.empty()) mflat.push_back(make_event(0xffffffffu, 0xffff, 0, 0.0f));
     B.d_mix_eventss[vb].upload(mflat.data(), mflat.size(), ms);      // pageable source: staged before the call returns
     B.d_mix_ev_begins[vb].upload(mbegin.data(), mbegin.size(), ms);
-    gd::MixLaunch M;
-    memset(&M, 0, sizeof M);
-    M.state = B.mix_pool.d.p; M.n = n; M.state_cap = B.mix_pool.cap; M.slots = B.d_mix_slots.p; M.n_lpad = n_lpad;
-    M.cfg = B.d_cfg.p; M.events = B.d_mix_eventss[vb].p; M.ev_begin = B.d_mix_ev_begins[vb].p;
-    M.voice_buf = B.d_voice_bufs[vb].p; M.voice_stride = (long long)vstride; M.chan_mask = 0x1fu | (any_poly ? 0x20u : 0u) | (any_gran ? 0x40u : 0u);
-    for (int s = 0; s < gd::MAX_FX; s++) M.ring[s] = B.ring[s].p;
-    M.ring_cap = ring_cap;
-    M.frames = (int)nf;
-    M.out = out_dev + (out_mode == OUT_MONO ? (size_t)f0 : (size_t)2 * f0); M.out_stride = (long long)stride; M.out_mode = out_mode; M.out_rows = nullptr;
-    M.rc = B.rc; M.geo = B.geo;
-    M.center_l = gm::g_cosf(0.5f * 1.57079632679489661923f); M.center_r = gm::g_sinf(0.5f * 1.57079632679489661923f);
-    B.d_mix_fast.alloc(n); B.d_mix_consts.alloc(n);
-    M.fast = B.d_mix_fast.p; M.consts = B.d_mix_consts.p;
-    M.peaks = B.d_peaks.p;
-    M.premix = B.d_premix.p; M.premix_stride = (long long)vstride;
-    M.ext = ext_pairs ? B.d_ext[vb].p : nullptr; M.ext_stride = (long long)vstride;
-    M.chain_units = B.d_chain_units.p;
-    tev(tm0, ms);
+    M.events = B.d_mix_eventss[vb].p; M.ev_begin = B.d_mix_ev_begins[vb].p; M.voice_buf = B.d_voice_bufs[vb].p; M.frames = (int)nf;
+    M.out = out + (M.out_mode == OUT_MONO ? (size_t)f0 : (size_t)2 * f0);
+    M.ext = ext_pairs ? B.d_ext[vb].p : nullptr;
+    trace.mark(trace.tm0, ms);
     gd::mix_prepare_kernel<<<(n + 127) / 128, 128, 0, ms>>>(M);
     gd::mix_fast_kernel<<<dim3((nf + 1023) / 1024, n), 256, 0, ms>>>(M);
-    {
-      static std::set<int> opted;      // per device: allow the mix kernel its dynamic shared memory (> 48 KB with the static tiles)
-      if (opted.insert(B.device).second) {
-        GH_CUDA(cudaFuncSetAttribute(gd::mix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gd::MIX_DYN_SMEM));
-        GH_CUDA(cudaFuncSetAttribute(gd::chain_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gd::CHAIN_SMEM));
-      }
-    }
     B.mix_timer.begin(ms);
     // settled tilt / delay / spring chains: whole warps of engines go to the pipelined chain kernel, mix_kernel takes the rest
     const bool chain_fast = getenv("GOOEY_B200_NO_CHAIN_FAST") == nullptr;     // (tests compare the two paths bit for bit)
@@ -1017,53 +1042,61 @@ inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, 
     g_launches.fetch_add(3, std::memory_order_relaxed);
     GH_CUDA(cudaGetLastError());
     GH_CUDA(cudaEventRecord(B.ev_mixed[vb], ms));
-    if (on_piece) (*on_piece)(f0, nf, B.ev_mixed[vb]);
-    tev(tm1, ms);
-    if (trace) {
-      const auto h3 = std::chrono::steady_clock::now();
-      auto msf = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
-      fprintf(stderr, "[gooey trace] host, piece %zu: wait + event lists %.1f ms, voice launches %.1f ms, mixer launches %.1f ms\n", pc, msf(h0, h1), msf(h1, h2), msf(h2, h3));
-    }
   }
-  GH_CUDA(cudaStreamWaitEvent(st, B.ev_mixed[0], 0));
-  if (two_bufs && cuts.size() > 1) GH_CUDA(cudaStreamWaitEvent(st, B.ev_mixed[1], 0));
-  GH_CUDA(cudaEventRecord(B.ev1, st));
-  if (trace) {
+
+  // ---- read-back, once the voice stream has joined the last mixes: meters, LFO phases, loop and rack state, clocks ----
+  void read_back() {
+    GH_CUDA(cudaStreamWaitEvent(st, B.ev_mixed[0], 0));
+    if (two_bufs && cuts.size() > 1) GH_CUDA(cudaStreamWaitEvent(st, B.ev_mixed[1], 0));
+    GH_CUDA(cudaEventRecord(B.ev1, st));
+    trace.device_lines(st, cuts);
+    // the call's maxima join the engines' read-and-reset peaks (one small copy; the caller synchronises the stream anyway)
+    B.h_peaks.resize((size_t)n * gd::N_PEAKS);
+    GH_CUDA(cudaMemcpyAsync(B.h_peaks.data(), B.d_peaks.p, B.h_peaks.size() * 4, cudaMemcpyDeviceToHost, st));
+    GH_CUDA(cudaMemcpyAsync(&B.h_chain_units, B.d_chain_units.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    if (!B.h_lfo_streams.empty()) GH_CUDA(cudaMemcpyAsync(B.h_lfo_streams.data(), B.d_lfo_streams.p, B.h_lfo_streams.size() * sizeof(gd::LfoStream), cudaMemcpyDeviceToHost, st));
+    if (!B.h_loop_descs.empty()) GH_CUDA(cudaMemcpyAsync(B.h_loop_descs.data(), B.d_loop_descs.p, B.h_loop_descs.size() * sizeof(gd::LoopMixer), cudaMemcpyDeviceToHost, st));
+    if (!B.h_rack_descs.empty()) GH_CUDA(cudaMemcpyAsync(B.h_rack_descs.data(), B.d_rack_descs.p, B.h_rack_descs.size() * sizeof(gd::SamplerRack), cudaMemcpyDeviceToHost, st));
     GH_CUDA(cudaStreamSynchronize(st));
-    for (size_t pc = 0; pc < tv0.size(); pc++) {
-      float a = 0, b = 0, c = 0, d = 0;
-      cudaEventElapsedTime(&a, tv0[0], tv0[pc]); cudaEventElapsedTime(&b, tv0[pc], tv1[pc]); cudaEventElapsedTime(&c, tv0[0], tm0[pc]); cudaEventElapsedTime(&d, tm0[pc], tm1[pc]);
-      fprintf(stderr, "[gooey trace] piece %zu frames %u: voices start %.1f ms, take %.1f ms; mix start %.1f ms, takes %.1f ms\n", pc, cuts[pc] - (pc ? cuts[pc - 1] : 0), a, b, c, d);
+    for (size_t q = 0; q < loop_refs.size(); q++)      // playback state back into the engines' loop channels / sampler voices
+      for (int c = 0; c < gd::LOOP_CHANNELS; c++) E[loop_refs[q]]->loops[c].absorb(B.h_loop_descs[q].ch[c]);
+    for (size_t q = 0; q < rack_refs.size(); q++) {
+      auto& R = E[rack_refs[q].engine]->samplers[rack_refs[q].rack];
+      memcpy(R.voices, B.h_rack_descs[q].v, sizeof R.voices);
+      R.next_age = B.h_rack_descs[q].next_age;
+      for (int v = 0; v < gd::SAMPLER_VOICES; v++) {    // a voice the device started plays its pad's buffer (a pad cannot change during a call)
+        if (!R.voices[v].samples) R.voices_release(v);
+        else R.voice_buf[v] = R.slots[R.voices[v].slot].buf;
+      }
     }
-    for (auto* v : {&tv0, &tv1, &tm0, &tm1}) for (auto e : *v) cudaEventDestroy(e);
-  }
-  // meters: the call's maxima join the engines' read-and-reset peaks (one small copy; the caller synchronises the stream anyway)
-  B.h_peaks.resize((size_t)n * gd::N_PEAKS);
-  GH_CUDA(cudaMemcpyAsync(B.h_peaks.data(), B.d_peaks.p, B.h_peaks.size() * 4, cudaMemcpyDeviceToHost, st));
-  GH_CUDA(cudaMemcpyAsync(&B.h_chain_units, B.d_chain_units.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-  if (!B.h_lfo_streams.empty()) GH_CUDA(cudaMemcpyAsync(B.h_lfo_streams.data(), B.d_lfo_streams.p, B.h_lfo_streams.size() * sizeof(gd::LfoStream), cudaMemcpyDeviceToHost, st));
-  if (!B.h_loop_descs.empty()) GH_CUDA(cudaMemcpyAsync(B.h_loop_descs.data(), B.d_loop_descs.p, B.h_loop_descs.size() * sizeof(gd::LoopMixer), cudaMemcpyDeviceToHost, st));
-  if (!B.h_rack_descs.empty()) GH_CUDA(cudaMemcpyAsync(B.h_rack_descs.data(), B.d_rack_descs.p, B.h_rack_descs.size() * sizeof(gd::SamplerRack), cudaMemcpyDeviceToHost, st));
-  GH_CUDA(cudaStreamSynchronize(st));
-  for (size_t q = 0; q < loop_refs.size(); q++)      // playback state back into the engines' loop channels / sampler voices
-    for (int c = 0; c < gd::LOOP_CHANNELS; c++) {
-      E[loop_refs[q]]->loops[c].absorb(B.h_loop_descs[q].ch[c]);
-    }
-  for (size_t q = 0; q < rack_refs.size(); q++) {
-    auto& R = E[rack_refs[q].engine]->samplers[rack_refs[q].rack];
-    memcpy(R.voices, B.h_rack_descs[q].v, sizeof R.voices);
-    R.next_age = B.h_rack_descs[q].next_age;
-    for (int v = 0; v < gd::SAMPLER_VOICES; v++) {    // a voice the device started plays its pad's buffer (a pad cannot change during a call)
-      if (!R.voices[v].samples) R.voices_release(v);
-      else R.voice_buf[v] = R.slots[R.voices[v].slot].buf;
+    for (size_t q = 0; q < lfo_refs.size(); q++) E[lfo_refs[q].engine]->lfos[lfo_refs[q].lfo].phase = B.h_lfo_streams[q].phase;
+    for (int i = 0; i < n; i++) {
+      for (int q = 0; q < gd::N_PEAKS; q++) { const float v = B.h_peaks[(size_t)i * gd::N_PEAKS + q]; if (v > E[i]->peaks[q]) E[i]->peaks[q] = v; }
+      E[i]->k += frames;
+      if (bounce) { for (auto& s : E[i]->strip) s.seq.stop(); for (auto& R : E[i]->samplers) if (R.registered) R.pat.seq.stop(); }
     }
   }
-  for (size_t q = 0; q < lfo_refs.size(); q++) E[lfo_refs[q].engine]->lfos[lfo_refs[q].lfo].phase = B.h_lfo_streams[q].phase;
-  for (int i = 0; i < n; i++) {
-    for (int q = 0; q < gd::N_PEAKS; q++) { const float v = B.h_peaks[(size_t)i * gd::N_PEAKS + q]; if (v > E[i]->peaks[q]) E[i]->peaks[q] = v; }
-    E[i]->k += frames;
-    if (bounce) { for (auto& s : E[i]->strip) s.seq.stop(); for (auto& R : E[i]->samplers) if (R.registered) R.pat.seq.stop(); }
-  }
+};
+
+// Renders `frames` frames of every engine of `E` (all on one bank) into out_dev: mono rows [n][stride] (the bounce
+// downmix 0.5 (l + r)) or interleaved stereo rows [n][stride >= 2 frames].  `bounce`: apply the reference's bounce
+// preamble first (ffi.rs:7840-7854): clock to 0, sequencers reset + start, strips / graph / master snapped.
+// on_piece (optional): called after the mix of frames [f0, f0 + nf) has been enqueued, with the event that marks it done.
+inline void engines_render(const std::vector<GooeyEngine*>& E, uint32_t frames, int out_mode, bool bounce, float* out_dev, size_t stride,
+                           const PieceHook* on_piece = nullptr) {
+  if (E.empty() || frames == 0) return;
+  EngineBank& B = *E[0]->bank;
+  std::lock_guard<std::recursive_mutex> lk(B.mu);
+  GH_CUDA(cudaSetDevice(B.device));
+  EngineRender R(B, E, frames, bounce);
+  R.check_batch();
+  R.schedule();
+  R.ext_sources();
+  R.device_state();
+  R.lfo_pool();
+  R.mixer_setup(out_mode, out_dev, stride);
+  for (size_t pc = 0; pc < R.cuts.size(); pc++) R.piece(pc, on_piece);
+  R.read_back();
 }
 
 }  // namespace gh

@@ -18,11 +18,11 @@ EngineBank& engine_bank(int device, float sr) {
   if (it == banks.end()) it = banks.emplace(std::make_pair(device, key), new EngineBank(device, sr)).first;
   return *it->second;
 }
-static GooeyEngine::Strip* strip_by_type(GooeyEngine* e, uint32_t type) {
-  for (auto& s : e->strip) if (s.type == type) return &s;
+static GooeyEngine::Voice* strip_by_type(GooeyEngine* e, uint32_t type) {
+  for (int c = 0; c < N_STRIPS; c++) if (e->voice[c].type == type) return &e->voice[c];
   return nullptr;
 }
-static void strip_set_param(GooeyEngine::Strip* s, uint32_t param, float value) {
+static void strip_set_param(GooeyEngine::Voice* s, uint32_t param, float value) {
   if (!s) return;
   ffi_param_to_events(s->type, param, value, [&](uint32_t kind, uint32_t p, float v) { s->pending.push_back(make_event(0, kind, p, v)); });
 }
@@ -54,6 +54,13 @@ static uint32_t bounce_frames(const GooeyEngine* e, uint32_t bars) {   // ffi.rs
 }
 }  // namespace gh
 
+const float GOOEY_POLY_PRESETS[5][14] = {   // PolySynthConfig::{default,pad,pluck,keys,strings} (poly_synth.rs:49-142), ffi preset ids 0-4
+    {0.0f, 0.2f, 0.6f, 0.15f, 0.3f, 0.55f, 0.7f, 0.7f, 0.8f, 0.5f, 0.65f, 0.4f, 0.75f, 0.7f},
+    {0.0f, 0.4f, 0.45f, 0.2f, 0.2f, 0.8f, 0.75f, 0.8f, 0.85f, 0.75f, 0.7f, 0.5f, 0.8f, 0.6f},
+    {0.3f, 0.1f, 0.7f, 0.25f, 0.6f, 0.0f, 0.75f, 0.0f, 0.65f, 0.0f, 0.7f, 0.1f, 0.65f, 0.7f},
+    {0.5f, 0.15f, 0.55f, 0.1f, 0.4f, 0.35f, 0.7f, 0.5f, 0.75f, 0.3f, 0.65f, 0.3f, 0.7f, 0.7f},
+    {0.0f, 0.5f, 0.5f, 0.1f, 0.15f, 0.85f, 0.7f, 0.9f, 0.85f, 0.8f, 0.7f, 0.6f, 0.8f, 0.5f}};
+
 extern "C" {
 
 int gooey_b200_set_device(int device) {
@@ -80,29 +87,30 @@ void gooey_engine_set_snare_param(GooeyEngine* e, uint32_t p, float v) { if (e) 
 void gooey_engine_set_hihat_param(GooeyEngine* e, uint32_t p, float v) { if (e) gh::strip_set_param(gh::strip_by_type(e, GOOEY_INSTRUMENT_HIHAT), p, v); }
 void gooey_engine_set_tom_param(GooeyEngine* e, uint32_t p, float v) { if (e) gh::strip_set_param(gh::strip_by_type(e, GOOEY_INSTRUMENT_TOM), p, v); }
 void gooey_engine_set_bass_param(GooeyEngine* e, uint32_t p, float v) { if (e) gh::strip_set_param(gh::strip_by_type(e, GOOEY_INSTRUMENT_BASS), p, v); }
-void gooey_engine_set_channel_param(GooeyEngine* e, uint32_t ch, uint32_t p, float v) { if (e && ch < 5) gh::strip_set_param(&e->strip[ch], p, v); }
+void gooey_engine_set_channel_param(GooeyEngine* e, uint32_t ch, uint32_t p, float v) { if (e && ch < 5) gh::strip_set_param(&e->voice[ch], p, v); }
 // ffi.rs:2304-2343: a different synthesizer type on `channel`; the new instrument is `<Voice>::new(sample_rate)` and
 // starts fresh, the strip (gain, pan, mute / solo, sequencer pattern) is kept.  Parameter edits still queued for the old
 // instrument were applied to it (and die with it).
 void gooey_engine_set_channel_instrument_type(GooeyEngine* e, uint32_t ch, uint32_t type) {
   if (!e || ch >= 5 || type > GOOEY_INSTRUMENT_BASS) return;
+  GooeyEngine::Voice& v = e->voice[ch];
   GooeyEngine::Strip& s = e->strip[ch];
-  if (s.type == type) return;
+  if (v.type == type) return;
   try {
     gh::EngineBank& B = *e->bank;
     std::lock_guard<std::recursive_mutex> lk(B.mu);
     const GooeyVoicePatch p = gh::default_patch(type);
     const int slot = B.voices.create(p, e->sr);
     if (slot < 0) return;
-    B.voices.release(s.type, s.slot);
-    s.type = type; s.slot = slot;
-    s.pending.clear();
-    s.pending.push_back(gh::make_event(0, gd::EV_SET_TIME, 0, 0.0f, e->k));   // the fresh voice joins the engine's clock
+    B.voices.release(v.type, v.slot);
+    v.type = type; v.slot = slot;
+    v.pending.clear();
+    v.pending.push_back(gh::make_event(0, gd::EV_SET_TIME, 0, 0.0f, e->k));   // the fresh voice joins the engine's clock
     s.blender.default_for_type(type);                                          // ffi.rs:2334-2342
-    if (s.blend_enabled) s.blender.apply(s.blend_x, s.blend_y, 0, [&](const gd::VoiceEvent& x) { s.pending.push_back(x); });
+    if (s.blend_enabled) s.blender.apply(s.blend_x, s.blend_y, 0, [&](const gd::VoiceEvent& x) { v.pending.push_back(x); });
   } catch (const std::exception& ex) { gh::set_error(ex.what()); gh::engine_fail(e, ex.what()); }
 }
-uint32_t gooey_engine_get_channel_instrument_type(const GooeyEngine* e, uint32_t ch) { return (e && ch < 5) ? e->strip[ch].type : 0xFFFFFFFFu; }   /* :2354-2371 */
+uint32_t gooey_engine_get_channel_instrument_type(const GooeyEngine* e, uint32_t ch) { return (e && ch < 5) ? e->voice[ch].type : 0xFFFFFFFFu; }   /* :2354-2371 */
 
 // ---- LFO pool (ffi.rs:4616-4993): eight tempo-synced sine LFOs, each routed to up to 16 (channel, parameter, depth) targets ----
 uint32_t gooey_engine_lfo_count(void) { return 8; }
@@ -141,7 +149,7 @@ void gooey_engine_blend_set_position(GooeyEngine* e, uint32_t inst, float x, flo
   GooeyEngine::Strip& s = e->strip[inst];
   if (!s.blend_enabled) return;
   s.blend_x = gd::clampf(x, 0.0f, 1.0f); s.blend_y = gd::clampf(y, 0.0f, 1.0f);
-  s.blender.apply(s.blend_x, s.blend_y, 0, [&](const gd::VoiceEvent& ev) { s.pending.push_back(ev); });
+  s.blender.apply(s.blend_x, s.blend_y, 0, [&](const gd::VoiceEvent& ev) { e->voice[inst].pending.push_back(ev); });
 }
 float gooey_engine_blend_get_position_x(const GooeyEngine* e, uint32_t inst) { return (e && inst < 5) ? e->strip[inst].blend_x : -1.0f; }
 float gooey_engine_blend_get_position_y(const GooeyEngine* e, uint32_t inst) { return (e && inst < 5) ? e->strip[inst].blend_y : -1.0f; }
@@ -153,7 +161,7 @@ void gooey_engine_blend_set_corner_preset(GooeyEngine* e, uint32_t inst, uint32_
 uint32_t gooey_engine_blend_get_corner_preset(const GooeyEngine* e, uint32_t inst, uint32_t corner) {
   return (e && inst < 5 && corner < 4) ? e->strip[inst].blender.corner_ids[corner] : 0xFFFFFFFFu;
 }
-void gooey_engine_blend_reset_corners(GooeyEngine* e, uint32_t inst) { if (e && inst < 5) e->strip[inst].blender.default_for_type(e->strip[inst].type); }
+void gooey_engine_blend_reset_corners(GooeyEngine* e, uint32_t inst) { if (e && inst < 5) e->strip[inst].blender.default_for_type(e->voice[inst].type); }
 void gooey_engine_sequencer_set_instrument_step_blend(GooeyEngine* e, uint32_t inst, uint32_t step, float x, float y) {
   if (!e || inst >= 5 || step >= e->strip[inst].seq.pattern.size()) return;
   gh::SeqStep& st = e->strip[inst].seq.pattern[step];
@@ -174,16 +182,11 @@ float gooey_engine_sequencer_get_instrument_step_blend_y(const GooeyEngine* e, u
   return e->strip[inst].seq.pattern[step].by;
 }
 
-void gooey_engine_load_bass_preset(GooeyEngine* e, uint32_t id) {
-  if (!e || id > 3) return;
-  static const float P[4][15] = {   // BassConfig::{acid,sub,reese,stab} (bass.rs:188-269); set_config = 15 set_targets
-      {0.24f, 0.40f, 0.80f, 0.00f, 0.00f, 0.10f, 0.15f, 0.70f, 0.85f, 0.15f, 0.08f, 0.35f, 0.10f, 0.30f, 0.80f},
-      {0.18f, 1.00f, 0.15f, 0.00f, 0.00f, 0.00f, 0.70f, 0.05f, 0.10f, 0.30f, 0.20f, 0.60f, 0.15f, 0.00f, 0.85f},
-      {0.18f, 0.30f, 0.80f, 0.80f, 0.50f, 0.05f, 0.35f, 0.30f, 0.50f, 0.40f, 0.15f, 0.55f, 0.12f, 0.60f, 0.80f},
-      {0.30f, 0.20f, 0.90f, 0.00f, 0.00f, 0.90f, 0.20f, 0.40f, 0.90f, 0.08f, 0.05f, 0.20f, 0.08f, 0.20f, 0.80f}};
-  GooeyEngine::Strip* s = gh::strip_by_type(e, GOOEY_INSTRUMENT_BASS);
-  if (!s) return;
-  for (uint32_t i = 0; i < 15; i++) s->pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, i, gh::clamp01(P[id][i])));
+void gooey_engine_load_bass_preset(GooeyEngine* e, uint32_t id) {   // BassConfig::{acid,sub,reese,stab} (gh::preset_flat); set_config = 15 set_targets
+  GooeyEngine::Voice* bass = e ? gh::strip_by_type(e, GOOEY_INSTRUMENT_BASS) : nullptr;
+  float v[24];
+  if (!bass || gh::preset_flat(GOOEY_INSTRUMENT_BASS, id, v) == 0) return;
+  for (uint32_t i = 0; i < 15; i++) bass->pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, i, gh::clamp01(v[i])));
 }
 
 void gooey_engine_set_bpm(GooeyEngine* e, float bpm) {
@@ -441,27 +444,19 @@ void gooey_engine_track_effect_set_param(GooeyEngine* e, uint32_t t, uint32_t po
 }
 
 // ---- poly synth (ffi.rs:5571-5648, 5899-5935; poly_synth.rs) ----
-static const float GOOEY_POLY_PRESETS[5][14] = {   // PolySynthConfig::{default,pad,pluck,keys,strings} (poly_synth.rs:49-142), ffi preset ids 0-4
-    {0.0f, 0.2f, 0.6f, 0.15f, 0.3f, 0.55f, 0.7f, 0.7f, 0.8f, 0.5f, 0.65f, 0.4f, 0.75f, 0.7f},
-    {0.0f, 0.4f, 0.45f, 0.2f, 0.2f, 0.8f, 0.75f, 0.8f, 0.85f, 0.75f, 0.7f, 0.5f, 0.8f, 0.6f},
-    {0.3f, 0.1f, 0.7f, 0.25f, 0.6f, 0.0f, 0.75f, 0.0f, 0.65f, 0.0f, 0.7f, 0.1f, 0.65f, 0.7f},
-    {0.5f, 0.15f, 0.55f, 0.1f, 0.4f, 0.35f, 0.7f, 0.5f, 0.75f, 0.3f, 0.65f, 0.3f, 0.7f, 0.7f},
-    {0.0f, 0.5f, 0.5f, 0.1f, 0.15f, 0.85f, 0.7f, 0.9f, 0.85f, 0.8f, 0.7f, 0.6f, 0.8f, 0.5f}};
 void gooey_engine_poly_set_preset(GooeyEngine* e, uint32_t preset) {   // set_config: 14 smoothed targets, no snap
   if (!e) return;
-  gh::aux_touch(e, false);
+  auto& pending = gh::aux_touch(e, gh::CH_POLY);
   const float* t = GOOEY_POLY_PRESETS[preset < 5 ? preset : 0];
-  for (uint32_t i = 0; i < 14; i++) e->poly.pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, i, t[i]));
+  for (uint32_t i = 0; i < 14; i++) pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, i, t[i]));
 }
 void gooey_engine_poly_set_param(GooeyEngine* e, uint32_t param, float value) {
   if (!e || param >= 14) return;
-  gh::aux_touch(e, false);
-  e->poly.pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, param, gd::clampf(value, 0.0f, 1.0f)));
+  gh::aux_touch(e, gh::CH_POLY).push_back(gh::make_event(0, gd::EV_SET_TARGET, param, gd::clampf(value, 0.0f, 1.0f)));
 }
 void gooey_engine_poly_release(GooeyEngine* e) {
   if (!e) return;
-  gh::aux_touch(e, false);
-  e->poly.pending.push_back(gh::make_event(0, gd::EV_POLY_RELEASE, 0, 0.0f));
+  gh::aux_touch(e, gh::CH_POLY).push_back(gh::make_event(0, gd::EV_POLY_RELEASE, 0, 0.0f));
 }
 // The tail of gooey_engine_poly_trigger_chord (ffi.rs:5594-5611) once `music::apply_voicing` has produced the MIDI notes:
 // preset as smoothed targets, release_all, trigger every note.  (The chord -> notes tables of src/music are host-side
@@ -470,8 +465,8 @@ void gooey_engine_poly_trigger_notes(GooeyEngine* e, const uint8_t* notes, uint3
   if (!e || (!notes && n)) return;
   gooey_engine_poly_set_preset(e, preset);
   const float v = gd::clampf(velocity, 0.0f, 1.0f);
-  e->poly.pending.push_back(gh::make_event(0, gd::EV_POLY_RELEASE, 0, 0.0f));
-  for (uint32_t i = 0; i < n; i++) e->poly.pending.push_back(gh::make_event(0, gd::EV_POLY_NOTE, notes[i], v));
+  e->voice[gh::CH_POLY].pending.push_back(gh::make_event(0, gd::EV_POLY_RELEASE, 0, 0.0f));
+  for (uint32_t i = 0; i < n; i++) e->voice[gh::CH_POLY].pending.push_back(gh::make_event(0, gd::EV_POLY_NOTE, notes[i], v));
 }
 
 // ffi.rs:5571-5611: diatonic seventh chord of (root, scale) at `degree`, voiced, on the poly synth
@@ -489,13 +484,7 @@ uint32_t gooey_b200_chord_notes(uint32_t root, uint32_t scale_type, uint32_t deg
 }
 
 // ---- granulator (ffi.rs:5969-5990, 7702-7827; granulator.rs) ----
-static void gran_attach(GooeyEngine* e) {
-  gh::aux_touch(e, true);
-  const uint64_t ptr = (uint64_t)(uintptr_t)e->gran_buf->p;
-  float lo; uint32_t lo_bits = (uint32_t)ptr; memcpy(&lo, &lo_bits, 4);
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_GRAN_BUFFER, 0, lo, (uint32_t)(ptr >> 32)));   // kills all grains, like set_buffer
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_SET_AUX, gd::AUX_GRAN_BUFINFO, e->gran_sr, e->gran_len));
-}
+static void gran_attach(GooeyEngine* e) { gh::gran_buffer_events(gh::aux_touch(e, gh::CH_GRAN), 0, e->gran_buf->p, e->gran_sr, e->gran_len); }
 bool gooey_engine_granulator_set_buffer(GooeyEngine* e, const float* samples, uint32_t len, float sample_rate) {
   if (!e || !samples || len == 0) return false;
   if (!std::isfinite(sample_rate) || !(sample_rate > 0.0f)) return false;            // SampleBuffer::from_mono (granulator.rs:60-90)
@@ -522,23 +511,19 @@ bool gooey_b200_granulator_share_buffer(GooeyEngine* dst, const GooeyEngine* src
 }
 void gooey_engine_granulator_trigger(GooeyEngine* e, float velocity) {
   if (!e) return;
-  gh::aux_touch(e, true);
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_TRIGGER, 0, gd::clampf(velocity, 0.0f, 1.0f)));
+  gh::aux_touch(e, gh::CH_GRAN).push_back(gh::make_event(0, gd::EV_TRIGGER, 0, gd::clampf(velocity, 0.0f, 1.0f)));
 }
 void gooey_engine_granulator_set_param(GooeyEngine* e, uint32_t param, float value) {
   if (!e || param >= 12) return;
-  gh::aux_touch(e, true);
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_SET_TARGET, param, gd::clampf(value, 0.0f, 1.0f)));
+  gh::aux_touch(e, gh::CH_GRAN).push_back(gh::make_event(0, gd::EV_SET_TARGET, param, gd::clampf(value, 0.0f, 1.0f)));
 }
 void gooey_engine_granulator_set_seed(GooeyEngine* e, uint32_t seed) {
   if (!e) return;
-  gh::aux_touch(e, true);
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_GRAN_SEED, 0, 0.0f, seed));
+  gh::aux_touch(e, gh::CH_GRAN).push_back(gh::make_event(0, gd::EV_GRAN_SEED, 0, 0.0f, seed));
 }
 void gooey_engine_granulator_snap_params(GooeyEngine* e) {
   if (!e) return;
-  gh::aux_touch(e, true);
-  e->gran.pending.push_back(gh::make_event(0, gd::EV_SNAP, 0, 0.0f));
+  gh::aux_touch(e, gh::CH_GRAN).push_back(gh::make_event(0, gd::EV_SNAP, 0, 0.0f));
 }
 uint32_t gooey_engine_granulator_buffer_len(const GooeyEngine* e) { return e ? e->gran_len : 0; }                        /* :7665 */
 float gooey_engine_granulator_buffer_sample_rate(const GooeyEngine* e) { return e ? e->gran_sr : 0.0f; }               /* :7680 */

@@ -250,11 +250,8 @@ static int voice_of_kind(GooeyVoiceBatch* b, uint32_t voice, uint32_t kind, cons
   }
   return GOOEY_E_OK;
 }
-static void gran_queue(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, const gh::GranSource& src) {   // gran_attach's order (engine_api.cuh)
-  const uint64_t ptr = (uint64_t)(uintptr_t)src.buf->p;
-  float lo; uint32_t lo_bits = (uint32_t)ptr; memcpy(&lo, &lo_bits, 4);
-  b->pending[voice].push_back(make_event(frame, gd::EV_GRAN_BUFFER, 0, lo, (uint32_t)(ptr >> 32)));   // kills all grains, like set_buffer
-  b->pending[voice].push_back(make_event(frame, gd::EV_SET_AUX, gd::AUX_GRAN_BUFINFO, src.sr, src.len));
+static void gran_queue(GooeyVoiceBatch* b, uint32_t voice, uint32_t frame, const gh::GranSource& src) {
+  gran_buffer_events(b->pending[voice], frame, src.buf->p, src.sr, src.len);
   b->gran_queued[voice].emplace_back(frame, src);
   b->gran_latest[voice] = src;
 }

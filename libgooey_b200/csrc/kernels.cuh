@@ -11,8 +11,8 @@
 //                    reads the planes through 32x32 shared-memory tiles and writes the output the same way
 //                    (128-bit coalesced stores).
 //   slow_kernel  (S) one thread per voice, the reference's whole tick per sample.  Used for voices whose parameters
-//                    are still gliding when the call starts or are edited without a snap (A marks them), and for
-//                    the voice types that have no split yet (bass, poly, granulator).
+//                    are still gliding when the call starts or are edited without a snap (A marks them), for
+//                    LFO-routed basses, and for poly synths under GOOEY_B200_BACKEND=serial (pool.cuh launch_back).
 // Output layout: out[row * stride + frame] (voice-major).  State layout: word-interleaved SoA, state[w * n_pad + slot].
 #pragma once
 #include <cuda_runtime.h>

@@ -13,8 +13,6 @@
 // sub-voice is active, lane 0 runs poly_tick for the block, so the two paths share one state and alternate freely.
 // Nothing is re-associated: the output is bit-identical to slow_kernel<PolyV>.
 #define GOOEY_OWN_KERNELS_TU
-#include <mutex>
-#include <set>
 #include "device_rt.h"
 #include "bass_wave.cuh"
 #include "poly_wave.cuh"
@@ -244,15 +242,7 @@ void poly_wave_launch(const VoiceLaunch& L, cudaStream_t st) {
   // Every kernel of a render runs at the maximum shared-memory carve-out (pool.cuh same_carveout): kernels whose
   // carve-outs differ cannot share an SM.
   auto kernel = poly_wave_kernel<POLY_WAVE_WARPS>;
-  static std::mutex mu;
-  static std::set<int> done;
-  int dev = 0;
-  GH_CUDA(cudaGetDevice(&dev));
-  {
-    std::lock_guard<std::mutex> lk(mu);
-    if (done.insert(dev).second)
-      GH_CUDA(cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-  }
+  gh::func_attr_once((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
   kernel<<<(L.n + POLY_WAVE_WARPS - 1) / POLY_WAVE_WARPS, POLY_WAVE_WARPS * 32, 0, st>>>(L);
 }
 void poly_wave_set_midi_freq(const double mf[128]) { GH_CUDA(cudaMemcpyToSymbol(c_midi_freq, mf, 128 * sizeof(double))); }

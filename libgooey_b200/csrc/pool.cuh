@@ -14,7 +14,6 @@
 #include <atomic>
 #include <map>
 #include <type_traits>
-#include <set>
 #include <mutex>
 #include <tuple>
 #include "device_rt.h"
@@ -139,6 +138,14 @@ inline gd::VoiceEvent make_event(uint32_t frame, uint32_t kind, uint32_t param, 
   gd::VoiceEvent e; e.frame = frame; e.kind = (uint16_t)kind; e.param = (uint16_t)param; e.value = value; e.aux = aux;
   return e;
 }
+// Granulator::set_buffer at `frame`: the buffer's device address (low word in the bits of the value), which kills every grain,
+// then its sample rate and length.
+inline void gran_buffer_events(std::vector<gd::VoiceEvent>& out, uint32_t frame, const float* buf, float sr, uint32_t len) {
+  const uint64_t ptr = (uint64_t)(uintptr_t)buf;
+  float lo; uint32_t lo_bits = (uint32_t)ptr; memcpy(&lo, &lo_bits, 4);
+  out.push_back(make_event(frame, gd::EV_GRAN_BUFFER, 0, lo, (uint32_t)(ptr >> 32)));
+  out.push_back(make_event(frame, gd::EV_SET_AUX, gd::AUX_GRAN_BUFINFO, sr, len));
+}
 
 // The engine clock: tt[k] = value of a f64 accumulator after k additions of 1/sr, exactly as the reference's
 // `current_time += 1.0 / sample_rate` (bounce.rs:48-53, ffi.rs:1379).  The host keeps one checkpoint every CK additions
@@ -219,17 +226,8 @@ template <> struct WaveOf<gd::TomV> { using W = gd::wave::TomW; static constexpr
 inline void coop_launch(int cnt, cudaStream_t s, const gd::VoiceLaunch& L) {
   using SM = gd::coop::Smem<gd::coop::TomC, COOP_NV>;
   auto kernel = gd::coop::coop_kernel<gd::coop::TomC, COOP_NV>;
-  static std::mutex mu;
-  static std::set<int> done;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  {
-    std::lock_guard<std::mutex> lk(mu);
-    if (done.insert(dev).second) {
-      GH_CUDA(cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SM)));
-      GH_CUDA(cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    }
-  }
+  func_attr_once((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SM));
+  func_attr_once((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
   kernel<<<(cnt + COOP_NV - 1) / COOP_NV, COOP_NV * 32, sizeof(SM), s>>>(L);
 }
 
@@ -237,13 +235,7 @@ inline void coop_launch(int cnt, cudaStream_t s, const gd::VoiceLaunch& L) {
 // back end with 19 KB of scan tables per CTA and one with 3.5 KB would be given disjoint SMs instead of interleaving
 // their warps.  Every kernel of the render is therefore pinned to the same (maximum shared) carve-out, once per device.
 template <class K> inline void same_carveout(K kernel) {
-  static std::mutex mu;
-  static std::set<std::pair<int, const void*>> done;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  std::lock_guard<std::mutex> lk(mu);
-  if (done.insert({dev, (const void*)kernel}).second)
-    GH_CUDA(cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  func_attr_once((const void*)kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
 }
 #define GH_LAUNCH(kernel, grid, block, stream, ...) do { same_carveout(kernel); kernel<<<grid, block, 0, stream>>>(__VA_ARGS__); } while (0)
 
