@@ -12,7 +12,7 @@
 //                    (128-bit coalesced stores).
 //   slow_kernel  (S) one thread per voice, the reference's whole tick per sample.  Used for voices whose parameters
 //                    are still gliding when the call starts or are edited without a snap (A marks them), for
-//                    LFO-routed basses, and for poly synths under GOOEY_B200_BACKEND=serial (pool.cuh launch_back).
+//                    LFO-routed basses, and for basses and poly synths under GOOEY_B200_BACKEND=serial (pool.cuh launch_back).
 // Output layout: out[row * stride + frame] (voice-major).  State layout: word-interleaved SoA, state[w * n_pad + slot].
 #pragma once
 #include <cuda_runtime.h>

@@ -197,8 +197,9 @@ ClockTable& clock_table(float sr);
 //   kick / snare / hi-hat / tom, fewer voices     wave_kernel<...W>           (wave.cuh)
 //   kick / snare / hi-hat, >= SERIAL_FROM voices  back_kernel<V, 32>          (kernels.cuh)
 // The other types have one back end each: bass_wave_kernel (slow_kernel<BassV> for LFO-routed basses), poly_wave_kernel
-// and gran_wave_kernel.  GOOEY_B200_BACKEND=serial puts every drum on back_kernel and every poly synth on
-// slow_kernel<PolyV> (instead of poly_wave_kernel): the per-sample-order references of the parity tests.
+// and gran_wave_kernel.  GOOEY_B200_BACKEND=serial puts every drum on back_kernel, every bass on slow_kernel<BassV>
+// (instead of bass_wave_kernel) and every poly synth on slow_kernel<PolyV> (instead of poly_wave_kernel): the
+// per-sample-order references of the parity tests.
 enum class Back { Wave, Coop, Serial };
 // The cooperative back end issues ~3x fewer instructions per voice-frame but walks a block through barrier-separated phases,
 // so a voice's timeline is slower than in the warp-per-voice back end while voices are too few to fill the device with CTAs:
@@ -256,7 +257,7 @@ template <class V> inline const char* launch_back(const gd::VoiceLaunch& L, cuda
   return "back_kernel";
 }
 template <> inline const char* launch_back<gd::BassV>(const gd::VoiceLaunch& L, cudaStream_t s) {
-  if (L.routes) { slow_launch<gd::BassV>(L, s); return "slow_kernel<BassV>"; }   // LFO-routed basses
+  if (L.routes || serial_backend()) { slow_launch<gd::BassV>(L, s); return "slow_kernel<BassV>"; }   // LFO-routed basses, the serial reference
   GH_LAUNCH((gd::bass_wave_kernel<2>), (L.n + 1) / 2, 64, s, L);                 // one warp per bass voice, lane = frame (bass_wave.cuh)
   return "bass_wave_kernel";
 }
